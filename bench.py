@@ -6,6 +6,7 @@ guess + MultiPhaseDDP::solve for every problem of the rank's shard.
 
   python bench.py --gpus N --steps K --warmup W            # our arm (CUDA path through the C ABI)
   python bench.py --impl reference --gpus N --steps K ...  # CPU arm: the reference's HS-DDP path on host cores
+  python bench.py ... --dump-outputs DIR                   # also write what the last timed step computed (DIR/<name>.npy)
 
 Workload: SURVEY.md §8(d) config 3 — 16,384 mixed-gait Mini Cheetah problems
 (trot / bound / pronk with flight phases and reset maps), plan 0.6 s, dt 0.01, ReB+AL.
@@ -26,6 +27,7 @@ import json
 import os
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -59,7 +61,39 @@ def parse():
     ap.add_argument("--no-strong", action="store_true")
     ap.add_argument("--no-generic", action="store_true", help="skip the generic SinglePhase<12,12,0> / <36,12,12> sweep timing")
     ap.add_argument("--no-latency", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed as DIR/<name>.npy (float64, "
+                    "at most 64 MB; with several ranks, DIR/rank<r>/); the inputs depend only on the arguments")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the CUDA path (--impl ours)")
+    return args
+
+
+def dump_outputs(pkg, B, out_dir, seed=0):
+    """What a caller reads back after a solve of the batch, as float64 .npy files of at most 64 MB in all: the result
+    record of every problem (info_<field>; a seeded sample beyond ~190k problems, indices in info_problem) and, for a
+    seeded sample of at most 128 problems (indices in sample_problem), the trajectories Xbar / Ubar, the feed-forward
+    dU and the gains K [stage, row, col] of every stage."""
+    os.makedirs(out_dir, exist_ok=True)
+    rng = np.random.default_rng(seed)
+    fields = [f for f in pkg.INFO_DTYPE.names if f != "_pad"]
+    rows = {"Xbar": B.max_nodes, "Ubar": B.max_stages, "dU": B.max_stages, "K": B.max_stages}
+    cols = {"Xbar": 24, "Ubar": 24, "dU": 24, "K": 576}
+    n_info = min(B.n, (16 << 20) // (8 * (len(fields) + 1)))
+    n_traj = min(B.n, 128, (44 << 20) // (8 * sum(rows[k] * cols[k] for k in rows)))
+    pick_info = np.sort(rng.choice(B.n, n_info, replace=False))
+    pick = np.sort(rng.choice(B.n, n_traj, replace=False))
+    info = B.info()[pick_info]
+    out = {"info_problem": pick_info, "sample_problem": pick}
+    out.update({"info_" + f: info[f] for f in fields})
+    for name, nr in rows.items():
+        buf = np.zeros((B.n, 1, cols[name]))
+        a = np.stack([B.get_rows(name, r, 1, out=buf)[pick, 0] for r in range(nr)], axis=1)  # row by row: K of a batch is GBs
+        out[name] = np.swapaxes(a.reshape(n_traj, nr, 24, 24), -1, -2) if name == "K" else a  # K: column-major on the device
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a, np.float64))
 
 
 def config_block(args, world, name, n_schedules):
@@ -171,12 +205,13 @@ def cpu_baseline_block(r, cores, count, orc, extra=None):
 def cpu_native_rate(orc, tabs, k0, x0, plan, cores):
     """The same oracle compiled -O3 -march=native ON THIS HOST (SURVEY.md §8d: reported separately); best effort."""
     try:
-        so = "/tmp/liboracle_hsddp_native.so"
-        src = [os.path.join(ROOT, "oracle", f) for f in ("hsddp_oracle.cpp", "oracle_capi.cpp")]
-        subprocess.check_call(["g++", "-O3", "-march=native", "-std=c++17", "-fPIC", "-pthread", "-w", "-shared", "-o", so] + src + ["-ldl"],
-                              stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL, timeout=300)
         import ctypes as C
-        L = C.CDLL(so)
+        with tempfile.TemporaryDirectory() as tmp:  # private to this run: the tree may be read-only, /tmp is shared
+            so = os.path.join(tmp, "liboracle_hsddp_native.so")
+            src = [os.path.join(ROOT, "oracle", f) for f in ("hsddp_oracle.cpp", "oracle_capi.cpp")]
+            subprocess.check_call(["g++", "-O3", "-march=native", "-std=c++17", "-fPIC", "-pthread", "-w", "-shared", "-o", so] + src + ["-ldl"],
+                                  stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL, timeout=300)
+            L = C.CDLL(so)
         L.orc_batch_solve.restype = C.c_double
         L.orc_batch_solve.argtypes = orc.lib().orc_batch_solve.argtypes
         L.orc_load_ref.argtypes = [C.c_char_p]
@@ -261,7 +296,7 @@ def main():
     opt = pkg.Options()
     n_cmd = 8  # controls / gains shipped per MPC update (HKDMPC.cpp:245-248)
 
-    def time_batch(w, steps, warmup, want_e2e):
+    def time_batch(w, steps, warmup, want_e2e, dump_dir=None):
         """Resident and end-to-end timing of one workload on this rank's GPU; returns a dict (times are max over ranks)."""
         B = pkg.MultiPhaseDDPBatch(local_rank)
         B.set_problems(w.schedules, w.schedule_id)
@@ -298,6 +333,8 @@ def main():
         ms_total = sh.max_over_ranks(B.event_elapsed_ms(0, 1), dev)
         info = B.info()
         cnt = B.counters()
+        if dump_dir:
+            dump_outputs(pkg, B, dump_dir)
         out = dict(B=B, ms_total=ms_total, info=info, clocks=clocks, launches=cnt["solve_launches"] + cnt["step_launches"],
                    sweep_stages_per_step=cnt["sweep_stages"] / max(1, steps), kernel_ms=B.last_solve_ms())
         if want_e2e:
@@ -319,7 +356,8 @@ def main():
 
     # ---- weak: args.problems per GPU ----
     w = getattr(wl, args.config)(pkg, args.problems, args.plan, **({"first": rank * args.problems} if args.config == "config3" else {}))
-    t = time_batch(w, args.steps, args.warmup, True)
+    dump_dir = args.dump_outputs and (os.path.join(args.dump_outputs, "rank%d" % rank) if world > 1 else args.dump_outputs)
+    t = time_batch(w, args.steps, args.warmup, True, dump_dir)
     B = t["B"]
     g = sh.gather_stats(sh.local_stats(t["info"], t["sweep_stages_per_step"]), dev)
     tot = sh.reduce_stats(g)

@@ -81,12 +81,19 @@ def _oracle_pair(orc, w, i, tables):
     whole solve measures how strongly THIS problem amplifies rounding noise.  A problem is
     well-posed for parity when both give the same step sequence and agree to 1e-11; the
     non-converging long-flight problems of config 4 are not (SURVEY.md §7.2: report such
-    problems as ill-posed for parity rather than failures)."""
+    problems as ill-posed for parity rather than failures).  Without the compiled reference model
+    the oracle runs on the port, and the FMA-contracted build of the same restatement is the
+    second arithmetic (oracle/parity_check.py)."""
     P = _oracle_problem(orc, w, i, tables)
     s, otr = P.solve()
-    if not orc.ref_available():
-        return P, s, otr, True, 0.0
     gait, k0 = w.keys[w.schedule_id[i]]
+    if not orc.ref_available():
+        import parity_check as pc
+        base, others = pc.oracle_runs(orc, [tables[gait]], [k0], w.x0[i:i + 1], P.n_states, P.n_stages, w.plan,
+                                      k_rows=P.n_stages, variants=("fma",))
+        assert others, "no second arithmetic variant of the oracle to classify problems with"
+        well, sens = pc.classify(base, others)
+        return P, s, otr, bool(well[0]), float(sens[0])
     Q = orc.Problem(tables[gait], k0, w.plan, model=orc.MODEL_PORT)
     Q.x0 = w.x0[i]
     s2, otr2 = Q.solve()

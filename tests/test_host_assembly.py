@@ -66,9 +66,9 @@ def test_window_past_the_table_is_rejected(pkg):
 
 
 def test_text_loader_reproduces_the_fixture(pkg):
-    path = "/root/reference/Reference/Data/trot/quad_reference.csv"
-    if not os.path.exists(path):
-        pytest.skip("reference tree not present")
+    """tests/golden/quad_reference_trot.csv: the first 120 rows of the trot table in the reference's quad_reference.csv
+    format (3 decimals, which every value of the fixture round-trips through exactly)."""
+    path = os.path.join(GOLDEN, "quad_reference_trot.csv")
     S1 = pkg.Schedule(pkg.QuadReference(path), 0, 0.6)
     S2 = pkg.Schedule(pkg.QuadReference(GAIT_PATH("trot")), 0, 0.6)
     for name in ("xr", "ur", "prel_r", "xinit"):
@@ -103,8 +103,7 @@ def test_cpp_shim_compiles_and_fails_loudly_without_gpu(pkg, tmp_path):
     import torch
     if torch.cuda.is_available():
         pytest.skip("a GPU is present; the GPU run of the example is in test_gpu_parity.py")
-    ref = "/root/reference/Reference/Data/trot/quad_reference.csv"
-    r = subprocess.run([exe, ref if os.path.exists(ref) else "/nonexistent"], capture_output=True, text=True)
+    r = subprocess.run([exe, os.path.join(GOLDEN, "quad_reference_trot.csv")], capture_output=True, text=True)
     assert r.returncode != 0 and "error" in r.stderr
 
 
