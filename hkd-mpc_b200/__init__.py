@@ -33,7 +33,14 @@ ARR = dict(Xbar=0, X=1, Defect=3, dX=4, G0=5, Ubar=10, U=11, dU=12, K=20, A=21, 
 
 
 class HsddpError(RuntimeError):
-    pass
+    """A C-ABI call failed; `code` is its HSDDP_ERR_* return value."""
+
+    def __init__(self, msg, code=None):
+        super().__init__(msg)
+        self.code = code
+
+
+ERR_ARG, ERR_CUDA, ERR_UNSUPPORTED, ERR_STATE = -1, -2, -3, -4
 
 
 class Options(C.Structure):
@@ -136,6 +143,8 @@ def lib():
         L.hsddp_batch_reset.argtypes = [vp]
         L.hsddp_batch_mpc_update.argtypes = [vp]
         L.hsddp_batch_last_update_ms.argtypes = [vp, C.POINTER(C.c_float)]
+        L.hsddp_batch_restart_problems.argtypes = [vp, C.c_int, ip, ip, ip, dp, C.POINTER(Options)]
+        L.hsddp_batch_get_schedule_ids.argtypes = [vp, ip]
         for f in ("hsddp_batch_solve", "hsddp_batch_solve_async", "hsddp_batch_compute_cost", "hsddp_batch_lq_approximation",
                   "hsddp_batch_prepare_merit", "hsddp_batch_update_al_params", "hsddp_batch_update_reb_params"):
             getattr(L, f).argtypes = [vp, C.POINTER(Options)]
@@ -192,7 +201,7 @@ def _fp(a):
 
 def _check(rc, what):
     if rc != 0:
-        raise HsddpError(f"{what} failed with code {rc}: {lib().hsddp_last_error().decode()}")
+        raise HsddpError(f"{what} failed with code {rc}: {lib().hsddp_last_error().decode()}", rc)
 
 
 # --------------------------------------------------------------------------
@@ -358,6 +367,25 @@ class MultiPhaseDDPBatch:
     def mpc_update(self):
         """HKDProblem::update for every problem (receding-horizon shift by one MPC step, on the device)."""
         _check(lib().hsddp_batch_mpc_update(self.h), "hsddp_batch_mpc_update")
+
+    def restart(self, problems, gait, window, x0, first_solve=None):
+        """HKDMPCSolver::initialize for some problems of the batch: problem problems[k] restarts on the reference window that
+        starts at sample window[k] of gait gait[k] (index into the gait list of set_problems_from_gaits) from state x0[k], with
+        the cold-start guess and fresh ReB / AL parameters; the other problems keep everything.  first_solve (Options or None):
+        max_AL_iter / max_DDP_iter of the next solve of these problems only.  Call it after mpc_update and
+        set_initial_condition of the tick, before solve."""
+        p = np.ascontiguousarray(problems, np.int32).ravel()
+        g = np.ascontiguousarray(np.broadcast_to(np.asarray(gait, np.int32), p.shape))
+        w = np.ascontiguousarray(np.broadcast_to(np.asarray(window, np.int32), p.shape))
+        x = np.ascontiguousarray(x0, np.float64).reshape(len(p), 24)
+        _check(lib().hsddp_batch_restart_problems(self.h, len(p), _ip(p), _ip(g), _ip(w), _dp(x), None if first_solve is None else C.byref(first_solve)),
+               "hsddp_batch_restart_problems")
+
+    def schedule_ids(self):
+        """Schedule slot of every problem (the index device_schedule takes)."""
+        out = np.zeros(self.n, np.int32)
+        _check(lib().hsddp_batch_get_schedule_ids(self.h, _ip(out)), "hsddp_batch_get_schedule_ids")
+        return out
 
     def last_update_ms(self):
         ms = C.c_float()

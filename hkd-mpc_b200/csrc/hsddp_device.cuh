@@ -113,6 +113,7 @@ struct SolveCtl {
     int iter, iter_ou, iter_in, n_sweeps, n_trials, status;
     int active;  // 1 while the solve is running
     int have_trial;  // 1: trial_cost / trial_feas hold the last compute_cost of this outer iteration's line search
+    int max_al, max_ddp;  // iteration budget of this solve: the options' max_AL_iter / max_DDP_iter or the problem's override
     double cost0, feas0;
     double trial_cost, trial_feas;
 };
@@ -154,6 +155,8 @@ struct BatchPtrs {
     double *ls_X, *ls_Defect, *ls_Xsim, *ls_U, *ls_Ut, *ls_gcon, *ls_hcon, *ls_res;
     int* ls_mail;
     const int* order;                         // persistent kernel: the work queue visits problems in this order (nullptr: by index)
+    const int* budget;                        // [P][2] max_AL_iter, max_DDP_iter of the next solve of a restarted problem, -1: the
+                                              // solve's options (nullptr until a restart sets one, hsddp_batch_restart_problems)
     hsddp_info* info;                         // [P]
     hsddp_iter_record* trace;                 // [P][HSDDP_TRACE_CAP]
     unsigned long long* counters;             // [0] = sum over problems of (backward sweeps x stages)

@@ -12,6 +12,8 @@
 #include <cstring>
 #include <string>
 #include <vector>
+#include <map>
+#include <algorithm>
 #include "hsddp_device.cuh"
 #include "hsddp_sweep.cuh"
 #include "hsddp_sweep_w1.cuh"
@@ -225,7 +227,7 @@ __device__ inline void outer_end_block(Smem& sm) {
         int status = -1;
         if (st.max_tconstr < opt.tconstr_thresh && fabs(st.max_pconstr) < opt.pconstr_thresh && st.feas <= opt.dynamics_feas_thresh) status = HSDDP_STATUS_CONVERGED;
         else if (fabs(st.max_tconstr - st.max_tconstr_prev) < 0.0001 && fabs(st.max_pconstr - st.max_pconstr_prev) < 0.0001 && st.feas <= opt.dynamics_feas_thresh) status = HSDDP_STATUS_STALLED;
-        else if (sm.ctl.iter_ou >= opt.max_AL_iter) status = HSDDP_STATUS_MAX_ITER;
+        else if (sm.ctl.iter_ou >= sm.ctl.max_al) status = HSDDP_STATUS_MAX_ITER;
         __syncthreads();
         if (status >= 0) {
             if (threadIdx.x == 0) { sm.ctl.status = status; sm.ctl.active = 0; }
@@ -233,16 +235,18 @@ __device__ inline void outer_end_block(Smem& sm) {
             return;
         }
         outer_start_block(sm);
-        if (opt.max_DDP_iter > 0) return;  // (an empty inner loop falls straight through to the next outer end)
+        if (sm.ctl.max_ddp > 0) return;  // (an empty inner loop falls straight through to the next outer end)
     }
 }
 
-__device__ inline void solve_begin_block(Smem& sm) {
+__device__ inline void solve_begin_block(Smem& sm, const BatchPtrs& bp) {
     const int tid = threadIdx.x;
     __syncthreads();
     if (tid == 0) {
         SolveCtl c = {};
         c.status = HSDDP_STATUS_MAX_ITER; c.active = 1;
+        c.max_al = sm.opt.max_AL_iter; c.max_ddp = sm.opt.max_DDP_iter;
+        if (bp.budget && bp.budget[2 * sm.pid] >= 0) { c.max_al = bp.budget[2 * sm.pid]; c.max_ddp = bp.budget[2 * sm.pid + 1]; }
         sm.ctl = c;
         sm.st.actual_cost = 0; sm.st.max_pconstr = 0; sm.st.max_pconstr_prev = 0; sm.st.max_tconstr = 0; sm.st.max_tconstr_prev = 0;
     }
@@ -252,13 +256,13 @@ __device__ inline void solve_begin_block(Smem& sm) {
     compute_cost_block(sm);
     if (tid == 0) { sm.ctl.cost0 = sm.st.actual_cost; sm.ctl.feas0 = sm.st.feas; }
     __syncthreads();
-    if (sm.opt.max_AL_iter <= 0) {
+    if (sm.ctl.max_al <= 0) {
         if (tid == 0) sm.ctl.active = 0;
         __syncthreads();
         return;
     }
     outer_start_block(sm);
-    if (sm.opt.max_DDP_iter <= 0) outer_end_block(sm);
+    if (sm.ctl.max_ddp <= 0) outer_end_block(sm);
 }
 
 __device__ inline void iter_prep_block(Smem& sm, const BatchPtrs& bp) {
@@ -337,7 +341,7 @@ __device__ inline void iter_forward_block(Smem& sm, const BatchPtrs& bp) {
         if ((fabs((cost_prev - sm.st.actual_cost) / cost_prev) < opt.cost_thresh) && (sm.st.feas <= opt.dynamics_feas_thresh)) leave_inner = true;  // :358-359
     }
     __syncthreads();
-    if (leave_inner || sm.ctl.iter_in >= opt.max_DDP_iter) outer_end_block(sm);
+    if (leave_inner || sm.ctl.iter_in >= sm.ctl.max_ddp) outer_end_block(sm);
 }
 
 __device__ inline void solve_finish_block(Smem& sm, const BatchPtrs& bp) {
@@ -355,7 +359,7 @@ __device__ inline void solve_finish_block(Smem& sm, const BatchPtrs& bp) {
 
 template <bool CLUSTER_LS = false>
 __device__ inline void solve_block(Smem& sm, const BatchPtrs& bp) {
-    solve_begin_block(sm);
+    solve_begin_block(sm, bp);
     while (sm.ctl.active) {
         iter_prep_block(sm, bp);
         iter_sweep_block(sm, bp);
@@ -496,7 +500,7 @@ __global__ void __launch_bounds__(kThreads, PH == 2 ? HSDDP_MINB_SWEEP : HSDDP_M
     if (threadIdx.x == 0) for (int i = 0; i < 16; ++i) sm.profacc[i] = 0;
     __syncthreads();
 #endif
-    if (PH == PH_BEGIN) solve_begin_block(sm);
+    if (PH == PH_BEGIN) solve_begin_block(sm, bp);
     if (PH == PH_PREP) iter_prep_block(sm, bp);
     if (PH == PH_SWEEP) iter_sweep_block(sm, bp);
     if (PH == PH_FORWARD) {
@@ -657,11 +661,13 @@ __device__ __forceinline__ int ref_index_at(float t, float dt, int sz) {
     return k;
 }
 
-// pass 1: phase tables, one thread per schedule.  status[i] != 0 marks an unusable window.
+// pass 1: phase tables, one thread per schedule.  status[i] != 0 marks an unusable window.  Schedule i goes to slot
+// slot[i] (nullptr: slot i) and may have at most stage_cap stages.
 __global__ void k_build_phase_tables(GaitLib lib, int n_sched, const int* sched_gait, const int* sched_window, float plan, int node_stride,
-                                     DevSchedule* out, int* status, MpcSched* mpc) {
+                                     DevSchedule* out, int* status, MpcSched* mpc, const int* slot, int stage_cap) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n_sched) return;
+    const int si = slot ? slot[i] : i;
     const int gi = sched_gait[i], k0 = sched_window[i];
     const float dtg = lib.dt[gi];
     const int sz = (int)roundf(__fdiv_rn(plan, dtg)) + 1;
@@ -686,7 +692,7 @@ __global__ void k_build_phase_tables(GaitLib lib, int n_sched, const int* sched_
             if (change || approx_geq_f(t, plan)) {
                 if (n_phases >= MAXPH) { st = 2; break; }
                 const int hz = (int)roundf(__fdiv_rn(__fsub_rn(t, phase_start), dt_sim));
-                if (hz < 1 || so + hz > HSDDP_MAX_STAGES) { st = 2; break; }
+                if (hz < 1 || so + hz > stage_cap) { st = 2; break; }
                 d.horizon[n_phases] = hz; d.node_off[n_phases] = no; d.stage_off[n_phases] = so;
                 unsigned cm = 0;
                 for (int l = 0; l < 4; ++l) cm |= (cprev[l] ? 1u : 0u) << l;
@@ -707,11 +713,11 @@ __global__ void k_build_phase_tables(GaitLib lib, int n_sched, const int* sched_
     }
     if (!st && (n_phases < 1 || no > node_stride)) st = 2;
     d.n_phases = n_phases; d.n_stages = so; d.n_nodes = no; d.dt = (double)dt_sim;
-    d.ref_off = (long long)i * node_stride;
-    out[i] = d;
+    d.ref_off = (long long)si * node_stride;
+    out[si] = d;
     status[i] = st;
     m.status = st;
-    if (mpc) mpc[i] = m;
+    if (mpc) mpc[si] = m;
     (void)dt_mpc;
 }
 
@@ -719,11 +725,11 @@ __global__ void k_build_phase_tables(GaitLib lib, int n_sched, const int* sched_
 // contact-after-phase masks (thread of node 0 of each schedule, after every node of that schedule has read them —
 // so the start times are first copied to shared memory by the whole block).
 __global__ void k_build_reference_rows(GaitLib lib, int n_sched, const int* sched_gait, const int* sched_window, float plan, int node_stride,
-                                       DevSchedule* scheds, const int* status, double* xr, double* ur, double* prel, double* xinit) {
+                                       DevSchedule* scheds, const int* status, double* xr, double* ur, double* prel, double* xinit, const int* slot) {
     const int i = blockIdx.x;
     if (i >= n_sched || status[i]) return;
     __shared__ float start_time[MAXPH];
-    DevSchedule& d = scheds[i];
+    DevSchedule& d = scheds[slot ? slot[i] : i];
     const int n_phases = d.n_phases;
     if (threadIdx.x < n_phases) start_time[threadIdx.x] = __uint_as_float(d.nmask[threadIdx.x]);
     __syncthreads();
@@ -792,9 +798,10 @@ __global__ void k_mpc_update_schedules(GaitLib lib, int n_sched, const int* sche
                                        DevSchedule* scheds, MpcSched* mpc, int* err) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n_sched) return;
+    const int gi = sched_gait[i];
+    if (gi < 0) return;  // a free slot (hsddp_batch_restart_problems)
     DevSchedule d = scheds[i];
     MpcSched m = mpc[i];
-    const int gi = sched_gait[i];
     const float dtg = lib.dt[gi];
     const float dt_sim = 0.01f, dt_mpc = 0.01f;
     const int sz = (int)roundf(__fdiv_rn(plan, dtg)) + 1;
@@ -866,7 +873,7 @@ __global__ void k_mpc_update_schedules(GaitLib lib, int n_sched, const int* sche
 __global__ void k_mpc_reference_rows(GaitLib lib, int n_sched, const int* sched_gait, const int* sched_window, float plan,
                                      const DevSchedule* scheds, const MpcSched* mpc, double* xr, double* ur, double* prel) {
     const int i = blockIdx.x;
-    if (i >= n_sched || mpc[i].status) return;
+    if (i >= n_sched || mpc[i].status || sched_gait[i] < 0) return;  // (gait -1: a free slot)
     const DevSchedule& d = scheds[i];
     const MpcSched& m = mpc[i];
     const int gi = sched_gait[i];
@@ -969,6 +976,68 @@ __global__ void __launch_bounds__(kThreads) k_mpc_shift(BatchPtrs bp, const MpcS
     if (tid < 24) Ubar[tid] = 0.0;  // trajectory_ptrs.front()->Ubar[0].setZero(), HKDProblem.cpp:220
 }
 
+// ---------------------------------------------------------------------------
+// HKDMPCSolver::initialize (HKDMPC.cpp:44-69) for a subset of the batch (hsddp_batch_restart_problems).  Launched only after
+// the new schedules have been built and checked, so nothing here can fail.  One block per restarted problem j:
+//   - problem[j] is bound to schedule slot slot[j]; block 0 also writes the slot table of the call: gait / window of every new
+//     slot, gait -1 for every slot no problem uses any more (the receding-horizon update skips those);
+//   - every per-problem array is zeroed over the batch's full row count (what a fresh batch starts from: rows the new schedule
+//     does not have stay zero, and no lq / tq record of the old schedule survives), then the cold start of a new problem;
+//   - the initial state x0[j] and the iteration budget of the next solve (-1: the solve's options).
+// ---------------------------------------------------------------------------
+struct RestartArgs {
+    const int *problem, *slot;           // [n]
+    const int *cslot, *cgait, *cwindow;  // [n_commit]
+    const double* x0;                    // [n][24]
+    int n_commit, max_al, max_ddp;
+    int *sched_gait, *sched_window;
+};
+
+__device__ __forceinline__ void zero_rows(double* p, size_t n) {
+    for (size_t e = threadIdx.x; e < n; e += kThreads) p[e] = 0.0;
+}
+
+__global__ void __launch_bounds__(kThreads) k_restart(BatchPtrs bp, RestartArgs ra) {
+    __shared__ Smem sm;
+    const int j = blockIdx.x, pid = ra.problem[j];
+    if (blockIdx.x == 0)
+        for (int e = threadIdx.x; e < ra.n_commit; e += kThreads) { ra.sched_gait[ra.cslot[e]] = ra.cgait[e]; ra.sched_window[ra.cslot[e]] = ra.cwindow[e]; }
+    if (threadIdx.x == 0) const_cast<int*>(bp.sched_id)[pid] = ra.slot[j];
+    const size_t P = pid, SN = (size_t)bp.max_nodes * 24, SS = (size_t)bp.max_stages * 24;
+    zero_rows(bp.Xbar + P * SN, SN); zero_rows(bp.X + P * SN, SN); zero_rows(bp.Xsim_t + P * SN, SN);
+    zero_rows(bp.Defect + P * SN, SN); zero_rows(bp.dX + P * SN, SN);
+    zero_rows(bp.Ubar + P * SS, SS); zero_rows(bp.U + P * SS, SS); zero_rows(bp.U_t + P * SS, SS); zero_rows(bp.dU + P * SS, SS);
+    zero_rows(bp.KdX + P * bp.max_stages * 12, (size_t)bp.max_stages * 12);
+    zero_rows(bp.K + P * bp.max_stages * 288, (size_t)bp.max_stages * 288);
+    zero_rows(bp.lq + P * bp.max_stages * CR_STRIDE, (size_t)bp.max_stages * CR_STRIDE);
+    zero_rows(bp.tq + P * MAXPH * TQ_STRIDE, (size_t)MAXPH * TQ_STRIDE);
+    zero_rows(bp.gcon + P * bp.max_stages * 20, (size_t)bp.max_stages * 20);
+    zero_rows(bp.reb + P * bp.max_stages * 40, (size_t)bp.max_stages * 40);
+    zero_rows(bp.hcon + P * MAXPH * 4, (size_t)MAXPH * 4);
+    zero_rows(bp.al + P * MAXPH * 16, (size_t)MAXPH * 16);
+    zero_rows(bp.g0h0 + P * 600, 600);
+    zero_rows((double*)(bp.trace + P * HSDDP_TRACE_CAP), HSDDP_TRACE_CAP * sizeof(hsddp_iter_record) / sizeof(double));
+    if (bp.ls_X) {  // trial arrays of the concurrent line search (small batches)
+        const size_t Q = P * 4;
+        zero_rows(bp.ls_X + Q * SN, 4 * SN); zero_rows(bp.ls_Defect + Q * SN, 4 * SN); zero_rows(bp.ls_Xsim + Q * SN, 4 * SN);
+        zero_rows(bp.ls_U + Q * SS, 4 * SS); zero_rows(bp.ls_Ut + Q * SS, 4 * SS);
+        zero_rows(bp.ls_gcon + Q * bp.max_stages * 20, 4 * (size_t)bp.max_stages * 20);
+        zero_rows(bp.ls_hcon + Q * MAXPH * 4, 4 * (size_t)MAXPH * 4);
+        zero_rows(bp.ls_res + Q * 8, 32);
+        if (threadIdx.x == 0) bp.ls_mail[pid] = 0;
+    }
+    if (threadIdx.x == 0) {
+        bp.info[pid] = hsddp_info{};
+        bp.ctl[pid] = SolveCtl{};
+        if (bp.budget) { int* q = const_cast<int*>(bp.budget) + 2 * pid; q[0] = ra.max_al; q[1] = ra.max_ddp; }
+    }
+    if (threadIdx.x < 24) bp.x0[P * 24 + threadIdx.x] = ra.x0[24 * (size_t)j + threadIdx.x];
+    __syncthreads();
+    bind_problem(sm, bp, pid);
+    cold_start_block(sm);
+    if (threadIdx.x == 0) bp.state[pid] = sm.st;
+}
+
 // FP64 throughput probes (roofline denominators measured on the box)
 __global__ void k_dfma_probe(double* out, int iters) {
     double a0 = threadIdx.x * 1e-3, a1 = a0 + 1, a2 = a0 + 2, a3 = a0 + 3, a4 = a0 + 4, a5 = a0 + 5, a6 = a0 + 6, a7 = a0 + 7;
@@ -1060,6 +1129,17 @@ struct hsddp_batch {
     int node_stride = 0, n_sched = 0;
     bool h_sched_stale = false;
     cudaEvent_t ev_u0 = nullptr, ev_u1 = nullptr;
+    int n_gaits = 0;
+    // problem restarts (hsddp_batch_restart_problems).  Nothing below is allocated before the first restart.  n_sched counts
+    // the schedule SLOTS; a slot is free when no problem uses it (gait -1 on the device, listed in slot_free).
+    std::vector<int> slot_refs;    // problems per slot (empty until the first restart)
+    std::vector<int> slot_free;    // free slots, marked on the device
+    int* d_restart = nullptr;      // per-call argument lists (ints), d_restart_cap of them
+    double* d_restart_x0 = nullptr;
+    size_t d_restart_cap = 0, d_restart_x0_cap = 0;
+    int* d_budget = nullptr;       // BatchPtrs::budget
+    long long budget_rounds = -1;  // largest max_AL_iter x max_DDP_iter among the pending overrides (-1: none pending)
+    bool slots_marked = false;     // the slots no problem used are on the free list (done by the first restart)
 };
 
 namespace {
@@ -1090,6 +1170,24 @@ int dalloc(hsddp_batch* b, T** p, size_t n) {
     return HSDDP_OK;
 }
 
+// device scratch of at least `n` elements, kept in `allocs` (freed with the problem set)
+template <class T>
+int scratch(hsddp_batch* b, T** p, size_t* cap, size_t n) {
+    if (*cap >= n) return HSDDP_OK;
+    void* q = nullptr;
+    CK(cudaMalloc(&q, n * sizeof(T)));
+    if (*p) {
+        CK(cudaStreamSynchronize(b->stream));
+        for (void*& a : b->allocs)
+            if (a == (void*)*p) a = q;
+        cudaFree(*p);
+    } else {
+        b->allocs.push_back(q);
+    }
+    *p = (T*)q; *cap = n;
+    return HSDDP_OK;
+}
+
 void free_problem_allocs(hsddp_batch* b) {
     for (void* p : b->allocs) cudaFree(p);
     b->allocs.clear();
@@ -1097,6 +1195,10 @@ void free_problem_allocs(hsddp_batch* b) {
     b->has_problems = false;
     b->mpc_ready = false;
     b->h_sched_stale = false;
+    b->slot_refs.clear(); b->slot_free.clear();
+    b->d_restart = nullptr; b->d_restart_x0 = nullptr; b->d_restart_cap = b->d_restart_x0_cap = 0;
+    b->d_budget = nullptr; b->budget_rounds = -1;
+    b->slots_marked = false;
 }
 
 hsddp_options default_options() {
@@ -1106,6 +1208,13 @@ hsddp_options default_options() {
     o.max_DDP_iter = 10; o.max_AL_iter = 5; o.cost_thresh = 1e-3; o.tconstr_thresh = 1e-3; o.pconstr_thresh = 1e-3;
     o.dynamics_feas_thresh = 1e-3; o.merit_scale = 0.2; o.merit_offset = 1e2; o.AL_active = 1; o.ReB_active = 1; o.MS = 1;
     return o;
+}
+
+// the iteration budget rules of check_opt
+const char* check_budget(int max_AL_iter, int max_DDP_iter) {
+    if (max_DDP_iter < 0 || max_AL_iter < 0) return "max_DDP_iter / max_AL_iter must be >= 0";
+    if ((long long)max_DDP_iter * (long long)max_AL_iter > 1000000LL) return "max_DDP_iter x max_AL_iter exceeds 1e6";
+    return nullptr;
 }
 
 int check_opt(const hsddp_options* opt) {
@@ -1120,8 +1229,7 @@ int check_opt(const hsddp_options* opt) {
     else if (!fin(opt->gamma) || !fin(opt->update_penalty) || !fin(opt->update_relax) || !fin(opt->update_ReB)) bad = "gamma / update_penalty / update_relax / update_ReB must be finite";
     else if (!fin(opt->cost_thresh) || !fin(opt->tconstr_thresh) || !fin(opt->pconstr_thresh) || !fin(opt->dynamics_feas_thresh)) bad = "thresholds must be finite";
     else if (!fin(opt->merit_scale) || opt->merit_scale == 1.0 || !fin(opt->merit_offset)) bad = "merit_scale must be finite and != 1, merit_offset finite";
-    else if (opt->max_DDP_iter < 0 || opt->max_AL_iter < 0) bad = "max_DDP_iter / max_AL_iter must be >= 0";
-    else if ((long long)opt->max_DDP_iter * (long long)opt->max_AL_iter > 1000000LL) bad = "max_DDP_iter x max_AL_iter exceeds 1e6";
+    else bad = check_budget(opt->max_AL_iter, opt->max_DDP_iter);
     if (bad) { g_last_error = std::string("invalid hsddp_options: ") + bad; return HSDDP_ERR_ARG; }
     return HSDDP_OK;
 }
@@ -1412,8 +1520,10 @@ int hsddp_batch_set_problems_from_gaits(hsddp_batch* b, int n_gaits, const int32
     MpcSched* d_mpc; int* d_err;
     if ((rc = dalloc(b, &d_mpc, (size_t)n_schedules)) || (rc = dalloc(b, &d_err, (size_t)4))) return rc;
     CK(cudaMemsetAsync(d_err, 0, 4 * sizeof(int), b->stream));
-    k_build_phase_tables<<<(n_schedules + 127) / 128, 128, 0, b->stream>>>(lib, n_schedules, d_sg, d_sw, plan_duration, node_stride, d_sched, d_status, d_mpc);
-    k_build_reference_rows<<<n_schedules, 128, 0, b->stream>>>(lib, n_schedules, d_sg, d_sw, plan_duration, node_stride, d_sched, d_status, d_xr, d_ur, d_prel, d_xinit);
+    k_build_phase_tables<<<(n_schedules + 127) / 128, 128, 0, b->stream>>>(lib, n_schedules, d_sg, d_sw, plan_duration, node_stride, d_sched, d_status, d_mpc,
+                                                                           nullptr, HSDDP_MAX_STAGES);
+    k_build_reference_rows<<<n_schedules, 128, 0, b->stream>>>(lib, n_schedules, d_sg, d_sw, plan_duration, node_stride, d_sched, d_status, d_xr, d_ur, d_prel, d_xinit,
+                                                               nullptr);
     CK(cudaGetLastError());
     b->n_step_launches += 2;
     // the host keeps the phase tables too (dense gain / Jacobian getters, workspace sizing)
@@ -1436,7 +1546,7 @@ int hsddp_batch_set_problems_from_gaits(hsddp_batch* b, int n_gaits, const int32
     if ((rc = alloc_workspace(b, n_problems, max_stages, max_nodes))) return rc;
     b->has_problems = true;
     b->lib = lib; b->d_sched_gait = d_sg; b->d_sched_window = d_sw; b->d_mpc = d_mpc; b->d_mpc_err = d_err;
-    b->plan = plan_duration; b->node_stride = node_stride; b->n_sched = n_schedules; b->mpc_ready = true;
+    b->plan = plan_duration; b->node_stride = node_stride; b->n_sched = n_schedules; b->n_gaits = n_gaits; b->mpc_ready = true;
     return hsddp_batch_reset(b);
     });
 }
@@ -1509,6 +1619,152 @@ int hsddp_batch_get_schedule(hsddp_batch* b, int i, int32_t* n_phases, int32_t* 
     if (xinit) CK(cudaMemcpy(xinit, b->bp.xinit + o * 24, nn * 24 * sizeof(double), cudaMemcpyDeviceToHost));
     return HSDDP_OK;
     });
+}
+
+// `add` more schedule slots: the slot arrays are reallocated and the existing slots copied device to device (ref_off stays
+// valid: slot s keeps reference rows [s * node_stride, (s + 1) * node_stride)).  The new slots are free.
+static int grow_slots(hsddp_batch* b, int add) {
+    const size_t cap = (size_t)b->n_sched, ncap = cap + (size_t)add, rows = (size_t)b->node_stride;
+    BatchPtrs& bp = b->bp;
+    void* old[8] = {(void*)bp.sched, (void*)b->d_mpc, (void*)b->d_sched_gait, (void*)b->d_sched_window,
+                    (void*)bp.xr, (void*)bp.ur, (void*)bp.prel, (void*)bp.xinit};
+    const size_t elem[8] = {sizeof(DevSchedule), sizeof(MpcSched), sizeof(int), sizeof(int), 24 * rows * sizeof(double),
+                            24 * rows * sizeof(double), 12 * rows * sizeof(double), 24 * rows * sizeof(double)};
+    void* nw[8] = {};
+    for (int a = 0; a < 8; ++a) {
+        const cudaError_t e = cudaMalloc(&nw[a], ncap * elem[a]);
+        if (e != cudaSuccess) {
+            for (int q = 0; q < a; ++q) cudaFree(nw[q]);
+            g_last_error = std::string("growing the schedule slots: ") + cudaGetErrorString(e);
+            return HSDDP_ERR_CUDA;
+        }
+    }
+    for (int a = 0; a < 8; ++a) {
+        CK(cudaMemcpyAsync(nw[a], old[a], cap * elem[a], cudaMemcpyDeviceToDevice, b->stream));
+        CK(cudaMemsetAsync((char*)nw[a] + cap * elem[a], a == 2 ? 0xff : 0, (ncap - cap) * elem[a], b->stream));  // (gait -1: free)
+    }
+    CK(cudaStreamSynchronize(b->stream));
+    for (int a = 0; a < 8; ++a) {
+        for (void*& p : b->allocs)
+            if (p == old[a]) p = nw[a];
+        cudaFree(old[a]);
+    }
+    bp.sched = (DevSchedule*)nw[0]; b->d_mpc = (MpcSched*)nw[1]; b->d_sched_gait = (int*)nw[2]; b->d_sched_window = (int*)nw[3];
+    bp.xr = (double*)nw[4]; bp.ur = (double*)nw[5]; bp.prel = (double*)nw[6]; bp.xinit = (double*)nw[7];
+    b->n_sched = (int)ncap;
+    b->slot_refs.resize(ncap, 0);
+    b->h_sched.resize(ncap);
+    b->h_sched_stale = true;
+    for (size_t s = ncap; s-- > cap;) b->slot_free.push_back((int)s);  // (taken from the back: lowest index first)
+    return HSDDP_OK;
+}
+
+int hsddp_batch_restart_problems(hsddp_batch* b, int n, const int32_t* problem, const int32_t* gait, const int32_t* window,
+                                 const double* x0, const hsddp_options* first_solve) {
+    return guarded([&]() -> int {
+    if (!b) return HSDDP_ERR_ARG;
+    if (!b->has_problems) { g_last_error = "no problems set"; return HSDDP_ERR_STATE; }
+    if (!b->mpc_ready) { g_last_error = "hsddp_batch_restart_problems needs the gait library on the device: set the problems with hsddp_batch_set_problems_from_gaits"; return HSDDP_ERR_STATE; }
+    const int P = b->bp.n_problems;
+    if (n <= 0 || n > P || !problem || !gait || !window || !x0) { g_last_error = "restart: n must be in [1, n_problems] and every list given"; return HSDDP_ERR_ARG; }
+    if (first_solve)
+        if (const char* bad = check_budget(first_solve->max_AL_iter, first_solve->max_DDP_iter)) { g_last_error = std::string("invalid first_solve: ") + bad; return HSDDP_ERR_ARG; }
+    std::vector<char> seen(P, 0);
+    for (int k = 0; k < n; ++k) {
+        if (problem[k] < 0 || problem[k] >= P) { g_last_error = "restart: problem index out of range"; return HSDDP_ERR_ARG; }
+        if (seen[problem[k]]) { g_last_error = "restart: repeated problem index"; return HSDDP_ERR_ARG; }
+        seen[problem[k]] = 1;
+        if (gait[k] < 0 || gait[k] >= b->n_gaits) { g_last_error = "restart: unknown gait"; return HSDDP_ERR_ARG; }
+        if (window[k] < 0) { g_last_error = "restart: window does not fit the gait table"; return HSDDP_ERR_ARG; }
+    }
+    CK(cudaSetDevice(b->device));
+    if (b->slot_refs.empty()) {
+        b->slot_refs.assign(b->n_sched, 0);
+        for (int s : b->h_sched_id) b->slot_refs[s]++;
+    }
+    int rc;
+    if (first_solve && !b->d_budget) {
+        if ((rc = dalloc(b, &b->d_budget, (size_t)2 * P))) return rc;
+        CK(cudaMemsetAsync(b->d_budget, 0xff, sizeof(int) * 2 * P, b->stream));
+        b->bp.budget = b->d_budget;
+    }
+    // the call's distinct (gait, window) pairs, one new slot each
+    std::map<std::pair<int, int>, int> pair_index;
+    std::vector<int> bgait, bwin, pair_of(n);
+    for (int k = 0; k < n; ++k) {
+        auto it = pair_index.emplace(std::make_pair((int)gait[k], (int)window[k]), (int)bgait.size());
+        if (it.second) { bgait.push_back(gait[k]); bwin.push_back(window[k]); }
+        pair_of[k] = it.first->second;
+    }
+    const int m = (int)bgait.size();
+    if ((int)b->slot_free.size() < m) {
+        // grow by half the capacity at least (a growth copies every slot), but never beyond the n_problems + n slots a call can
+        // need: at most n_problems are referenced, plus the m <= n being built
+        const int need = m - (int)b->slot_free.size();
+        const int add = std::max(need, std::min(b->n_sched / 2, P + n - b->n_sched));
+        if ((rc = grow_slots(b, add))) return rc;
+    }
+    // slot bookkeeping after the call (applied only once the build has succeeded)
+    std::vector<int> free_after = b->slot_free, bslot(m), refs = b->slot_refs;
+    for (int j = 0; j < m; ++j) { bslot[j] = free_after.back(); free_after.pop_back(); }
+    for (int k = 0; k < n; ++k) { refs[b->h_sched_id[problem[k]]]--; refs[bslot[pair_of[k]]]++; }
+    std::vector<char> on_free(b->n_sched, 0);
+    for (int s : free_after) on_free[s] = 1;
+    std::vector<int> freed;
+    auto release = [&](int s) { if (refs[s] == 0 && !on_free[s]) { on_free[s] = 1; freed.push_back(s); } };
+    if (!b->slots_marked) for (int s = 0; s < b->n_sched; ++s) release(s);  // (also the slots no problem used from the start)
+    else for (int k = 0; k < n; ++k) release(b->h_sched_id[problem[k]]);
+    const int c = m + (int)freed.size();
+    // argument lists: problem[n] slot[n] | gait[m] window[m] slot[m] status[m] | commit slot[c] gait[c] window[c]
+    std::vector<int> h(2 * (size_t)n + 4 * (size_t)m + 3 * (size_t)c);
+    int* hp = h.data();
+    int *a_prob = hp, *a_slot = hp + n, *a_bg = hp + 2 * n, *a_bw = a_bg + m, *a_bs = a_bw + m, *a_st = a_bs + m;
+    int *a_cs = a_st + m, *a_cg = a_cs + c, *a_cw = a_cg + c;
+    for (int k = 0; k < n; ++k) { a_prob[k] = problem[k]; a_slot[k] = bslot[pair_of[k]]; }
+    for (int j = 0; j < m; ++j) { a_bg[j] = bgait[j]; a_bw[j] = bwin[j]; a_bs[j] = bslot[j]; a_st[j] = 0; a_cs[j] = bslot[j]; a_cg[j] = bgait[j]; a_cw[j] = bwin[j]; }
+    for (int j = m; j < c; ++j) { a_cs[j] = freed[j - m]; a_cg[j] = -1; a_cw[j] = 0; }
+    if ((rc = scratch(b, &b->d_restart, &b->d_restart_cap, h.size())) || (rc = scratch(b, &b->d_restart_x0, &b->d_restart_x0_cap, (size_t)n * 24))) return rc;
+    int* d = b->d_restart;
+    CK(cudaMemcpyAsync(d, h.data(), h.size() * sizeof(int), cudaMemcpyHostToDevice, b->stream));
+    CK(cudaMemcpyAsync(b->d_restart_x0, x0, (size_t)n * 24 * sizeof(double), cudaMemcpyHostToDevice, b->stream));
+    // build into the free slots, then one host synchronise for the build status
+    const int *d_bg = d + 2 * n, *d_bw = d_bg + m, *d_bs = d_bw + m;
+    int* d_st = const_cast<int*>(d_bs + m);
+    DevSchedule* d_sched = const_cast<DevSchedule*>(b->bp.sched);
+    k_build_phase_tables<<<(m + 127) / 128, 128, 0, b->stream>>>(b->lib, m, d_bg, d_bw, b->plan, b->node_stride, d_sched, d_st, b->d_mpc, d_bs,
+                                                                 b->bp.max_stages);
+    k_build_reference_rows<<<m, 128, 0, b->stream>>>(b->lib, m, d_bg, d_bw, b->plan, b->node_stride, d_sched, d_st, const_cast<double*>(b->bp.xr),
+                                                     const_cast<double*>(b->bp.ur), const_cast<double*>(b->bp.prel), const_cast<double*>(b->bp.xinit), d_bs);
+    CK(cudaGetLastError());
+    b->n_step_launches += 2;
+    CK(cudaMemcpyAsync(a_st, d_st, sizeof(int) * m, cudaMemcpyDeviceToHost, b->stream));
+    CK(cudaStreamSynchronize(b->stream));
+    for (int j = 0; j < m; ++j) {
+        if (a_st[j] == 1) { g_last_error = "restart: window does not fit the gait table"; return HSDDP_ERR_ARG; }
+        if (a_st[j]) { g_last_error = "restart: schedule exceeds HSDDP_MAX_PHASES / the batch's node capacity"; return HSDDP_ERR_UNSUPPORTED; }
+    }
+    // commit
+    b->slot_refs.swap(refs);
+    for (int s : freed) free_after.push_back(s);
+    b->slot_free.swap(free_after);
+    for (int k = 0; k < n; ++k) b->h_sched_id[problem[k]] = bslot[pair_of[k]];
+    b->h_sched_stale = true;
+    b->slots_marked = true;
+    RestartArgs ra{d, d + n, d_st + m, d_st + m + c, d_st + m + 2 * c, b->d_restart_x0, c,
+                   first_solve ? first_solve->max_AL_iter : -1, first_solve ? first_solve->max_DDP_iter : -1, b->d_sched_gait, b->d_sched_window};
+    k_restart<<<n, kThreads, 0, b->stream>>>(b->bp, ra);
+    CK(cudaGetLastError());
+    b->n_step_launches++;
+    if (first_solve) b->budget_rounds = std::max(b->budget_rounds, (long long)first_solve->max_AL_iter * first_solve->max_DDP_iter);
+    return HSDDP_OK;
+    });
+}
+
+int hsddp_batch_get_schedule_ids(hsddp_batch* b, int32_t* out) {
+    if (!b || !out) return HSDDP_ERR_ARG;
+    if (!b->has_problems) { g_last_error = "no problems set"; return HSDDP_ERR_STATE; }
+    std::copy(b->h_sched_id.begin(), b->h_sched_id.end(), out);
+    return HSDDP_OK;
 }
 
 int hsddp_batch_set_initial_condition(hsddp_batch* b, const double* x0) {
@@ -1588,7 +1844,8 @@ static int solve_phased(hsddp_batch* b, const hsddp_options& o, bool hybrid) {
     CK(cudaMemsetAsync(b->d_count, 0, 2 * hsddp_batch::kMaxGroups * sizeof(int), b->stream));
     k_iota<<<(P + 255) / 256, 256, 0, b->stream>>>(b->d_active[0], P);
     CK(cudaEventRecord(b->ev_fork, b->stream));
-    const int all_rounds = (int)std::min<long long>((long long)std::max(0, o.max_AL_iter) * (long long)std::max(0, o.max_DDP_iter), 1000000LL);
+    // (restarted problems may have a larger budget for this solve: BatchPtrs::budget)
+    const int all_rounds = (int)std::min<long long>(std::max((long long)std::max(0, o.max_AL_iter) * (long long)std::max(0, o.max_DDP_iter), b->budget_rounds), 1000000LL);
     const int rounds = hybrid ? std::min(all_rounds, std::max(0, b->hybrid_rounds)) : all_rounds;
     ResumeLists rl{};
     rl.n = 0;
@@ -1645,6 +1902,14 @@ int hsddp_batch_set_solve_mode(hsddp_batch* b, int mode) {
     return HSDDP_OK;
 }
 
+// the per-problem budgets of restarted problems apply to one solve: cleared on the stream once it is queued
+static int consume_budget(hsddp_batch* b) {
+    if (b->budget_rounds < 0) return HSDDP_OK;
+    CK(cudaMemsetAsync(b->d_budget, 0xff, sizeof(int) * 2 * b->bp.n_problems, b->stream));
+    b->budget_rounds = -1;
+    return HSDDP_OK;
+}
+
 int hsddp_batch_solve_async(hsddp_batch* b, const hsddp_options* opt) {
     if (!b || !b->has_problems) { g_last_error = "no problems set"; return HSDDP_ERR_STATE; }
     int rc = check_opt(opt);
@@ -1658,8 +1923,11 @@ int hsddp_batch_solve_async(hsddp_batch* b, const hsddp_options* opt) {
     // (measured on config 3, persistent vs phased, ms, final code of round 2: 2,048 problems 57 vs 69, 4,096: 98 vs 100,
     // 5,120: ~121 vs 117, 6,144: 145 vs 135, 8,192: 199 vs 163 -- profiles/r02an_*: the switch is at 5.5 waves of blocks, 4,884 problems)
     const bool phased = b->solve_mode == 2 || (b->solve_mode == 0 && 2 * b->bp.n_problems >= 11 * b->n_sm * b->blocks_per_sm);
-    if (phased) return solve_phased(b, o, false);
-    if (b->solve_mode == 3) return solve_phased(b, o, true);
+    if (phased || b->solve_mode == 3) {
+        rc = solve_phased(b, o, !phased);
+        if (rc == HSDDP_OK) rc = consume_budget(b);
+        return rc;
+    }
     CK(cudaMemsetAsync(b->bp.work_counter, 0, sizeof(int), b->stream));
     CK(cudaEventRecord(b->ev0, b->stream));
     if (b->cluster_ls && b->bp.ls_mail && b->bp.n_problems <= hsddp_batch::kClusterLsMax && o.MS) {
@@ -1675,6 +1943,7 @@ int hsddp_batch_solve_async(hsddp_batch* b, const hsddp_options* opt) {
     CK(cudaGetLastError());
     b->n_solve_launches++;
     CK(cudaEventRecord(b->ev1, b->stream));
+    if ((rc = consume_budget(b))) return rc;
     if (b->use_order && b->bp.n_problems > 2 * b->n_sm) {  // (after the timed region of last_solve_ms: ~10 us, part of every bench step)
         k_order_by_iterations<<<1, 256, 0, b->stream>>>(b->bp.info, b->bp.n_problems, b->d_order);
         CK(cudaGetLastError());

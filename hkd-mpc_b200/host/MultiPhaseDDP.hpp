@@ -125,6 +125,21 @@ public:
     }
     // HKDProblem::update (HKDProblem.cpp:117-222) for every problem: the receding-horizon shift before an MPC re-solve
     void update() { check(hsddp_batch_mpc_update(b_), "hsddp_batch_mpc_update"); }
+    // HKDMPCSolver::initialize (HKDMPC.cpp:44-69) for the listed problems only: new reference window (gait, window start),
+    // cold-start guess, fresh ReB / AL parameters, x0 (24 doubles per listed problem); first_solve (nullable) sets
+    // max_AL_iter / max_DDP_iter of their next solve.  The other problems keep their warm state.
+    void restart_problems(const std::vector<int32_t>& problem, const std::vector<int32_t>& gait, const std::vector<int32_t>& window,
+                          const std::vector<double>& x0, const HSDDP_OPTION* first_solve = nullptr) {
+        if (gait.size() != problem.size() || window.size() != problem.size() || x0.size() != 24 * problem.size())
+            throw std::invalid_argument("restart_problems: one gait, one window and 24 doubles of x0 per problem");
+        check(hsddp_batch_restart_problems(b_, (int)problem.size(), problem.data(), gait.data(), window.data(), x0.data(), first_solve),
+              "hsddp_batch_restart_problems");
+    }
+    std::vector<int32_t> get_schedule_ids() {
+        std::vector<int32_t> v(n_);
+        check(hsddp_batch_get_schedule_ids(b_, v.data()), "hsddp_batch_get_schedule_ids");
+        return v;
+    }
     void set_initial_condition(const std::vector<double>& x0) {
         if ((int)x0.size() != 24 * n_) throw std::invalid_argument("x0 must hold 24 doubles per problem");
         check(hsddp_batch_set_initial_condition(b_, x0.data()), "hsddp_batch_set_initial_condition");
@@ -238,6 +253,30 @@ public:
         }
     }
     void reset() { for (auto& p : parts_) p->reset(); }
+    // restart_problems with GLOBAL problem indices: each listed problem goes to the device whose shard holds it.  The indices
+    // are checked for all devices first; a device that refuses its part throws after the devices before it have restarted theirs.
+    void restart_problems(const std::vector<int32_t>& problem, const std::vector<int32_t>& gait, const std::vector<int32_t>& window,
+                          const std::vector<double>& x0, const HSDDP_OPTION* first_solve = nullptr) {
+        if (gait.size() != problem.size() || window.size() != problem.size() || x0.size() != 24 * problem.size())
+            throw std::invalid_argument("restart_problems: one gait, one window and 24 doubles of x0 per problem");
+        std::vector<char> seen(n_, 0);
+        for (int32_t p : problem) {
+            if (p < 0 || p >= n_ || seen[p]) throw std::invalid_argument("restart_problems: problem index out of range or repeated");
+            seen[p] = 1;
+        }
+        for (int g = 0; g < n_devices(); ++g) {
+            int lo, hi;
+            shard_range(n_, g, n_devices(), lo, hi);
+            std::vector<int32_t> lp, lg, lw;
+            std::vector<double> lx;
+            for (size_t k = 0; k < problem.size(); ++k) {
+                if (problem[k] < lo || problem[k] >= hi) continue;
+                lp.push_back(problem[k] - lo); lg.push_back(gait[k]); lw.push_back(window[k]);
+                lx.insert(lx.end(), x0.begin() + 24 * k, x0.begin() + 24 * (k + 1));
+            }
+            if (!lp.empty()) parts_[g]->restart_problems(lp, lg, lw, lx, first_solve);
+        }
+    }
     void solve(HSDDP_OPTION option) {
         for (auto& p : parts_) p->solve_async(option);
         for (auto& p : parts_) p->sync();

@@ -181,6 +181,24 @@ int hsddp_batch_mpc_update(hsddp_batch* b);
 /* milliseconds of the last update's kernels (CUDA events) */
 int hsddp_batch_last_update_ms(hsddp_batch* b, float* ms);
 
+/* HKDMPCSolver::initialize (HKDMPC/HKDMPC.cpp:44-69) for a SUBSET of the batch: problem[k] is re-targeted to the reference
+ * window that starts at sample window[k] of gait gait[k] (index into the gait library of hsddp_batch_set_problems_from_gaits),
+ * gets the cold-start guess, fresh ReB / AL parameters and initial state x0[k] ([n][24], host), as a new problem would.
+ * The other problems are untouched.  first_solve (nullable): max_AL_iter / max_DDP_iter of the NEXT solve for these
+ * problems only (e.g. 5 x 10 while the batch ticks at 2 x 1); its other fields are ignored.
+ * Needs the gait library on the device (HSDDP_ERR_STATE otherwise).  HSDDP_ERR_ARG for out-of-range or repeated problem
+ * indices, an unknown gait, a window that does not fit its table, or an invalid budget; HSDDP_ERR_UNSUPPORTED for a
+ * schedule beyond HSDDP_MAX_PHASES / the batch's node capacity.  On any error nothing has changed.
+ * A restarted problem gets a schedule slot of its own (problems restarted to the same gait and window in one call share
+ * one); slots no problem uses any more are reused, so a handle never holds more than n_problems + n slots
+ * (or the schedule count it was set with, if larger).
+ * In an MPC tick: hsddp_batch_mpc_update, hsddp_batch_set_initial_condition, then this (the restarted problems start at their
+ * new window after this tick's shift; x0 here overrides the state just set), then hsddp_batch_solve. */
+int hsddp_batch_restart_problems(hsddp_batch* b, int n, const int32_t* problem, const int32_t* gait, const int32_t* window,
+                                 const double* x0, const hsddp_options* first_solve);
+/* schedule index of every problem ([n_problems]); pass it to hsddp_batch_get_schedule */
+int hsddp_batch_get_schedule_ids(hsddp_batch* b, int32_t* out);
+
 /* MultiPhaseDDP::solve(HSDDP_OPTION) (MultiPhaseDDP.cpp:232-428) for every problem:
  * one persistent kernel, one thread block per problem, iteration control on the device. */
 int hsddp_batch_solve(hsddp_batch* b, const hsddp_options* opt);
