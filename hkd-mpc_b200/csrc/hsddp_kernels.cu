@@ -981,21 +981,21 @@ __global__ void __launch_bounds__(kThreads) k_mpc_shift(BatchPtrs bp, const MpcS
 // the new schedules have been built and checked, so nothing here can fail.  One block per restarted problem j:
 //   - problem[j] is bound to schedule slot slot[j]; block 0 also writes the slot table of the call: gait / window of every new
 //     slot, gait -1 for every slot no problem uses any more (the receding-horizon update skips those);
-//   - every per-problem array is zeroed over the batch's full row count (what a fresh batch starts from: rows the new schedule
-//     does not have stay zero, and no lq / tq record of the old schedule survives), then the cold start of a new problem;
+//   - the workspace arrays marked WS_RESTART are zeroed over the batch's full row count (what a fresh batch starts from: rows
+//     the new schedule does not have stay zero, and no lq / tq record of the old schedule survives), info / ctl are reset,
+//     then the cold start of a new problem;
 //   - the initial state x0[j] and the iteration budget of the next solve (-1: the solve's options).
 // ---------------------------------------------------------------------------
+constexpr int kRestartClearMax = 32;
 struct RestartArgs {
     const int *problem, *slot;           // [n]
     const int *cslot, *cgait, *cwindow;  // [n_commit]
     const double* x0;                    // [n][24]
     int n_commit, max_al, max_ddp;
     int *sched_gait, *sched_window;
+    int n_clear;
+    struct { unsigned* base; size_t words; } clear[kRestartClearMax];  // arrays to zero: base, 4-byte words per problem
 };
-
-__device__ __forceinline__ void zero_rows(double* p, size_t n) {
-    for (size_t e = threadIdx.x; e < n; e += kThreads) p[e] = 0.0;
-}
 
 __global__ void __launch_bounds__(kThreads) k_restart(BatchPtrs bp, RestartArgs ra) {
     __shared__ Smem sm;
@@ -1003,28 +1003,10 @@ __global__ void __launch_bounds__(kThreads) k_restart(BatchPtrs bp, RestartArgs 
     if (blockIdx.x == 0)
         for (int e = threadIdx.x; e < ra.n_commit; e += kThreads) { ra.sched_gait[ra.cslot[e]] = ra.cgait[e]; ra.sched_window[ra.cslot[e]] = ra.cwindow[e]; }
     if (threadIdx.x == 0) const_cast<int*>(bp.sched_id)[pid] = ra.slot[j];
-    const size_t P = pid, SN = (size_t)bp.max_nodes * 24, SS = (size_t)bp.max_stages * 24;
-    zero_rows(bp.Xbar + P * SN, SN); zero_rows(bp.X + P * SN, SN); zero_rows(bp.Xsim_t + P * SN, SN);
-    zero_rows(bp.Defect + P * SN, SN); zero_rows(bp.dX + P * SN, SN);
-    zero_rows(bp.Ubar + P * SS, SS); zero_rows(bp.U + P * SS, SS); zero_rows(bp.U_t + P * SS, SS); zero_rows(bp.dU + P * SS, SS);
-    zero_rows(bp.KdX + P * bp.max_stages * 12, (size_t)bp.max_stages * 12);
-    zero_rows(bp.K + P * bp.max_stages * 288, (size_t)bp.max_stages * 288);
-    zero_rows(bp.lq + P * bp.max_stages * CR_STRIDE, (size_t)bp.max_stages * CR_STRIDE);
-    zero_rows(bp.tq + P * MAXPH * TQ_STRIDE, (size_t)MAXPH * TQ_STRIDE);
-    zero_rows(bp.gcon + P * bp.max_stages * 20, (size_t)bp.max_stages * 20);
-    zero_rows(bp.reb + P * bp.max_stages * 40, (size_t)bp.max_stages * 40);
-    zero_rows(bp.hcon + P * MAXPH * 4, (size_t)MAXPH * 4);
-    zero_rows(bp.al + P * MAXPH * 16, (size_t)MAXPH * 16);
-    zero_rows(bp.g0h0 + P * 600, 600);
-    zero_rows((double*)(bp.trace + P * HSDDP_TRACE_CAP), HSDDP_TRACE_CAP * sizeof(hsddp_iter_record) / sizeof(double));
-    if (bp.ls_X) {  // trial arrays of the concurrent line search (small batches)
-        const size_t Q = P * 4;
-        zero_rows(bp.ls_X + Q * SN, 4 * SN); zero_rows(bp.ls_Defect + Q * SN, 4 * SN); zero_rows(bp.ls_Xsim + Q * SN, 4 * SN);
-        zero_rows(bp.ls_U + Q * SS, 4 * SS); zero_rows(bp.ls_Ut + Q * SS, 4 * SS);
-        zero_rows(bp.ls_gcon + Q * bp.max_stages * 20, 4 * (size_t)bp.max_stages * 20);
-        zero_rows(bp.ls_hcon + Q * MAXPH * 4, 4 * (size_t)MAXPH * 4);
-        zero_rows(bp.ls_res + Q * 8, 32);
-        if (threadIdx.x == 0) bp.ls_mail[pid] = 0;
+    const size_t P = pid;
+    for (int a = 0; a < ra.n_clear; ++a) {
+        unsigned* p = ra.clear[a].base + P * ra.clear[a].words;
+        for (size_t e = threadIdx.x; e < ra.clear[a].words; e += kThreads) p[e] = 0u;
     }
     if (threadIdx.x == 0) {
         bp.info[pid] = hsddp_info{};
@@ -1161,13 +1143,27 @@ int guarded(F&& body) {
     }
 }
 
-template <class T>
-int dalloc(hsddp_batch* b, T** p, size_t n) {
+int dalloc_bytes(hsddp_batch* b, void** p, size_t bytes) {
     void* q = nullptr;
-    CK(cudaMalloc(&q, n * sizeof(T)));
+    CK(cudaMalloc(&q, bytes));
     b->allocs.push_back(q);
-    *p = (T*)q;
+    *p = q;
     return HSDDP_OK;
+}
+
+template <class T>
+int dalloc(hsddp_batch* b, T** p, size_t n) { return dalloc_bytes(b, (void**)p, n * sizeof(T)); }
+
+// *p := q in `allocs`; the old allocation (if any) is freed, so nothing may still use it on the device
+void replace_alloc(hsddp_batch* b, void** p, void* q) {
+    if (*p) {
+        for (void*& a : b->allocs)
+            if (a == *p) a = q;
+        cudaFree(*p);
+    } else {
+        b->allocs.push_back(q);
+    }
+    *p = q;
 }
 
 // device scratch of at least `n` elements, kept in `allocs` (freed with the problem set)
@@ -1176,16 +1172,98 @@ int scratch(hsddp_batch* b, T** p, size_t* cap, size_t n) {
     if (*cap >= n) return HSDDP_OK;
     void* q = nullptr;
     CK(cudaMalloc(&q, n * sizeof(T)));
-    if (*p) {
-        CK(cudaStreamSynchronize(b->stream));
-        for (void*& a : b->allocs)
-            if (a == (void*)*p) a = q;
-        cudaFree(*p);
-    } else {
-        b->allocs.push_back(q);
-    }
-    *p = (T*)q; *cap = n;
+    if (*p) CK(cudaStreamSynchronize(b->stream));
+    replace_alloc(b, (void**)p, q);
+    *cap = n;
     return HSDDP_OK;
+}
+
+// Every array of the batch's workspace (DESIGN.md §3.1), from the batch dimensions in b->bp.  alloc_workspace allocates and
+// zero-fills each one, k_restart zeroes a restarted problem's part of those marked WS_RESTART, and the C ABI's stored views
+// (hsddp_batch_get_array / _rows / set_array) are the entries with an HSDDP_ARR_* id.  Budget and command buffers are
+// allocated lazily elsewhere, so batches that never restart or read commands do not pay for them.
+enum : unsigned {
+    WS_SET = 1,      // hsddp_batch_set_array may overwrite it
+    WS_RESTART = 2,  // k_restart zeroes it (every array a solve reads that the restart does not write itself)
+    WS_SMALL = 4,    // only for n_problems <= kClusterLsMax: trial arrays of the concurrent line search, four per problem
+    WS_BATCH = 8,    // one per batch, not per problem
+};
+struct WsArray {
+    void** field;      // the BatchPtrs / handle member it fills
+    size_t rows, row_bytes;  // per problem (per batch: WS_BATCH); a C ABI row is row_bytes / 8 doubles
+    int abi;           // HSDDP_ARR_* id of the stored view, -1: none
+    unsigned flags;
+    size_t bytes() const { return rows * row_bytes; }
+};
+
+std::vector<WsArray> workspace_arrays(hsddp_batch* b) {
+    BatchPtrs& bp = b->bp;
+    const size_t S = bp.max_nodes, N = bp.max_stages, D = sizeof(double), I = sizeof(int);
+    return {
+        {(void**)&bp.x0, 1, 24 * D, -1, 0},
+        {(void**)&bp.Xbar, S, 24 * D, HSDDP_ARR_XBAR, WS_SET | WS_RESTART},
+        {(void**)&bp.X, S, 24 * D, HSDDP_ARR_X, WS_SET | WS_RESTART},
+        {(void**)&bp.Xsim_t, S, 24 * D, -1, WS_RESTART},
+        {(void**)&bp.Defect, S, 24 * D, HSDDP_ARR_DEFECT, WS_RESTART},
+        {(void**)&bp.dX, S, 24 * D, HSDDP_ARR_DX, WS_SET | WS_RESTART},
+        {(void**)&bp.Ubar, N, 24 * D, HSDDP_ARR_UBAR, WS_SET | WS_RESTART},
+        {(void**)&bp.U, N, 24 * D, HSDDP_ARR_U, WS_SET | WS_RESTART},
+        {(void**)&bp.U_t, N, 24 * D, -1, WS_RESTART},
+        {(void**)&bp.dU, N, 24 * D, HSDDP_ARR_DU, WS_SET | WS_RESTART},
+        {(void**)&bp.KdX, N, 12 * D, -1, WS_RESTART},
+        {(void**)&bp.K, N, 288 * D, -1, WS_RESTART},  // (HSDDP_ARR_K is the dense view, get_gains)
+        {(void**)&bp.lq, N, CR_STRIDE * D, -1, WS_RESTART},
+        {(void**)&bp.tq, MAXPH, TQ_STRIDE * D, -1, WS_RESTART},
+        {(void**)&bp.gcon, N, 20 * D, HSDDP_ARR_GCON, WS_RESTART},
+        {(void**)&bp.reb, N, 40 * D, HSDDP_ARR_REB, WS_RESTART},
+        {(void**)&bp.hcon, MAXPH, 4 * D, HSDDP_ARR_HCON, WS_RESTART},
+        {(void**)&bp.al, MAXPH, 16 * D, HSDDP_ARR_AL, WS_RESTART},
+        {(void**)&bp.g0h0, 1, 600 * D, -1, WS_RESTART},  // (HSDDP_ARR_G0 / H0 are strided views of it)
+        {(void**)&bp.state, 1, sizeof(SolverState), -1, 0},
+        {(void**)&bp.ctl, 1, sizeof(SolveCtl), -1, 0},
+        {(void**)&b->d_active[0], 1, I, -1, 0},
+        {(void**)&b->d_active[1], 1, I, -1, 0},
+        {(void**)&b->d_order, 1, I, -1, 0},
+        {(void**)&bp.ls_X, 4 * S, 24 * D, -1, WS_SMALL | WS_RESTART},
+        {(void**)&bp.ls_Defect, 4 * S, 24 * D, -1, WS_SMALL | WS_RESTART},
+        {(void**)&bp.ls_Xsim, 4 * S, 24 * D, -1, WS_SMALL | WS_RESTART},
+        {(void**)&bp.ls_U, 4 * N, 24 * D, -1, WS_SMALL | WS_RESTART},
+        {(void**)&bp.ls_Ut, 4 * N, 24 * D, -1, WS_SMALL | WS_RESTART},
+        {(void**)&bp.ls_gcon, 4 * N, 20 * D, -1, WS_SMALL | WS_RESTART},
+        {(void**)&bp.ls_hcon, 4 * MAXPH, 4 * D, -1, WS_SMALL | WS_RESTART},
+        {(void**)&bp.ls_res, 4, 8 * D, -1, WS_SMALL | WS_RESTART},
+        {(void**)&bp.ls_mail, 1, I, -1, WS_SMALL | WS_RESTART},
+        {(void**)&b->d_count, 2 * hsddp_batch::kMaxGroups, I, -1, WS_BATCH},
+        {(void**)&bp.info, 1, sizeof(hsddp_info), -1, 0},
+        {(void**)&bp.trace, HSDDP_TRACE_CAP, sizeof(hsddp_iter_record), -1, WS_RESTART},
+        {(void**)&bp.counters, 32, sizeof(unsigned long long), -1, WS_BATCH},
+        {(void**)&bp.work_counter, 4, I, -1, WS_BATCH},
+        {(void**)&bp.sm_slots, 256, I, -1, WS_BATCH},
+        {(void**)&b->d_ok, 1, I, -1, 0},
+        {(void**)&b->d_darg, 1, D, -1, 0},
+    };
+}
+
+// the table entry of stored view `which` of the C ABI
+bool stored_array(hsddp_batch* b, int which, WsArray* out) {
+    if (which < 0) return false;
+    for (const WsArray& a : workspace_arrays(b))
+        if (a.abi == which) { *out = a; return true; }
+    return false;
+}
+
+// The schedule-slot storage of a batch built from gaits: per slot its phase table, update state, gait / window and
+// node_stride reference rows (slot s owns rows [s * node_stride, (s + 1) * node_stride), so ref_off survives a growth).
+struct SlotArray { void** field; size_t bytes; };
+
+std::vector<SlotArray> slot_arrays(hsddp_batch* b) {
+    BatchPtrs& bp = b->bp;
+    const size_t rows = (size_t)b->node_stride, D = sizeof(double);
+    return {
+        {(void**)&bp.sched, sizeof(DevSchedule)}, {(void**)&b->d_mpc, sizeof(MpcSched)},
+        {(void**)&b->d_sched_gait, sizeof(int)}, {(void**)&b->d_sched_window, sizeof(int)},
+        {(void**)&bp.xr, 24 * rows * D}, {(void**)&bp.ur, 24 * rows * D}, {(void**)&bp.prel, 12 * rows * D}, {(void**)&bp.xinit, 24 * rows * D},
+    };
 }
 
 void free_problem_allocs(hsddp_batch* b) {
@@ -1327,68 +1405,16 @@ int hsddp_batch_destroy(hsddp_batch* b) {
     return HSDDP_OK;
 }
 
-// per-problem workspace (DESIGN.md §3.1); bp.n_problems / max_stages / max_nodes are set by the caller
-static int alloc_workspace(hsddp_batch* b, int n_problems, int max_stages, int max_nodes) {
-    BatchPtrs& bp = b->bp;
-    int rc;
-    const size_t P = (size_t)n_problems, SN = (size_t)max_nodes * 24, SS = (size_t)max_stages * 24;
-    if ((rc = dalloc(b, &bp.x0, P * 24))) return rc;
-    if ((rc = dalloc(b, &bp.Xbar, P * SN))) return rc;
-    if ((rc = dalloc(b, &bp.X, P * SN))) return rc;
-    if ((rc = dalloc(b, &bp.Xsim_t, P * SN))) return rc;
-    if ((rc = dalloc(b, &bp.Defect, P * SN))) return rc;
-    if ((rc = dalloc(b, &bp.dX, P * SN))) return rc;
-    if ((rc = dalloc(b, &bp.Ubar, P * SS))) return rc;
-    if ((rc = dalloc(b, &bp.U, P * SS))) return rc;
-    if ((rc = dalloc(b, &bp.U_t, P * SS))) return rc;
-    if ((rc = dalloc(b, &bp.dU, P * SS))) return rc;
-    if ((rc = dalloc(b, &bp.KdX, P * max_stages * 12))) return rc;
-    if ((rc = dalloc(b, &bp.K, P * max_stages * 288))) return rc;
-    if ((rc = dalloc(b, &bp.lq, P * max_stages * CR_STRIDE))) return rc;
-    if ((rc = dalloc(b, &bp.tq, P * MAXPH * TQ_STRIDE))) return rc;
-    if ((rc = dalloc(b, &bp.gcon, P * max_stages * 20))) return rc;
-    if ((rc = dalloc(b, &bp.reb, P * max_stages * 40))) return rc;
-    if ((rc = dalloc(b, &bp.hcon, P * MAXPH * 4))) return rc;
-    if ((rc = dalloc(b, &bp.al, P * MAXPH * 16))) return rc;
-    if ((rc = dalloc(b, &bp.g0h0, P * 600))) return rc;
-    if ((rc = dalloc(b, &bp.state, P))) return rc;
-    if ((rc = dalloc(b, &bp.ctl, P))) return rc;
-    if ((rc = dalloc(b, &b->d_active[0], P))) return rc;
-    if ((rc = dalloc(b, &b->d_active[1], P))) return rc;
-    if ((rc = dalloc(b, &b->d_order, P))) return rc;
-    if (n_problems <= hsddp_batch::kClusterLsMax) {  // trial arrays of the concurrent line search (small batches only)
-        const size_t Q = P * 4;
-        if ((rc = dalloc(b, &bp.ls_X, Q * SN)) || (rc = dalloc(b, &bp.ls_Defect, Q * SN)) || (rc = dalloc(b, &bp.ls_Xsim, Q * SN)) ||
-            (rc = dalloc(b, &bp.ls_U, Q * SS)) || (rc = dalloc(b, &bp.ls_Ut, Q * SS)) || (rc = dalloc(b, &bp.ls_gcon, Q * max_stages * 20)) ||
-            (rc = dalloc(b, &bp.ls_hcon, Q * MAXPH * 4)) || (rc = dalloc(b, &bp.ls_res, Q * 8)) || (rc = dalloc(b, &bp.ls_mail, P)))
-            return rc;
-        CK(cudaMemset(bp.ls_X, 0, Q * SN * sizeof(double)));
-        CK(cudaMemset(bp.ls_Defect, 0, Q * SN * sizeof(double)));
-        CK(cudaMemset(bp.ls_Xsim, 0, Q * SN * sizeof(double)));
-        CK(cudaMemset(bp.ls_U, 0, Q * SS * sizeof(double)));
-        CK(cudaMemset(bp.ls_Ut, 0, Q * SS * sizeof(double)));
-        CK(cudaMemset(bp.ls_res, 0, Q * 8 * sizeof(double)));
-        CK(cudaMemset(bp.ls_mail, 0, P * sizeof(int)));
+// the workspace (workspace_arrays), zero-filled; bp.n_problems / max_stages / max_nodes are set by the caller
+static int alloc_workspace(hsddp_batch* b) {
+    const size_t P = (size_t)b->bp.n_problems;
+    for (const WsArray& a : workspace_arrays(b)) {
+        if ((a.flags & WS_SMALL) && P > (size_t)hsddp_batch::kClusterLsMax) continue;
+        const size_t bytes = a.bytes() * ((a.flags & WS_BATCH) ? 1 : P);
+        if (int rc = dalloc_bytes(b, a.field, bytes)) return rc;
+        CK(cudaMemsetAsync(*a.field, 0, bytes, b->stream));
     }
     b->have_order = false;
-    if ((rc = dalloc(b, &b->d_count, (size_t)2 * hsddp_batch::kMaxGroups))) return rc;
-    CK(cudaMemset(bp.ctl, 0, P * sizeof(SolveCtl)));
-    if ((rc = dalloc(b, &bp.info, P))) return rc;
-    if ((rc = dalloc(b, &bp.trace, P * HSDDP_TRACE_CAP))) return rc;
-    if ((rc = dalloc(b, &bp.counters, (size_t)32))) return rc;
-    if ((rc = dalloc(b, &bp.work_counter, (size_t)4))) return rc;
-    if ((rc = dalloc(b, &bp.sm_slots, (size_t)256))) return rc;
-    CK(cudaMemset(bp.sm_slots, 0, 256 * sizeof(int)));
-    if ((rc = dalloc(b, &b->d_ok, P))) return rc;
-    if ((rc = dalloc(b, &b->d_darg, P))) return rc;
-    CK(cudaMemset(bp.x0, 0, P * 24 * sizeof(double)));
-    CK(cudaMemset(bp.info, 0, P * sizeof(hsddp_info)));
-    CK(cudaMemset(bp.trace, 0, P * HSDDP_TRACE_CAP * sizeof(hsddp_iter_record)));
-    CK(cudaMemset(bp.state, 0, P * sizeof(SolverState)));
-    CK(cudaMemset(bp.counters, 0, 32 * sizeof(unsigned long long)));
-    CK(cudaMemset(bp.tq, 0, P * MAXPH * TQ_STRIDE * sizeof(double)));
-    CK(cudaMemset(bp.lq, 0, P * max_stages * CR_STRIDE * sizeof(double)));
-    CK(cudaMemset(bp.g0h0, 0, P * 600 * sizeof(double)));
     return HSDDP_OK;
 }
 
@@ -1463,7 +1489,7 @@ int hsddp_batch_set_problems(hsddp_batch* b, int n_schedules, const hsddp_schedu
     CK(cudaMemcpy(d_xinit, xinit.data(), xinit.size() * sizeof(double), cudaMemcpyHostToDevice));
     bp.sched = d_sched; bp.sched_id = d_sid; bp.xr = d_xr; bp.ur = d_ur; bp.prel = d_prel; bp.xinit = d_xinit;
 
-    if ((rc = alloc_workspace(b, n_problems, max_stages, max_nodes))) return rc;
+    if ((rc = alloc_workspace(b))) return rc;
     b->has_problems = true;
     return hsddp_batch_reset(b);
     });
@@ -1488,11 +1514,11 @@ int hsddp_batch_set_problems_from_gaits(hsddp_batch* b, int n_gaits, const int32
     for (int i = 0; i < n_problems; ++i)
         if (schedule_id[i] < 0 || schedule_id[i] >= n_schedules) { g_last_error = "schedule_id out of range"; return HSDDP_ERR_ARG; }
     // gait library -> HBM
-    double *d_bs, *d_qj, *d_ft, *d_grf; int *d_ct, *d_ro, *d_nr, *d_sg, *d_sw, *d_status; float* d_dt;
+    double *d_bs, *d_qj, *d_ft, *d_grf; int *d_ct, *d_ro, *d_nr, *d_status; float* d_dt;
     int rc;
     if ((rc = dalloc(b, &d_bs, rows * 12)) || (rc = dalloc(b, &d_qj, rows * 12)) || (rc = dalloc(b, &d_ft, rows * 12)) || (rc = dalloc(b, &d_grf, rows * 12)) ||
         (rc = dalloc(b, &d_ct, rows * 4)) || (rc = dalloc(b, &d_ro, (size_t)n_gaits)) || (rc = dalloc(b, &d_nr, (size_t)n_gaits)) || (rc = dalloc(b, &d_dt, (size_t)n_gaits)) ||
-        (rc = dalloc(b, &d_sg, (size_t)n_schedules)) || (rc = dalloc(b, &d_sw, (size_t)n_schedules)) || (rc = dalloc(b, &d_status, (size_t)n_schedules)))
+        (rc = dalloc(b, &d_status, (size_t)n_schedules)))
         return rc;
     CK(cudaMemcpy(d_bs, body_state, rows * 12 * sizeof(double), cudaMemcpyHostToDevice));
     CK(cudaMemcpy(d_qj, qJ, rows * 12 * sizeof(double), cudaMemcpyHostToDevice));
@@ -1502,8 +1528,6 @@ int hsddp_batch_set_problems_from_gaits(hsddp_batch* b, int n_gaits, const int32
     CK(cudaMemcpy(d_ro, row_off.data(), n_gaits * sizeof(int), cudaMemcpyHostToDevice));
     CK(cudaMemcpy(d_nr, gait_rows, n_gaits * sizeof(int), cudaMemcpyHostToDevice));
     CK(cudaMemcpy(d_dt, gait_dt, n_gaits * sizeof(float), cudaMemcpyHostToDevice));
-    CK(cudaMemcpy(d_sg, sched_gait, n_schedules * sizeof(int), cudaMemcpyHostToDevice));
-    CK(cudaMemcpy(d_sw, sched_window, n_schedules * sizeof(int), cudaMemcpyHostToDevice));
     GaitLib lib{d_bs, d_qj, d_ft, d_grf, d_ct, d_ro, d_nr, d_dt};
 
     BatchPtrs& bp = b->bp;
@@ -1511,19 +1535,21 @@ int hsddp_batch_set_problems_from_gaits(hsddp_batch* b, int n_gaits, const int32
     if (cparams) bp.cp = *cparams;
     else { bp.cp.grf_delta = 0.1; bp.cp.grf_delta_min = 0.1; bp.cp.grf_eps = 0.1; bp.cp.td_sigma = 50; bp.cp.td_sigma_max = 1e4; bp.cp.td_lambda = 0; bp.cp.mu = 0.7; }
     const int node_stride = std::min(HSDDP_MAX_STAGES, (int)std::lround(plan_duration / 0.01f) + 1) + MAXPH;
-    DevSchedule* d_sched; int* d_sid; double *d_xr, *d_ur, *d_prel, *d_xinit;
-    const size_t total_nodes = (size_t)n_schedules * node_stride;
-    if ((rc = dalloc(b, &d_sched, (size_t)n_schedules)) || (rc = dalloc(b, &d_sid, (size_t)n_problems)) || (rc = dalloc(b, &d_xr, total_nodes * 24)) ||
-        (rc = dalloc(b, &d_ur, total_nodes * 24)) || (rc = dalloc(b, &d_prel, total_nodes * 12)) || (rc = dalloc(b, &d_xinit, total_nodes * 24)))
-        return rc;
+    b->node_stride = node_stride;
+    for (const SlotArray& a : slot_arrays(b))  // one schedule slot per schedule
+        if ((rc = dalloc_bytes(b, a.field, (size_t)n_schedules * a.bytes))) return rc;
+    int *d_sid, *d_err;
+    if ((rc = dalloc(b, &d_sid, (size_t)n_problems)) || (rc = dalloc(b, &d_err, (size_t)4))) return rc;
+    CK(cudaMemcpy(b->d_sched_gait, sched_gait, n_schedules * sizeof(int), cudaMemcpyHostToDevice));
+    CK(cudaMemcpy(b->d_sched_window, sched_window, n_schedules * sizeof(int), cudaMemcpyHostToDevice));
     CK(cudaMemcpy(d_sid, schedule_id, sizeof(int) * n_problems, cudaMemcpyHostToDevice));
-    MpcSched* d_mpc; int* d_err;
-    if ((rc = dalloc(b, &d_mpc, (size_t)n_schedules)) || (rc = dalloc(b, &d_err, (size_t)4))) return rc;
     CK(cudaMemsetAsync(d_err, 0, 4 * sizeof(int), b->stream));
-    k_build_phase_tables<<<(n_schedules + 127) / 128, 128, 0, b->stream>>>(lib, n_schedules, d_sg, d_sw, plan_duration, node_stride, d_sched, d_status, d_mpc,
-                                                                           nullptr, HSDDP_MAX_STAGES);
-    k_build_reference_rows<<<n_schedules, 128, 0, b->stream>>>(lib, n_schedules, d_sg, d_sw, plan_duration, node_stride, d_sched, d_status, d_xr, d_ur, d_prel, d_xinit,
-                                                               nullptr);
+    DevSchedule* d_sched = const_cast<DevSchedule*>(bp.sched);
+    k_build_phase_tables<<<(n_schedules + 127) / 128, 128, 0, b->stream>>>(lib, n_schedules, b->d_sched_gait, b->d_sched_window, plan_duration, node_stride, d_sched,
+                                                                           d_status, b->d_mpc, nullptr, HSDDP_MAX_STAGES);
+    k_build_reference_rows<<<n_schedules, 128, 0, b->stream>>>(lib, n_schedules, b->d_sched_gait, b->d_sched_window, plan_duration, node_stride, d_sched, d_status,
+                                                               const_cast<double*>(bp.xr), const_cast<double*>(bp.ur), const_cast<double*>(bp.prel),
+                                                               const_cast<double*>(bp.xinit), nullptr);
     CK(cudaGetLastError());
     b->n_step_launches += 2;
     // the host keeps the phase tables too (dense gain / Jacobian getters, workspace sizing)
@@ -1542,11 +1568,11 @@ int hsddp_batch_set_problems_from_gaits(hsddp_batch* b, int n_gaits, const int32
     // (node rows with headroom: a receding-horizon update can add phases, i.e. nodes, while the stage count stays the same)
     max_nodes = std::min(node_stride, max_stages + MAXPH);
     bp.n_problems = n_problems; bp.max_stages = max_stages; bp.max_nodes = max_nodes;
-    bp.sched = d_sched; bp.sched_id = d_sid; bp.xr = d_xr; bp.ur = d_ur; bp.prel = d_prel; bp.xinit = d_xinit;
-    if ((rc = alloc_workspace(b, n_problems, max_stages, max_nodes))) return rc;
+    bp.sched_id = d_sid;
+    if ((rc = alloc_workspace(b))) return rc;
     b->has_problems = true;
-    b->lib = lib; b->d_sched_gait = d_sg; b->d_sched_window = d_sw; b->d_mpc = d_mpc; b->d_mpc_err = d_err;
-    b->plan = plan_duration; b->node_stride = node_stride; b->n_sched = n_schedules; b->n_gaits = n_gaits; b->mpc_ready = true;
+    b->lib = lib; b->d_mpc_err = d_err;
+    b->plan = plan_duration; b->n_sched = n_schedules; b->n_gaits = n_gaits; b->mpc_ready = true;
     return hsddp_batch_reset(b);
     });
 }
@@ -1624,33 +1650,25 @@ int hsddp_batch_get_schedule(hsddp_batch* b, int i, int32_t* n_phases, int32_t* 
 // `add` more schedule slots: the slot arrays are reallocated and the existing slots copied device to device (ref_off stays
 // valid: slot s keeps reference rows [s * node_stride, (s + 1) * node_stride)).  The new slots are free.
 static int grow_slots(hsddp_batch* b, int add) {
-    const size_t cap = (size_t)b->n_sched, ncap = cap + (size_t)add, rows = (size_t)b->node_stride;
-    BatchPtrs& bp = b->bp;
-    void* old[8] = {(void*)bp.sched, (void*)b->d_mpc, (void*)b->d_sched_gait, (void*)b->d_sched_window,
-                    (void*)bp.xr, (void*)bp.ur, (void*)bp.prel, (void*)bp.xinit};
-    const size_t elem[8] = {sizeof(DevSchedule), sizeof(MpcSched), sizeof(int), sizeof(int), 24 * rows * sizeof(double),
-                            24 * rows * sizeof(double), 12 * rows * sizeof(double), 24 * rows * sizeof(double)};
-    void* nw[8] = {};
-    for (int a = 0; a < 8; ++a) {
-        const cudaError_t e = cudaMalloc(&nw[a], ncap * elem[a]);
+    const size_t cap = (size_t)b->n_sched, ncap = cap + (size_t)add;
+    const std::vector<SlotArray> arrays = slot_arrays(b);
+    std::vector<void*> nw(arrays.size(), nullptr);
+    for (size_t a = 0; a < arrays.size(); ++a) {
+        const cudaError_t e = cudaMalloc(&nw[a], ncap * arrays[a].bytes);
         if (e != cudaSuccess) {
-            for (int q = 0; q < a; ++q) cudaFree(nw[q]);
+            for (void* q : nw) cudaFree(q);
             g_last_error = std::string("growing the schedule slots: ") + cudaGetErrorString(e);
             return HSDDP_ERR_CUDA;
         }
     }
-    for (int a = 0; a < 8; ++a) {
-        CK(cudaMemcpyAsync(nw[a], old[a], cap * elem[a], cudaMemcpyDeviceToDevice, b->stream));
-        CK(cudaMemsetAsync((char*)nw[a] + cap * elem[a], a == 2 ? 0xff : 0, (ncap - cap) * elem[a], b->stream));  // (gait -1: free)
+    for (size_t a = 0; a < arrays.size(); ++a) {
+        const size_t bytes = arrays[a].bytes;
+        const int fill = arrays[a].field == (void**)&b->d_sched_gait ? 0xff : 0;  // (gait -1: free)
+        CK(cudaMemcpyAsync(nw[a], *arrays[a].field, cap * bytes, cudaMemcpyDeviceToDevice, b->stream));
+        CK(cudaMemsetAsync((char*)nw[a] + cap * bytes, fill, (ncap - cap) * bytes, b->stream));
     }
     CK(cudaStreamSynchronize(b->stream));
-    for (int a = 0; a < 8; ++a) {
-        for (void*& p : b->allocs)
-            if (p == old[a]) p = nw[a];
-        cudaFree(old[a]);
-    }
-    bp.sched = (DevSchedule*)nw[0]; b->d_mpc = (MpcSched*)nw[1]; b->d_sched_gait = (int*)nw[2]; b->d_sched_window = (int*)nw[3];
-    bp.xr = (double*)nw[4]; bp.ur = (double*)nw[5]; bp.prel = (double*)nw[6]; bp.xinit = (double*)nw[7];
+    for (size_t a = 0; a < arrays.size(); ++a) replace_alloc(b, arrays[a].field, nw[a]);
     b->n_sched = (int)ncap;
     b->slot_refs.resize(ncap, 0);
     b->h_sched.resize(ncap);
@@ -1743,6 +1761,13 @@ int hsddp_batch_restart_problems(hsddp_batch* b, int n, const int32_t* problem, 
         if (a_st[j] == 1) { g_last_error = "restart: window does not fit the gait table"; return HSDDP_ERR_ARG; }
         if (a_st[j]) { g_last_error = "restart: schedule exceeds HSDDP_MAX_PHASES / the batch's node capacity"; return HSDDP_ERR_UNSUPPORTED; }
     }
+    RestartArgs ra{d, d + n, d_st + m, d_st + m + c, d_st + m + 2 * c, b->d_restart_x0, c,
+                   first_solve ? first_solve->max_AL_iter : -1, first_solve ? first_solve->max_DDP_iter : -1, b->d_sched_gait, b->d_sched_window, 0, {}};
+    for (const WsArray& a : workspace_arrays(b))
+        if ((a.flags & WS_RESTART) && *a.field) {
+            if (ra.n_clear == kRestartClearMax) { g_last_error = "restart: more workspace arrays than kRestartClearMax"; return HSDDP_ERR_STATE; }
+            ra.clear[ra.n_clear++] = {(unsigned*)*a.field, a.bytes() / sizeof(unsigned)};
+        }
     // commit
     b->slot_refs.swap(refs);
     for (int s : freed) free_after.push_back(s);
@@ -1750,8 +1775,6 @@ int hsddp_batch_restart_problems(hsddp_batch* b, int n, const int32_t* problem, 
     for (int k = 0; k < n; ++k) b->h_sched_id[problem[k]] = bslot[pair_of[k]];
     b->h_sched_stale = true;
     b->slots_marked = true;
-    RestartArgs ra{d, d + n, d_st + m, d_st + m + c, d_st + m + 2 * c, b->d_restart_x0, c,
-                   first_solve ? first_solve->max_AL_iter : -1, first_solve ? first_solve->max_DDP_iter : -1, b->d_sched_gait, b->d_sched_window};
     k_restart<<<n, kThreads, 0, b->stream>>>(b->bp, ra);
     CK(cudaGetLastError());
     b->n_step_launches++;
@@ -2067,28 +2090,6 @@ static int get_gains(hsddp_batch* b, int row0, int nrows, double* out) {
     return HSDDP_OK;
 }
 
-static int array_spec(hsddp_batch* b, int which, double** dev, size_t* per_problem) {
-    const BatchPtrs& bp = b->bp;
-    const size_t SN = (size_t)bp.max_nodes * 24, SS = (size_t)bp.max_stages * 24;
-    switch (which) {
-        case HSDDP_ARR_XBAR: *dev = bp.Xbar; *per_problem = SN; return 0;
-        case HSDDP_ARR_X: *dev = bp.X; *per_problem = SN; return 0;
-        case HSDDP_ARR_DEFECT: *dev = bp.Defect; *per_problem = SN; return 0;
-        case HSDDP_ARR_DX: *dev = bp.dX; *per_problem = SN; return 0;
-        case HSDDP_ARR_UBAR: *dev = bp.Ubar; *per_problem = SS; return 0;
-        case HSDDP_ARR_U: *dev = bp.U; *per_problem = SS; return 0;
-        case HSDDP_ARR_DU: *dev = bp.dU; *per_problem = SS; return 0;
-        case HSDDP_ARR_K: *dev = bp.K; *per_problem = (size_t)bp.max_stages * 288; return 3;
-        case HSDDP_ARR_GCON: *dev = bp.gcon; *per_problem = (size_t)bp.max_stages * 20; return 0;
-        case HSDDP_ARR_HCON: *dev = bp.hcon; *per_problem = (size_t)MAXPH * 4; return 0;
-        case HSDDP_ARR_AL: *dev = bp.al; *per_problem = (size_t)MAXPH * 16; return 0;
-        case HSDDP_ARR_REB: *dev = bp.reb; *per_problem = (size_t)bp.max_stages * 40; return 0;
-        case HSDDP_ARR_G0: *dev = bp.g0h0; *per_problem = 600; return 1;  // strided special cases
-        case HSDDP_ARR_H0: *dev = bp.g0h0; *per_problem = 600; return 2;
-        default: return -1;
-    }
-}
-
 int hsddp_batch_get_array(hsddp_batch* b, int which, double* out) {
     return guarded([&]() -> int {
     if (!b || !b->has_problems || !out) return HSDDP_ERR_ARG;
@@ -2143,33 +2144,32 @@ int hsddp_batch_get_array(hsddp_batch* b, int which, double* out) {
         }
         return HSDDP_OK;
     }
-    double* dev; size_t per;
-    const int kind = array_spec(b, which, &dev, &per);
-    if (kind < 0) return HSDDP_ERR_ARG;
-    if (kind == 3) return get_gains(b, 0, bp.max_stages, out);
-    if (kind == 0) {
-        CK(cudaMemcpyAsync(out, dev, P * per * sizeof(double), cudaMemcpyDeviceToHost, b->stream));
+    if (which == HSDDP_ARR_K) return get_gains(b, 0, bp.max_stages, out);
+    if (which == HSDDP_ARR_G0 || which == HSDDP_ARR_H0) {  // strided views of g0h0
+        const size_t off = (which == HSDDP_ARR_G0) ? 0 : 24, cnt = (which == HSDDP_ARR_G0) ? 24 : 576;
+        CK(cudaMemcpy2DAsync(out, cnt * sizeof(double), bp.g0h0 + off, 600 * sizeof(double), cnt * sizeof(double), P, cudaMemcpyDeviceToHost, b->stream));
         CK(cudaStreamSynchronize(b->stream));
-    } else {
-        const size_t off = (kind == 1) ? 0 : 24, cnt = (kind == 1) ? 24 : 576;
-        CK(cudaMemcpy2DAsync(out, cnt * sizeof(double), dev + off, 600 * sizeof(double), cnt * sizeof(double), P, cudaMemcpyDeviceToHost, b->stream));
-        CK(cudaStreamSynchronize(b->stream));
+        return HSDDP_OK;
     }
+    WsArray a;
+    if (!stored_array(b, which, &a)) return HSDDP_ERR_ARG;
+    CK(cudaMemcpyAsync(out, *a.field, P * a.bytes(), cudaMemcpyDeviceToHost, b->stream));
+    CK(cudaStreamSynchronize(b->stream));
     return HSDDP_OK;
     });
 }
 
 int hsddp_batch_set_array(hsddp_batch* b, int which, const double* in) {
+    return guarded([&]() -> int {
     if (!b || !b->has_problems || !in) return HSDDP_ERR_ARG;
-    if (which != HSDDP_ARR_XBAR && which != HSDDP_ARR_X && which != HSDDP_ARR_UBAR && which != HSDDP_ARR_U &&
-        which != HSDDP_ARR_DX && which != HSDDP_ARR_DU) return HSDDP_ERR_ARG;
+    WsArray a;
+    if (!stored_array(b, which, &a) || !(a.flags & WS_SET)) return HSDDP_ERR_ARG;
     CK(cudaSetDevice(b->device));
-    double* dev; size_t per;
-    if (array_spec(b, which, &dev, &per) != 0) return HSDDP_ERR_ARG;
-    CK(cudaMemcpyAsync(dev, in, (size_t)b->bp.n_problems * per * sizeof(double), cudaMemcpyHostToDevice, b->stream));
+    CK(cudaMemcpyAsync(*a.field, in, (size_t)b->bp.n_problems * a.bytes(), cudaMemcpyHostToDevice, b->stream));
     CK(cudaStreamSynchronize(b->stream));
     b->cold = false;
     return HSDDP_OK;
+    });
 }
 
 int hsddp_batch_get_array_rows(hsddp_batch* b, int which, int row0, int nrows, double* out) {
@@ -2177,20 +2177,10 @@ int hsddp_batch_get_array_rows(hsddp_batch* b, int which, int row0, int nrows, d
     if (!b || !b->has_problems || !out || row0 < 0 || nrows <= 0) return HSDDP_ERR_ARG;
     CK(cudaSetDevice(b->device));
     if (which == HSDDP_ARR_K) return get_gains(b, row0, nrows, out);
-    double* dev; size_t per;
-    if (array_spec(b, which, &dev, &per) != 0) return HSDDP_ERR_ARG;
-    size_t cols;
-    switch (which) {
-        case HSDDP_ARR_K: cols = 576; break;
-        case HSDDP_ARR_GCON: cols = 20; break;
-        case HSDDP_ARR_HCON: cols = 4; break;
-        case HSDDP_ARR_AL: cols = 16; break;
-        case HSDDP_ARR_REB: cols = 40; break;
-        default: cols = 24; break;
-    }
-    if ((size_t)(row0 + nrows) * cols > per) return HSDDP_ERR_ARG;
-    CK(cudaMemcpy2DAsync(out, (size_t)nrows * cols * sizeof(double), dev + (size_t)row0 * cols, per * sizeof(double),
-                         (size_t)nrows * cols * sizeof(double), (size_t)b->bp.n_problems, cudaMemcpyDeviceToHost, b->stream));
+    WsArray a;
+    if (!stored_array(b, which, &a) || (size_t)row0 + (size_t)nrows > a.rows) return HSDDP_ERR_ARG;
+    CK(cudaMemcpy2DAsync(out, nrows * a.row_bytes, (const char*)*a.field + row0 * a.row_bytes, a.bytes(), nrows * a.row_bytes,
+                         (size_t)b->bp.n_problems, cudaMemcpyDeviceToHost, b->stream));
     CK(cudaStreamSynchronize(b->stream));
     return HSDDP_OK;
     });

@@ -42,8 +42,12 @@ def _tick(B, x=None):
     return x
 
 
+# every array get() returns as stored (the dense views A, B, lx, lu, lxx, luu are rebuilt from the stage records)
+STORED = ("Xbar", "X", "Defect", "dX", "Ubar", "U", "dU", "K", "g", "h", "al", "reb", "G0", "H0")
+
+
 def _state(B):
-    return dict(info=B.info(), trace=B.trace(), Xbar=B.get("Xbar"), Ubar=B.get("Ubar"), K=B.get("K"), dU=B.get("dU"), sid=B.schedule_ids())
+    return dict(info=B.info(), trace=B.trace(), sid=B.schedule_ids(), **{k: B.get(k) for k in STORED})
 
 
 def _same_schedule(a, b):
@@ -55,7 +59,7 @@ def _assert_problem_equal(A, i, B, j, dA, dB, what):
     """Problem i of batch A and problem j of batch B: bitwise equal results (rows up to the smaller row stride; the rest zero)."""
     assert A["info"][i].tobytes() == B["info"][j].tobytes(), (what, A["info"][i], B["info"][j])
     assert A["trace"][i].tobytes() == B["trace"][j].tobytes(), what
-    for k in ("Xbar", "Ubar", "K", "dU"):
+    for k in STORED:
         a, b = A[k][i], B[k][j]
         r = min(len(a), len(b))
         assert a[:r].tobytes() == b[:r].tobytes(), (what, k)
