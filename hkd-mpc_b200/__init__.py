@@ -174,6 +174,7 @@ def lib():
         L.hsddp_batch_event_elapsed_ms.argtypes = [vp, C.c_int, C.c_int, C.POINTER(C.c_float)]
         L.hsddp_batch_get_counters.argtypes = [vp, C.POINTER(C.c_ulonglong)]
         L.hsddp_batch_reset_counters.argtypes = [vp]
+        L.hsddp_batch_get_speculation.argtypes = [vp, C.POINTER(C.c_ulonglong)]
         L.hsddp_batch_get_profile.argtypes = [vp, C.POINTER(C.c_ulonglong)]
         L.hsddp_phase_batch_create.argtypes = [C.c_int] * 6 + [C.POINTER(vp)]
         L.hsddp_phase_batch_destroy.argtypes = [vp]
@@ -515,6 +516,13 @@ class MultiPhaseDDPBatch:
         out = (C.c_ulonglong * 4)()
         _check(lib().hsddp_batch_get_counters(self.h, out), "get_counters")
         return dict(sweep_stages=int(out[0]), solve_launches=int(out[1]), step_launches=int(out[2]))
+
+    def speculation(self):
+        """Regularisation retries run side by side since set_problems / reset_counters (HSDDP_SWEEP_SPEC): problem-rounds
+        speculated, rounds that kept a later candidate than the first, rounds in which every candidate failed."""
+        out = (C.c_ulonglong * 3)()
+        _check(lib().hsddp_batch_get_speculation(self.h, out), "get_speculation")
+        return dict(rounds=int(out[0]), later=int(out[1]), exceeded=int(out[2]))
 
     def profile(self):
         out = (C.c_ulonglong * 16)()

@@ -118,6 +118,13 @@ struct SolveCtl {
     double trial_cost, trial_feas;
 };
 
+// one candidate of a speculated backward sweep: ok = 1 PD, 0 failed, -1 not run (its regularisation is past the limit);
+// dV_1 / dV_2 as the sweep left them
+struct SpecRec {
+    int ok, _pad;
+    double dV_1, dV_2;
+};
+
 struct BatchPtrs {
     int n_problems, max_stages, max_nodes, _pad;
     const DevSchedule* sched;
@@ -163,6 +170,19 @@ struct BatchPtrs {
     int* work_counter;                        // dynamic problem queue of the persistent kernel
     int* sm_slots;                            // [256] per-SM arrival counter: gives co-resident blocks distinct warp-role rotations
     hsddp_constraint_params cp;
+    // phased driver, regularisation retries run side by side (DESIGN.md §4.3): in rounds the four-warp sweep takes, the prep lists
+    // the problems that regularise (spec_list / spec_count, at most spec_cap, spec_entry[pid] = list entry or -1) and the sweep
+    // runs candidates 1 .. spec_S - 1 of each on extra blocks (candidate 0 is the problem's own block).  Candidate j > 0 writes
+    // its gains, feed-forward and g0h0 to its slice of spec_out; the last of the spec_S blocks to arrive (spec_arrive[entry])
+    // commits.  spec_list == nullptr: off.
+    int* spec_list;
+    int* spec_count;
+    int* spec_zero;                           // spec counter the prep clears for the next round (the zero_count scheme)
+    int* spec_arrive;
+    int* spec_entry;                          // [P]
+    SpecRec* spec_rec;                        // [spec_cap][spec_S]
+    double* spec_out;                         // [spec_cap][spec_S - 1] slices: K [max_stages][288] | dU [max_stages][24] | g0h0 [600]
+    int spec_S, spec_cap;
 };
 
 // Shared-memory working set of one block.

@@ -290,9 +290,7 @@ __device__ inline void iter_prep_block(Smem& sm, const BatchPtrs& bp) {
     lq_approximation_block(sm);
 }
 
-__device__ inline void iter_sweep_block(Smem& sm, const BatchPtrs& bp) {
-    int nsw = 0;
-    const bool success = backward_sweep_regularized_block(sm, nsw);
+__device__ inline void finish_sweep_block(Smem& sm, const BatchPtrs& bp, bool success, int nsw) {
     if (threadIdx.x == 0) {
         sm.ctl.n_sweeps += nsw;
         if (sm.ctl.iter <= HSDDP_TRACE_CAP) {
@@ -302,6 +300,140 @@ __device__ inline void iter_sweep_block(Smem& sm, const BatchPtrs& bp) {
         if (!success) { sm.ctl.status = HSDDP_STATUS_REG_OVERFLOW; sm.ctl.active = 0; }  // bad_solve (:321-324,421-427)
     }
     __syncthreads();
+}
+
+__device__ inline void iter_sweep_block(Smem& sm, const BatchPtrs& bp) {
+    int nsw = 0;
+    const bool success = backward_sweep_regularized_block(sm, nsw);
+    finish_sweep_block(sm, bp, success, nsw);
+}
+
+// ---------------------------------------------------------------------------
+// Regularisation retries side by side (phased driver, rounds of the four-warp sweep; DESIGN.md §4.3).
+// backward_sweep_regularized tries r_0 = st.reg, r_1, ... (r_{j+1} = max(r_j update_regularization, 1e-3), until one is PD or
+// r_j > 1e2) one after another, and every attempt reads the same inputs.  Candidate j of a listed problem runs attempt j on a
+// block of its own; the last of the spec_S blocks to arrive leaves what the loop would have left: the first PD attempt, or the
+// state after every candidate failed, from which it runs the rest of the loop itself.
+// ---------------------------------------------------------------------------
+// r := r_j of the retry sequence that starts at r; false: r_j is past the limit (the loop never runs attempt j)
+__device__ __forceinline__ bool retry_reg(double& r, int j, double up) {
+    for (int i = 0; i < j; ++i) {
+        r = fmax(r * up, 1e-03);
+        if (r > 1e2) return false;
+    }
+    return true;
+}
+
+// the prep of a round the four-warp sweep takes: list the problem if it regularises (its last sweep of this solve needed a
+// retry, or it starts from reg > 0).  Scheduling only: an unlisted problem runs the loop on its own block.
+__device__ inline void spec_flag_block(Smem& sm, const BatchPtrs& bp) {
+    if (threadIdx.x == 0) {
+        const int row = sm.ctl.iter - 1;  // this iteration's trace row; row - 1 is the last sweep's
+        bool flag = sm.st.reg > 0;
+        if (row >= 1 && row <= HSDDP_TRACE_CAP) flag = flag || bp.trace[(size_t)sm.pid * HSDDP_TRACE_CAP + row - 1].n_sweeps > 1;
+        int e = -1;
+        if (flag) {
+            e = atomicAdd(bp.spec_count, 1);
+            if (e < bp.spec_cap) bp.spec_list[e] = sm.pid;
+            else e = -1;
+        }
+        bp.spec_entry[sm.pid] = e;
+    }
+}
+
+// A candidate j > 0 marks the first dU word of every stage of its slice with this signalling-NaN pattern before it sweeps.  No
+// arithmetic result has it, so a failed candidate's slice shows which stages the sweep wrote (the sweep runs from the last stage down).
+constexpr unsigned long long kSpecUnwritten = 0x7ff0dead5eed0001ull;
+
+// Candidate j of list entry e has run its attempt (ran: its regularisation is within the limit; ok: PD).  The last of the spec_S
+// blocks to arrive takes over the state the sequential loop has after its last attempt among the candidates -- the first PD one,
+// w, or the m that ran all failed -- and returns true with success, reg = that attempt's regularisation and nsw = the attempts
+// so far.  The other blocks return false.
+__device__ inline bool spec_commit_block(Smem& sm, const BatchPtrs& bp, int e, int j, bool ran, bool ok, double& reg, int& nsw, bool& success) {
+    const int tid = threadIdx.x, S = bp.spec_S, N = sm.sc.n_stages;
+    const size_t ms = (size_t)bp.max_stages, slice = ms * 312 + 600;
+    SpecRec* rec = bp.spec_rec + (size_t)e * S;
+    const double* out = bp.spec_out + (size_t)e * (S - 1) * slice;  // + (c - 1) * slice: candidate c >= 1
+    if (tid == 0) rec[j] = SpecRec{ran ? (ok ? 1 : 0) : -1, 0, sm.st.dV_1, sm.st.dV_2};
+    __threadfence();
+    __syncthreads();
+    if (tid == 0) sm.ibuf[2] = atomicAdd(bp.spec_arrive + e, 1) == S - 1;
+    __syncthreads();
+    if (!sm.ibuf[2]) return false;
+    __threadfence();
+    if (tid == 0) {
+        bp.spec_arrive[e] = 0;  // (for the next round)
+        int w = -1, m = 0;
+        while (m < S) {
+            const int c = __ldcg(&rec[m].ok);
+            if (c < 0) break;
+            ++m;
+            if (c) { w = m - 1; break; }
+        }
+        const int c = w >= 0 ? w : m - 1;
+        sm.ibuf[2] = w; sm.ibuf[3] = m;
+        const size_t pid = (size_t)sm.pid;
+        sm.K = bp.K + pid * ms * 288; sm.dU = bp.dU + pid * ms * 24; sm.g0h0 = bp.g0h0 + pid * 600;
+        sm.st.dV_1 = __ldcg(&rec[c].dV_1); sm.st.dV_2 = __ldcg(&rec[c].dV_2); sm.st.sweep_ok = w >= 0 ? 1 : 0;
+        atomicAdd(bp.counters + 1, 1ull);
+        if (w != 0) atomicAdd(bp.counters + (w > 0 ? 2 : 3), 1ull);
+    }
+    __syncthreads();
+    const int w = sm.ibuf[2], m = sm.ibuf[3];
+    // the problem's arrays as the loop leaves them: candidate w's outputs, or, every candidate failed, per stage those of the last
+    // candidate that wrote the stage (candidate 0 wrote in place)
+    for (int c = (w >= 0 ? w : 1); c <= (w >= 0 ? w : m - 1); ++c) {
+        if (c == 0) continue;
+        const double* o = out + (c - 1) * slice;
+        const unsigned long long* mark = reinterpret_cast<const unsigned long long*>(o + ms * 288);
+        for (int x = tid; x < 288 * N; x += kThreads)
+            if (w >= 0 || __ldcg(mark + 24 * (x / 288)) != kSpecUnwritten) sm.K[x] = __ldcg(o + x);
+        for (int x = tid; x < 24 * N; x += kThreads)
+            if (w >= 0 || __ldcg(mark + 24 * (x / 24)) != kSpecUnwritten) sm.dU[x] = __ldcg(o + ms * 288 + x);
+        if (w >= 0)
+            for (int x = tid; x < 600; x += kThreads) sm.g0h0[x] = __ldcg(o + ms * 312 + x);
+        __syncthreads();
+    }
+    success = w >= 0;
+    nsw = success ? w + 1 : m;
+    reg = sm.st.reg;
+    retry_reg(reg, success ? w : m - 1, sm.opt.update_regularization);
+    return true;
+}
+
+// The backward sweep of a phased round (k_phase<PH_SWEEP>): the loop of backward_sweep_regularized_block for an unlisted problem
+// (e < 0), candidate j of list entry e for a listed one.  Returns false in the candidate blocks that did not commit: they must
+// not store the problem's state.
+__device__ inline bool sweep_round_block(Smem& sm, const BatchPtrs& bp, int e, int j) {
+    const int tid = threadIdx.x;
+    const double up = sm.opt.update_regularization;
+    double reg = sm.st.reg;
+    int nsw = 0;
+    bool success = false, run = e < 0 || retry_reg(reg, j, up);
+    if (e >= 0 && j > 0 && run) {  // outputs to the candidate's slice, with the first dU word of every stage marked unwritten
+        const size_t ms = (size_t)bp.max_stages;
+        double* o = bp.spec_out + ((size_t)e * (bp.spec_S - 1) + j - 1) * (ms * 312 + 600);
+        for (int s = tid; s < sm.sc.n_stages; s += kThreads) reinterpret_cast<unsigned long long*>(o + ms * 288)[24 * s] = kSpecUnwritten;
+        if (tid == 0) { sm.K = o; sm.dU = o + ms * 288; sm.g0h0 = o + ms * 312; }
+    }
+    __syncthreads();
+    for (;;) {  // (the kernel's only call of the sweep: its code stays one sweep long)
+        if (run) { ++nsw; success = backward_sweep_block(sm, reg); }
+        if (e >= 0) {
+            if (!spec_commit_block(sm, bp, e, j, run, success, reg, nsw, success)) return false;
+            e = -1;
+        }
+        if (success) break;
+        reg = fmax(reg * up, 1e-03);
+        if (reg > 1e2) break;
+        run = true;
+    }
+    reg = reg / 20;
+    if (reg < 1e-06) reg = 0;
+    if (tid == 0) sm.st.reg = reg;
+    __syncthreads();
+    finish_sweep_block(sm, bp, success, nsw);
+    return true;
 }
 
 template <bool CLUSTER_LS = false>
@@ -488,10 +620,22 @@ template <int PH>
 __global__ void __launch_bounds__(kThreads, PH == 2 ? HSDDP_MINB_SWEEP : HSDDP_MINB_OTHER) k_phase(BatchPtrs bp, hsddp_options opt) {
     __shared__ Smem sm;
     // (the counter of the list this round appends to is cleared even when no problem is left: the next round reads it)
-    if (PH == PH_PREP && bp.zero_count && blockIdx.x == 0 && threadIdx.x == 0) *bp.zero_count = 0;
-    if (bp.n_active && (int)blockIdx.x >= *bp.n_active) return;  // (the grid is the group's full size: see BatchPtrs::active)
+    if (PH == PH_PREP && bp.zero_count && blockIdx.x == 0 && threadIdx.x == 0) {
+        *bp.zero_count = 0;
+        if (bp.spec_zero) *bp.spec_zero = 0;
+    }
+    // sweep with speculation: the first spec_cap x (spec_S - 1) blocks are candidates 1 .. spec_S - 1 of the listed problems
+    // (the lowest block indices, so that the long retry chains start first), the problems' own blocks follow
+    int blk = (int)blockIdx.x, cand = 0, entry = -1;
+    if (PH == PH_SWEEP && bp.spec_list) {
+        const int ns = bp.spec_cap * (bp.spec_S - 1);
+        if (blk < ns) { entry = blk / (bp.spec_S - 1); cand = 1 + blk % (bp.spec_S - 1); }
+        blk -= ns;
+    }
+    if (bp.n_active && blk >= *bp.n_active) return;  // (the grid is the group's full size: see BatchPtrs::active)
     if (PH == PH_SWEEP && bp.n_active && bp.sweep_w1_min > 0 && *bp.n_active >= bp.sweep_w1_min) return;  // (k_sweep_w1 takes this round)
-    const int pid = bp.active ? bp.active[blockIdx.x] : (int)blockIdx.x;
+    if (PH == PH_SWEEP && cand > 0 && entry >= min(*bp.spec_count, bp.spec_cap)) return;
+    const int pid = cand > 0 ? bp.spec_list[entry] : bp.active ? bp.active[blk] : blk;
     if (threadIdx.x == 0) assign_rotation(bp.sm_slots, sm.rot);
     bind_problem(sm, bp, pid);
     if (threadIdx.x == 0) sm.opt = opt;
@@ -500,9 +644,16 @@ __global__ void __launch_bounds__(kThreads, PH == 2 ? HSDDP_MINB_SWEEP : HSDDP_M
     if (threadIdx.x == 0) for (int i = 0; i < 16; ++i) sm.profacc[i] = 0;
     __syncthreads();
 #endif
+    bool store = true;
     if (PH == PH_BEGIN) solve_begin_block(sm, bp);
-    if (PH == PH_PREP) iter_prep_block(sm, bp);
-    if (PH == PH_SWEEP) iter_sweep_block(sm, bp);
+    if (PH == PH_PREP) {
+        iter_prep_block(sm, bp);
+        if (bp.spec_list && (bp.sweep_w1_min == 0 || *bp.n_active < bp.sweep_w1_min)) spec_flag_block(sm, bp);
+    }
+    if (PH == PH_SWEEP) {
+        if (bp.spec_list && cand == 0) entry = bp.spec_entry[pid];
+        store = sweep_round_block(sm, bp, entry, cand);
+    }
     if (PH == PH_FORWARD) {
         if (sm.ctl.active) iter_forward_block(sm, bp);  // (a failed sweep already ended the solve)
     }
@@ -514,7 +665,7 @@ __global__ void __launch_bounds__(kThreads, PH == 2 ? HSDDP_MINB_SWEEP : HSDDP_M
             solve_finish_block(sm, bp);
         }
     }
-    if (threadIdx.x == 0) { bp.state[pid] = sm.st; bp.ctl[pid] = sm.ctl; }
+    if (store && threadIdx.x == 0) { bp.state[pid] = sm.st; bp.ctl[pid] = sm.ctl; }
 #ifdef HSDDP_PROFILE
     if (threadIdx.x == 0) for (int i = 0; i < 16; ++i) atomicAdd(&sm.prof[i], sm.profacc[i]);
 #endif
@@ -1088,6 +1239,16 @@ struct hsddp_batch {
     // shared-memory wavefronts per stage), four warps below (shorter dependent chain per problem when the GPU is not full)
     int sweep_kind = 2;
     int w1_min_blocks = 1036;      // (about one wave of k_sweep_w1, 148 SMs x 7 when it was set; measured flat between 800 and 2,072, 2 % worse at 3,000)
+    // phased driver, rounds of the four-warp sweep: regularisation retries of a problem that regularises run as candidates on
+    // sweep_spec blocks side by side (BatchPtrs::spec_list; 0 or 1: one after another on the problem's block).  Scratch per group:
+    // kSpecCap x (sweep_spec - 1) slices of max_stages x 312 + 600 doubles (0.55 GB for the benchmark: 4 groups, 60 stages, S = 8).
+    // 8 against 4 and off on 16,384 config-3 problems: 58.9-59.0 k, 57.5-57.7 k and 57.0-57.2 k solves/s (profiles/r03b_*)
+    int sweep_spec = 8;
+    static constexpr int kSpecCap = 128;
+    int* d_spec_int = nullptr;     // per group: list [kSpecCap] | arrival counters [kSpecCap] | list counters [2]; then spec_entry [P]
+    SpecRec* d_spec_rec = nullptr;
+    double* d_spec_out = nullptr;
+    size_t d_spec_int_cap = 0, d_spec_rec_cap = 0, d_spec_out_cap = 0;
     bool lr_w1 = true;             // phased driver: linear rollout as its own one-warp-per-problem kernel (k_lr_w1) between sweep and forward
     int* d_order = nullptr;        // persistent kernel: queue order by the previous solve's iteration counts (k_order_by_iterations)
     bool have_order = false, use_order = true;
@@ -1276,6 +1437,7 @@ void free_problem_allocs(hsddp_batch* b) {
     b->slot_refs.clear(); b->slot_free.clear();
     b->d_restart = nullptr; b->d_restart_x0 = nullptr; b->d_restart_cap = b->d_restart_x0_cap = 0;
     b->d_budget = nullptr; b->budget_rounds = -1;
+    b->d_spec_int = nullptr; b->d_spec_rec = nullptr; b->d_spec_out = nullptr; b->d_spec_int_cap = b->d_spec_rec_cap = b->d_spec_out_cap = 0;
     b->slots_marked = false;
 }
 
@@ -1361,6 +1523,7 @@ static int batch_init(hsddp_batch* b, int device) {
     CK(cudaFuncSetAttribute(k_sweep_w1, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
     CK(cudaFuncSetAttribute(k_lr_w1, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
     if (const char* e = getenv("HSDDP_W1_MIN_BLOCKS")) b->w1_min_blocks = atoi(e);  // tuning / experiments only
+    if (const char* e = getenv("HSDDP_SWEEP_SPEC")) { const int v = atoi(e); b->sweep_spec = (v >= 2 && v <= 32) ? v : 0; }
     if (const char* e = getenv("HSDDP_LR_W1")) b->lr_w1 = atoi(e) != 0;              // tuning / experiments only
     if (const char* e = getenv("HSDDP_QUEUE_ORDER")) b->use_order = atoi(e) != 0;   // tuning / experiments only
     if (const char* e = getenv("HSDDP_CLUSTER_LS")) b->cluster_ls = atoi(e) != 0;   // tuning / experiments only
@@ -1863,8 +2026,18 @@ static int solve_phased(hsddp_batch* b, const hsddp_options& o, bool hybrid) {
             CK(cudaEventCreateWithFlags(&b->gevent[g], cudaEventDisableTiming));
         }
     }
+    const bool use_block = b->sweep_kind != 1, use_w1 = b->sweep_kind != 0;
+    const int S = use_block && b->sweep_spec > 1 ? b->sweep_spec : 0, cap = hsddp_batch::kSpecCap;
+    const size_t slice = (size_t)b->bp.max_stages * 312 + 600, spec_ints = (size_t)G * (2 * cap + 2) + P;
+    if (S) {
+        int rs = scratch(b, &b->d_spec_int, &b->d_spec_int_cap, spec_ints);
+        if (!rs) rs = scratch(b, &b->d_spec_rec, &b->d_spec_rec_cap, (size_t)G * cap * S);
+        if (!rs) rs = scratch(b, &b->d_spec_out, &b->d_spec_out_cap, (size_t)G * cap * (S - 1) * slice);
+        if (rs) return rs;
+    }
     CK(cudaEventRecord(b->ev0, b->stream));
     CK(cudaMemsetAsync(b->d_count, 0, 2 * hsddp_batch::kMaxGroups * sizeof(int), b->stream));
+    if (S) CK(cudaMemsetAsync(b->d_spec_int, 0, spec_ints * sizeof(int), b->stream));
     k_iota<<<(P + 255) / 256, 256, 0, b->stream>>>(b->d_active[0], P);
     CK(cudaEventRecord(b->ev_fork, b->stream));
     // (restarted problems may have a larger budget for this solve: BatchPtrs::budget)
@@ -1872,7 +2045,6 @@ static int solve_phased(hsddp_batch* b, const hsddp_options& o, bool hybrid) {
     const int rounds = hybrid ? std::min(all_rounds, std::max(0, b->hybrid_rounds)) : all_rounds;
     ResumeLists rl{};
     rl.n = 0;
-    const bool use_block = b->sweep_kind != 1, use_w1 = b->sweep_kind != 0;
     int rc = HSDDP_OK;
     for (int g = 0; g < G && rc == HSDDP_OK; ++g) {
         const int lo = (int)((long long)P * g / G), n = (int)((long long)P * (g + 1) / G) - lo;
@@ -1888,11 +2060,18 @@ static int solve_phased(hsddp_batch* b, const hsddp_options& o, bool hybrid) {
         bp.active = list[0]; bp.n_active = nullptr; bp.next_active = list[1]; bp.next_count = cnt[1]; bp.zero_count = nullptr;
         k_phase<PH_BEGIN><<<n, kThreads, 0, st>>>(bp, o);
         b->n_solve_launches++;
+        int* spec = b->d_spec_int + (size_t)g * (2 * cap + 2);
+        if (S) {
+            bp.spec_list = spec; bp.spec_arrive = spec + cap; bp.spec_entry = b->d_spec_int + (size_t)G * (2 * cap + 2);
+            bp.spec_rec = b->d_spec_rec + (size_t)g * cap * S; bp.spec_out = b->d_spec_out + (size_t)g * cap * (S - 1) * slice;
+            bp.spec_S = S; bp.spec_cap = cap;
+        }
         for (int r = 1; r <= rounds; ++r) {
             const int cur = r & 1;
             bp.active = list[cur]; bp.n_active = cnt[cur]; bp.next_active = list[cur ^ 1]; bp.next_count = cnt[cur ^ 1]; bp.zero_count = cnt[cur ^ 1];
+            if (S) { bp.spec_count = spec + 2 * cap + cur; bp.spec_zero = spec + 2 * cap + (cur ^ 1); }
             k_phase<PH_PREP><<<n, kThreads, 0, st>>>(bp, o);
-            if (use_block) k_phase<PH_SWEEP><<<n, kThreads, 0, st>>>(bp, o);
+            if (use_block) k_phase<PH_SWEEP><<<n + (S ? cap * (S - 1) : 0), kThreads, 0, st>>>(bp, o);
             if (use_w1) k_sweep_w1<<<n, 32, 0, st>>>(bp, o);
             if (bp.lr_external) k_lr_w1<<<n, 32, 0, st>>>(bp, o);
             k_phase<PH_FORWARD><<<n, kThreads, 0, st>>>(bp, o);
@@ -2234,6 +2413,14 @@ int hsddp_batch_get_counters(hsddp_batch* b, unsigned long long out[4]) {
     CK(cudaStreamSynchronize(b->stream));
     CK(cudaMemcpy(out, b->bp.counters, sizeof(unsigned long long), cudaMemcpyDeviceToHost));
     out[1] = b->n_solve_launches; out[2] = b->n_step_launches; out[3] = 0;
+    return HSDDP_OK;
+}
+
+int hsddp_batch_get_speculation(hsddp_batch* b, unsigned long long out[3]) {
+    if (!b || !b->has_problems || !out) return HSDDP_ERR_ARG;
+    CK(cudaSetDevice(b->device));
+    CK(cudaStreamSynchronize(b->stream));
+    CK(cudaMemcpy(out, b->bp.counters + 1, 3 * sizeof(unsigned long long), cudaMemcpyDeviceToHost));
     return HSDDP_OK;
 }
 

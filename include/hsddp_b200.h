@@ -314,6 +314,10 @@ int hsddp_batch_event_elapsed_ms(hsddp_batch* b, int slot0, int slot1, float* ms
  * out[0] = sum over problems of (backward sweeps x stages), out[1] = k_solve launches, out[2] = k_step launches */
 int hsddp_batch_get_counters(hsddp_batch* b, unsigned long long out[4]);
 int hsddp_batch_reset_counters(hsddp_batch* b);
+/* regularisation retries run side by side (phased driver, HSDDP_SWEEP_SPEC), since set_problems/reset_counters:
+ * out[0] = problem-rounds speculated, out[1] = of those, rounds whose first PD attempt was not the first one,
+ * out[2] = rounds in which every candidate failed (the problem's block went on retrying alone) */
+int hsddp_batch_get_speculation(hsddp_batch* b, unsigned long long out[3]);
 /* per-phase cycle counters (all zero unless the library was built with -DHSDDP_PROFILE) */
 int hsddp_batch_get_profile(hsddp_batch* b, unsigned long long out[16]);
 
