@@ -26,8 +26,6 @@
 
 namespace hsddp {
 
-constexpr int hsddp_batch_max_groups = 16;
-
 // ---------------------------------------------------------------------------
 // iteration control
 // ---------------------------------------------------------------------------
@@ -501,19 +499,18 @@ __device__ inline void solve_block(Smem& sm, const BatchPtrs& bp) {
     solve_finish_block(sm, bp);
 }
 
-template <int MINB>
-__device__ __forceinline__ void solve_persistent(Smem& sm, const BatchPtrs& bp, const hsddp_options& opt, int cold_start);
+__device__ __forceinline__ void solve_persistent(Smem& sm, const BatchPtrs& bp, const hsddp_options& opt);
 
 // throughput build: HSDDP_MIN_BLOCKS resident blocks per SM (80 registers / thread)
-__global__ void __launch_bounds__(kThreads, HSDDP_MIN_BLOCKS) k_solve(BatchPtrs bp, hsddp_options opt, int cold_start) {
+__global__ void __launch_bounds__(kThreads, HSDDP_MIN_BLOCKS) k_solve(BatchPtrs bp, hsddp_options opt) {
     __shared__ Smem sm;
-    solve_persistent<0>(sm, bp, opt, cold_start);
+    solve_persistent(sm, bp, opt);
 }
 // latency build: the same code compiled for two resident blocks (255 registers / thread: nothing spills, nothing is
 // rematerialised); used when the batch does not fill the GPU anyway (single-solve latency, MPC tick of one robot)
-__global__ void __launch_bounds__(kThreads, 2) k_solve_lat(BatchPtrs bp, hsddp_options opt, int cold_start) {
+__global__ void __launch_bounds__(kThreads, 2) k_solve_lat(BatchPtrs bp, hsddp_options opt) {
     __shared__ Smem sm;
-    solve_persistent<1>(sm, bp, opt, cold_start);
+    solve_persistent(sm, bp, opt);
 }
 
 // latency build with the concurrent line search: one cluster of four blocks per problem (block rank 0 solves, ranks 1..3 evaluate
@@ -535,8 +532,7 @@ __global__ void __cluster_dims__(4, 1, 1) __launch_bounds__(kThreads, 2) k_solve
     }
 }
 
-template <int MINB>
-__device__ __forceinline__ void solve_persistent(Smem& sm, const BatchPtrs& bp, const hsddp_options& opt, int cold_start) {
+__device__ __forceinline__ void solve_persistent(Smem& sm, const BatchPtrs& bp, const hsddp_options& opt) {
     if (threadIdx.x == 0) assign_rotation(bp.sm_slots, sm.rot);
     for (;;) {
         __syncthreads();
@@ -550,7 +546,6 @@ __device__ __forceinline__ void solve_persistent(Smem& sm, const BatchPtrs& bp, 
         bind_problem(sm, bp, pid);
         if (threadIdx.x == 0) sm.opt = opt;
         __syncthreads();
-        if (cold_start) cold_start_block(sm);
 #ifdef HSDDP_PROFILE
         if (threadIdx.x == 0) for (int i = 0; i < 16; ++i) sm.profacc[i] = 0;
         __syncthreads();
@@ -560,47 +555,6 @@ __device__ __forceinline__ void solve_persistent(Smem& sm, const BatchPtrs& bp, 
 #ifdef HSDDP_PROFILE
         if (threadIdx.x == 0) for (int i = 0; i < 16; ++i) atomicAdd(&sm.prof[i], sm.profacc[i]);
 #endif
-    }
-}
-
-// Tail of a phased solve (hybrid driver): the problems still running after the phased rounds -- listed per group in HBM, the
-// lengths known only on the device -- are finished by a persistent kernel that resumes solve() at the top of a DDP iteration.
-// Late rounds of a phased solve are latency-bound (every round costs at least one problem's iteration, however few problems
-// are left); here every survivor gets a block of its own and runs at single-problem speed.
-struct ResumeLists {
-    const int* list[hsddp_batch_max_groups];
-    const int* count[hsddp_batch_max_groups];
-    int n;
-};
-template <int MINB>
-__global__ void __launch_bounds__(kThreads, MINB) k_solve_resume(BatchPtrs bp, hsddp_options opt, ResumeLists rl) {
-    __shared__ Smem sm;
-    if (threadIdx.x == 0) assign_rotation(bp.sm_slots, sm.rot);
-    for (;;) {
-        __syncthreads();
-        if (threadIdx.x == 0) {
-            int q = atomicAdd(bp.work_counter, 1), pid = -1;
-            for (int g = 0; g < rl.n; ++g) {
-                const int c = *rl.count[g];
-                if (q < c) { pid = rl.list[g][q]; break; }
-                q -= c;
-            }
-            sm.ibuf[3] = pid;
-        }
-        __syncthreads();
-        const int pid = sm.ibuf[3];
-        if (pid < 0) break;
-        bind_problem(sm, bp, pid);
-        if (threadIdx.x == 0) sm.opt = opt;
-        __syncthreads();
-        while (sm.ctl.active) {  // (a listed problem is running: its state was saved at the end of a forward phase)
-            iter_prep_block(sm, bp);
-            iter_sweep_block(sm, bp);
-            if (!sm.ctl.active) break;
-            iter_forward_block(sm, bp);
-        }
-        solve_finish_block(sm, bp);
-        if (threadIdx.x == 0) { bp.state[pid] = sm.st; bp.ctl[pid] = sm.ctl; }
     }
 }
 
@@ -1225,20 +1179,16 @@ struct hsddp_batch {
     std::vector<DevSchedule> h_sched;
     std::vector<int> h_sched_id;
     bool has_problems = false;
-    bool cold = true;
-    float last_ms = 0.f;
     int* d_ok = nullptr;
     double* d_darg = nullptr;
     // phased driver (one kernel per solve phase over the running problems)
     int solve_mode = 0;            // 0 auto, 1 persistent k_solve, 2 phased k_phase<...>
     int* d_active[2] = {nullptr, nullptr};
     int* d_count = nullptr;
-    int last_rounds = 0;
-    // phased driver's backward-sweep kernel: 0 four warps per problem (k_phase<PH_SWEEP>), 1 one warp per problem (k_sweep_w1),
-    // 2 auto: one warp per problem for launches of at least `w1_min_blocks` problems (full waves: fewer instructions and
-    // shared-memory wavefronts per stage), four warps below (shorter dependent chain per problem when the GPU is not full)
-    int sweep_kind = 2;
-    int w1_min_blocks = 1036;      // (about one wave of k_sweep_w1, 148 SMs x 7 when it was set; measured flat between 800 and 2,072, 2 % worse at 3,000)
+    // phased driver's backward-sweep kernel, chosen per round on the device: one warp per problem (k_sweep_w1) for rounds of at
+    // least kSweepW1Min running problems (full waves: fewer instructions and shared-memory wavefronts per stage), four warps
+    // (k_phase<PH_SWEEP>) below (shorter dependent chain per problem when the GPU is not full)
+    static constexpr int kSweepW1Min = 1036;  // (about one wave of k_sweep_w1, 148 SMs x 7 when it was set; measured flat between 800 and 2,072, 2 % worse at 3,000)
     // phased driver, rounds of the four-warp sweep: regularisation retries of a problem that regularises run as candidates on
     // sweep_spec blocks side by side (BatchPtrs::spec_list; 0 or 1: one after another on the problem's block).  Scratch per group:
     // kSpecCap x (sweep_spec - 1) slices of max_stages x 312 + 600 doubles (0.55 GB for the benchmark: 4 groups, 60 stages, S = 8).
@@ -1251,14 +1201,11 @@ struct hsddp_batch {
     size_t d_spec_int_cap = 0, d_spec_rec_cap = 0, d_spec_out_cap = 0;
     bool lr_w1 = true;             // phased driver: linear rollout as its own one-warp-per-problem kernel (k_lr_w1) between sweep and forward
     int* d_order = nullptr;        // persistent kernel: queue order by the previous solve's iteration counts (k_order_by_iterations)
-    bool have_order = false, use_order = true;
-    bool cluster_ls = true;        // latency kernel with the concurrent line search (k_solve_lat4) for batches of at most kClusterLsMax problems
+    bool have_order = false;
+    // latency kernel with the concurrent line search (k_solve_lat4) for batches of at most kClusterLsMax problems
     static constexpr int kClusterLsMax = 32;  // 4 blocks per problem: every block of every cluster still gets an SM of its own (148 SMs); beyond that the helpers compete with the solving blocks (64 problems: 13.0 ms without, 13.8 ms with)
-    static constexpr int kMaxGroups = 16;  // (default phased_groups = 8; HSDDP_PHASED_GROUPS may raise it for experiments)
-    int phased_min_group = 1024;   // smallest index range the phased driver drives on its own stream
-    // hybrid driver (mid-size batches): phased rounds while the GPU is full, then a persistent kernel finishes the survivors
-    int hybrid_rounds = 20, hybrid_groups = 4, hybrid_min_group = 256;
-    int phased_groups = 4;         // index ranges driven concurrently on their own streams (config 3, 16,384 problems, round 2: 1: 381 ms, 2: 354, 4: 336, 8: 341, 16: 354)
+    static constexpr int kMaxGroups = 4;  // index ranges the phased driver drives concurrently on their own streams (config 3, 16,384 problems, round 2: 1: 381 ms, 2: 354, 4: 336, 8: 341, 16: 354)
+    static constexpr int kPhasedMinGroup = 1024;  // smallest index range the phased driver drives on its own stream
     cudaStream_t gstream[kMaxGroups] = {};
     cudaEvent_t gevent[kMaxGroups] = {};
     cudaEvent_t ev_fork = nullptr;
@@ -1485,7 +1432,6 @@ int launch_step(hsddp_batch* b, const hsddp_options* opt, int op, double arg, do
     b->n_step_launches++;
     if (ok_host) CK(cudaMemcpyAsync(ok_host, b->d_ok, sizeof(int) * b->bp.n_problems, cudaMemcpyDeviceToHost, b->stream));
     if (sync || ok_host) CK(cudaStreamSynchronize(b->stream));
-    if (op != OP_RESET) b->cold = false;
     return HSDDP_OK;
 }
 
@@ -1507,30 +1453,11 @@ static int batch_init(hsddp_batch* b, int device) {
     b->n_sm = prop.multiProcessorCount;
     CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&b->blocks_per_sm, k_solve, kThreads, 0));
     if (b->blocks_per_sm < 1) b->blocks_per_sm = 1;
-    if (const char* e = getenv("HSDDP_BLOCKS_PER_SM")) {  // tuning / experiments only
-        const int v = atoi(e);
-        if (v >= 1 && v <= b->blocks_per_sm) b->blocks_per_sm = v;
-    }
     CK(cudaEventCreateWithFlags(&b->ev_fork, cudaEventDisableTiming));
-    if (const char* e = getenv("HSDDP_PHASED_GROUPS")) {  // tuning / experiments only
-        const int v = atoi(e);
-        if (v >= 1 && v <= hsddp_batch::kMaxGroups) b->phased_groups = v;
-    }
-    if (const char* e = getenv("HSDDP_PHASED_MIN_GROUP")) { const int v = atoi(e); if (v >= 1) b->phased_min_group = v; }  // tuning / experiments only
-    if (const char* e = getenv("HSDDP_HYBRID_ROUNDS")) b->hybrid_rounds = atoi(e);  // tuning / experiments only
-    if (const char* e = getenv("HSDDP_HYBRID_GROUPS")) { const int v = atoi(e); if (v >= 1 && v <= hsddp_batch::kMaxGroups) b->hybrid_groups = v; }
-    if (const char* e = getenv("HSDDP_SWEEP_KIND")) b->sweep_kind = atoi(e);  // tuning / experiments only
     CK(cudaFuncSetAttribute(k_sweep_w1, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
     CK(cudaFuncSetAttribute(k_lr_w1, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-    if (const char* e = getenv("HSDDP_W1_MIN_BLOCKS")) b->w1_min_blocks = atoi(e);  // tuning / experiments only
     if (const char* e = getenv("HSDDP_SWEEP_SPEC")) { const int v = atoi(e); b->sweep_spec = (v >= 2 && v <= 32) ? v : 0; }
     if (const char* e = getenv("HSDDP_LR_W1")) b->lr_w1 = atoi(e) != 0;              // tuning / experiments only
-    if (const char* e = getenv("HSDDP_QUEUE_ORDER")) b->use_order = atoi(e) != 0;   // tuning / experiments only
-    if (const char* e = getenv("HSDDP_CLUSTER_LS")) b->cluster_ls = atoi(e) != 0;   // tuning / experiments only
-    if (const char* e = getenv("HSDDP_SOLVE_MODE")) {  // tuning / experiments only
-        const int v = atoi(e);
-        if (v >= 0 && v <= 3) b->solve_mode = v;
-    }
     return HSDDP_OK;
 }
 
@@ -1760,7 +1687,6 @@ int hsddp_batch_mpc_update(hsddp_batch* b) {
     CK(cudaMemcpyAsync(&err, b->d_mpc_err, sizeof(int), cudaMemcpyDeviceToHost, b->stream));
     CK(cudaStreamSynchronize(b->stream));
     b->h_sched_stale = true;
-    b->cold = false;
     b->have_order = false;  // (the queue order of the previous problem layout is still a good hint, but the solve after a tick is 2 iterations long)
     if (err) {
         g_last_error = err == 1 ? "receding-horizon update: the reference table is exhausted" : "receding-horizon update: schedule exceeds HSDDP_MAX_PHASES / node capacity";
@@ -1963,9 +1889,7 @@ int hsddp_batch_set_initial_condition(hsddp_batch* b, const double* x0) {
 
 int hsddp_batch_reset(hsddp_batch* b) {
     // queued on the handle's stream without a host synchronise, so reset + solve run back to back
-    int rc = launch_step(b, nullptr, OP_RESET, 0.0, nullptr, nullptr, false);
-    if (rc == HSDDP_OK) b->cold = true;
-    return rc;
+    return launch_step(b, nullptr, OP_RESET, 0.0, nullptr, nullptr, false);
 }
 
 // Phased driver: every round advances all running problems by one DDP iteration with one launch per phase
@@ -2015,19 +1939,16 @@ __global__ void k_order_by_iterations(const hsddp_info* info, int n, int* order)
     }
 }
 
-static int solve_phased(hsddp_batch* b, const hsddp_options& o, bool hybrid) {
+static int solve_phased(hsddp_batch* b, const hsddp_options& o) {
     const int P = b->bp.n_problems;
-    int G = hybrid ? b->hybrid_groups : b->phased_groups;
-    G = std::min(G, std::max(1, P / (hybrid ? b->hybrid_min_group : b->phased_min_group)));  // problems per group at least ..._min_group
-    G = std::max(1, std::min(G, hsddp_batch::kMaxGroups));
+    const int G = std::min(hsddp_batch::kMaxGroups, std::max(1, P / hsddp_batch::kPhasedMinGroup));  // problems per group at least kPhasedMinGroup
     for (int g = 0; g < G; ++g) {
         if (!b->gstream[g]) {
             CK(cudaStreamCreateWithFlags(&b->gstream[g], cudaStreamNonBlocking));
             CK(cudaEventCreateWithFlags(&b->gevent[g], cudaEventDisableTiming));
         }
     }
-    const bool use_block = b->sweep_kind != 1, use_w1 = b->sweep_kind != 0;
-    const int S = use_block && b->sweep_spec > 1 ? b->sweep_spec : 0, cap = hsddp_batch::kSpecCap;
+    const int S = b->sweep_spec, cap = hsddp_batch::kSpecCap;
     const size_t slice = (size_t)b->bp.max_stages * 312 + 600, spec_ints = (size_t)G * (2 * cap + 2) + P;
     if (S) {
         int rs = scratch(b, &b->d_spec_int, &b->d_spec_int_cap, spec_ints);
@@ -2041,10 +1962,7 @@ static int solve_phased(hsddp_batch* b, const hsddp_options& o, bool hybrid) {
     k_iota<<<(P + 255) / 256, 256, 0, b->stream>>>(b->d_active[0], P);
     CK(cudaEventRecord(b->ev_fork, b->stream));
     // (restarted problems may have a larger budget for this solve: BatchPtrs::budget)
-    const int all_rounds = (int)std::min<long long>(std::max((long long)std::max(0, o.max_AL_iter) * (long long)std::max(0, o.max_DDP_iter), b->budget_rounds), 1000000LL);
-    const int rounds = hybrid ? std::min(all_rounds, std::max(0, b->hybrid_rounds)) : all_rounds;
-    ResumeLists rl{};
-    rl.n = 0;
+    const int rounds = (int)std::min<long long>(std::max((long long)std::max(0, o.max_AL_iter) * (long long)std::max(0, o.max_DDP_iter), b->budget_rounds), 1000000LL);
     int rc = HSDDP_OK;
     for (int g = 0; g < G && rc == HSDDP_OK; ++g) {
         const int lo = (int)((long long)P * g / G), n = (int)((long long)P * (g + 1) / G) - lo;
@@ -2054,7 +1972,7 @@ static int solve_phased(hsddp_batch* b, const hsddp_options& o, bool hybrid) {
         int* list[2] = {b->d_active[0] + lo, b->d_active[1] + lo};
         if (cudaStreamWaitEvent(st, b->ev_fork, 0) != cudaSuccess) { rc = HSDDP_ERR_CUDA; break; }
         BatchPtrs bp = b->bp;
-        bp.sweep_w1_min = b->sweep_kind == 0 ? 0 : b->sweep_kind == 1 ? 1 : b->w1_min_blocks;
+        bp.sweep_w1_min = hsddp_batch::kSweepW1Min;
         bp.lr_external = (b->lr_w1 && o.MS) ? 1 : 0;
         // round 0: begin (initial rollout, first outer iteration set-up) over every problem of the group
         bp.active = list[0]; bp.n_active = nullptr; bp.next_active = list[1]; bp.next_count = cnt[1]; bp.zero_count = nullptr;
@@ -2071,35 +1989,25 @@ static int solve_phased(hsddp_batch* b, const hsddp_options& o, bool hybrid) {
             bp.active = list[cur]; bp.n_active = cnt[cur]; bp.next_active = list[cur ^ 1]; bp.next_count = cnt[cur ^ 1]; bp.zero_count = cnt[cur ^ 1];
             if (S) { bp.spec_count = spec + 2 * cap + cur; bp.spec_zero = spec + 2 * cap + (cur ^ 1); }
             k_phase<PH_PREP><<<n, kThreads, 0, st>>>(bp, o);
-            if (use_block) k_phase<PH_SWEEP><<<n + (S ? cap * (S - 1) : 0), kThreads, 0, st>>>(bp, o);
-            if (use_w1) k_sweep_w1<<<n, 32, 0, st>>>(bp, o);
+            k_phase<PH_SWEEP><<<n + (S ? cap * (S - 1) : 0), kThreads, 0, st>>>(bp, o);
+            k_sweep_w1<<<n, 32, 0, st>>>(bp, o);
             if (bp.lr_external) k_lr_w1<<<n, 32, 0, st>>>(bp, o);
             k_phase<PH_FORWARD><<<n, kThreads, 0, st>>>(bp, o);
-            b->n_solve_launches += 3 + (use_block && use_w1 ? 1 : 0) + (bp.lr_external ? 1 : 0);
+            b->n_solve_launches += 4 + (bp.lr_external ? 1 : 0);
         }
         if (cudaGetLastError() != cudaSuccess) { rc = HSDDP_ERR_CUDA; g_last_error = "kernel launch failed in the phased driver"; }
-        // the survivors of the last round: list / counter the next round would have read
-        const int nxt = (rounds + 1) & 1;
-        rl.list[rl.n] = list[nxt]; rl.count[rl.n] = cnt[nxt]; rl.n++;
     }
-    b->last_rounds = rounds;
     // join (also on an error exit: the handle's stream continues after every group, so later calls never see half-finished state)
     for (int g = 0; g < G; ++g) {
         if (!b->gstream[g]) continue;
         if (cudaEventRecord(b->gevent[g], b->gstream[g]) == cudaSuccess) cudaStreamWaitEvent(b->stream, b->gevent[g], 0);
-    }
-    if (hybrid && rounds < all_rounds && rc == HSDDP_OK) {  // the tail: one persistent kernel over the survivors of every group
-        CK(cudaMemsetAsync(b->bp.work_counter, 0, sizeof(int), b->stream));
-        k_solve_resume<4><<<b->n_sm * 4, kThreads, 0, b->stream>>>(b->bp, o, rl);
-        CK(cudaGetLastError());
-        b->n_solve_launches++;
     }
     CK(cudaEventRecord(b->ev1, b->stream));
     return rc;
 }
 
 int hsddp_batch_set_solve_mode(hsddp_batch* b, int mode) {
-    if (!b || mode < 0 || mode > 3) return HSDDP_ERR_ARG;
+    if (!b || mode < 0 || mode > 2) return HSDDP_ERR_ARG;
     b->solve_mode = mode;
     return HSDDP_OK;
 }
@@ -2118,35 +2026,34 @@ int hsddp_batch_solve_async(hsddp_batch* b, const hsddp_options* opt) {
     if (rc) return rc;
     CK(cudaSetDevice(b->device));
     const hsddp_options o = opt ? *opt : default_options();
-    b->cold = false;
     // auto: the persistent kernel up to ~7 waves of blocks (its work queue visits the problems longest-first from the second
     // solve on, which keeps the tail short); beyond that the phased driver, whose phase-homogeneous kernels keep the
     // instruction cache hot and whose launch tails are hidden by driving four index ranges on their own streams
     // (measured on config 3, persistent vs phased, ms, final code of round 2: 2,048 problems 57 vs 69, 4,096: 98 vs 100,
     // 5,120: ~121 vs 117, 6,144: 145 vs 135, 8,192: 199 vs 163 -- profiles/r02an_*: the switch is at 5.5 waves of blocks, 4,884 problems)
     const bool phased = b->solve_mode == 2 || (b->solve_mode == 0 && 2 * b->bp.n_problems >= 11 * b->n_sm * b->blocks_per_sm);
-    if (phased || b->solve_mode == 3) {
-        rc = solve_phased(b, o, !phased);
+    if (phased) {
+        rc = solve_phased(b, o);
         if (rc == HSDDP_OK) rc = consume_budget(b);
         return rc;
     }
     CK(cudaMemsetAsync(b->bp.work_counter, 0, sizeof(int), b->stream));
     CK(cudaEventRecord(b->ev0, b->stream));
-    if (b->cluster_ls && b->bp.ls_mail && b->bp.n_problems <= hsddp_batch::kClusterLsMax && o.MS) {
+    if (b->bp.ls_mail && b->bp.n_problems <= hsddp_batch::kClusterLsMax && o.MS) {
         k_solve_lat4<<<4 * b->bp.n_problems, kThreads, 0, b->stream>>>(b->bp, o);
     } else if (b->bp.n_problems <= 2 * b->n_sm) {
-        k_solve_lat<<<b->bp.n_problems, kThreads, 0, b->stream>>>(b->bp, o, 0);
+        k_solve_lat<<<b->bp.n_problems, kThreads, 0, b->stream>>>(b->bp, o);
     } else {
         const int grid = std::min(b->bp.n_problems, b->n_sm * b->blocks_per_sm);
         BatchPtrs bp = b->bp;
-        bp.order = (b->use_order && b->have_order) ? b->d_order : nullptr;
-        k_solve<<<grid, kThreads, 0, b->stream>>>(bp, o, 0);
+        bp.order = b->have_order ? b->d_order : nullptr;
+        k_solve<<<grid, kThreads, 0, b->stream>>>(bp, o);
     }
     CK(cudaGetLastError());
     b->n_solve_launches++;
     CK(cudaEventRecord(b->ev1, b->stream));
     if ((rc = consume_budget(b))) return rc;
-    if (b->use_order && b->bp.n_problems > 2 * b->n_sm) {  // (after the timed region of last_solve_ms: ~10 us, part of every bench step)
+    if (b->bp.n_problems > 2 * b->n_sm) {  // (after the timed region of last_solve_ms: ~10 us, part of every bench step)
         k_order_by_iterations<<<1, 256, 0, b->stream>>>(b->bp.info, b->bp.n_problems, b->d_order);
         CK(cudaGetLastError());
         b->n_solve_launches++;
@@ -2346,7 +2253,6 @@ int hsddp_batch_set_array(hsddp_batch* b, int which, const double* in) {
     CK(cudaSetDevice(b->device));
     CK(cudaMemcpyAsync(*a.field, in, (size_t)b->bp.n_problems * a.bytes(), cudaMemcpyHostToDevice, b->stream));
     CK(cudaStreamSynchronize(b->stream));
-    b->cold = false;
     return HSDDP_OK;
     });
 }

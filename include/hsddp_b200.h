@@ -210,13 +210,11 @@ int hsddp_batch_sync(hsddp_batch* b);
  *                  second solve of a problem set on, the queue visits the problems in the order of their previous
  *                  work (iterations, backward sweeps, trials), longest first (a scheduling hint only: results do not depend on it)
  *   2 phased     — per DDP iteration one kernel per phase (prep / backward sweep / linear rollout / forward sweep) over the problems
- *                  still running, up to eight index ranges driven concurrently on their own streams.  The list of
+ *                  still running, up to four index ranges driven concurrently on their own streams.  The list of
  *                  running problems and its length stay in HBM, so the whole solve is queued without a host round trip
  *                  and hsddp_batch_solve_async returns as soon as the launches are queued
- *   3 hybrid     — the phased driver for the first 20 DDP iterations, then a persistent kernel resumes the problems that
- *                  are still running (late phased rounds are latency-bound).  Opt-in: measured 11 % faster than
- *                  persistent at 1,024 problems, 4 % at 4,096, 4 % slower at 2,048
- *   0 auto       — phased when the batch fills the GPU five and a half times over (>= 4,884 problems on a B200). */
+ *   0 auto       — phased when the batch fills the GPU five and a half times over (>= 4,884 problems on a B200).
+ * Any other mode is refused with HSDDP_ERR_ARG. */
 int hsddp_batch_set_solve_mode(hsddp_batch* b, int mode);
 /* milliseconds of the last solve kernel, CUDA events on the handle's stream */
 int hsddp_batch_last_solve_ms(hsddp_batch* b, float* ms);

@@ -11,11 +11,12 @@ SCAN = 8192
 
 
 def _handle(pkg, monkeypatch, spec):
-    # knobs are read at handle creation; the four-warp sweep in every round makes every round eligible
-    monkeypatch.setenv("HSDDP_SOLVE_MODE", "2")
-    monkeypatch.setenv("HSDDP_SWEEP_KIND", "0")
+    # HSDDP_SWEEP_SPEC is read at handle creation.  The batch (at most 32 problems) never reaches the one-warp sweep's
+    # threshold, so every round of the phased driver takes the four-warp sweep and is eligible
     monkeypatch.setenv("HSDDP_SWEEP_SPEC", str(spec))
-    return pkg.MultiPhaseDDPBatch(0)
+    B = pkg.MultiPhaseDDPBatch(0)
+    B.set_solve_mode(2)
+    return B
 
 
 def _solve(pkg, monkeypatch, w, spec, opt):
@@ -55,7 +56,7 @@ def regularising(pkg, workloads):
 
 
 @pytest.mark.parametrize("case", ["window", "overflow"])
-def test_speculated_retries_match_sequential(pkg, workloads, monkeypatch, regularising, case):
+def test_speculated_retries_match_sequential_in_the_phased_driver(pkg, workloads, monkeypatch, regularising, case):
     entries, _ = regularising
     w = workloads.from_entries(pkg, "regularising", entries)
     # overflow: r_2 = 1e3 > 1e2, so every problem whose sweep fails at reg 1e-3 ends in REG_OVERFLOW (candidates 2.. never run)

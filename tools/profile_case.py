@@ -9,8 +9,10 @@ wl = importlib.import_module("hkd-mpc_b200.workloads")
 n = int(sys.argv[1]) if len(sys.argv) > 1 else 296
 cfg = sys.argv[2] if len(sys.argv) > 2 else "config2"
 reps = int(sys.argv[3]) if len(sys.argv) > 3 else 1
+mode = int(sys.argv[4]) if len(sys.argv) > 4 else 0  # solve mode: 0 auto, 1 persistent, 2 phased
 w = getattr(wl, cfg)(pkg, n)
 B = pkg.MultiPhaseDDPBatch(0)
+B.set_solve_mode(mode)
 B.set_problems(w.schedules, w.schedule_id)
 B.set_initial_condition(w.x0)
 for _ in range(reps):

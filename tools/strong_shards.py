@@ -8,7 +8,7 @@ sys.path.insert(0, ROOT)
 pkg = importlib.import_module("hkd-mpc_b200")
 wl = importlib.import_module("hkd-mpc_b200.workloads")
 n = int(sys.argv[1]) if len(sys.argv) > 1 else 2048
-modes = [int(m) for m in (sys.argv[2] if len(sys.argv) > 2 else "1,3").split(",")]
+modes = [int(m) for m in (sys.argv[2] if len(sys.argv) > 2 else "1,2").split(",")]
 interleaved = len(sys.argv) > 3 and sys.argv[3] == "interleaved"  # shard r = problems r, r + R, r + 2 R, ... instead of a contiguous range
 R = 16384 // n
 for first in (range(R) if interleaved else range(0, 16384, n)):
