@@ -87,7 +87,7 @@ struct DevSchedule {
     unsigned nmask[MAXPH];  // contact after the phase
     long long ref_off;      // node offset of this schedule inside the concatenated reference arrays
     double dt;
-    unsigned char ph_of_stage[HSDDP_MAX_STAGES];           // filled on the host (hsddp_batch_set_problems)
+    unsigned char ph_of_stage[HSDDP_MAX_STAGES];           // filled by layout_phases
     unsigned char ph_of_node[HSDDP_MAX_STAGES + MAXPH];
     // shooting set of the phase: nodes 0 .. ss_size-1 (SinglePhase::update_SS_config).  horizon + 1 = every node (what
     // HKDProblem::initialization sets); after a receding-horizon update the LAST phase can have fewer: 0 for a phase created
@@ -98,6 +98,27 @@ struct DevSchedule {
     unsigned char tdmask[2][MAXPH];
 };
 static_assert(sizeof(DevSchedule) % 4 == 0, "bind_problem copies the schedule word by word");
+
+// The phase layout of a schedule from horizon[0 .. n_phases): phase p has horizon[p] stages and horizon[p] + 1 nodes, laid
+// out one phase after the other (node_off, stage_off, ph_of_stage, ph_of_node and the counts).  False, with the table partly
+// written, when a phase is empty or the schedule has more than stage_cap stages or node_cap nodes.  The caps must not exceed
+// the table sizes, HSDDP_MAX_STAGES and HSDDP_MAX_STAGES + MAXPH.
+__host__ __device__ inline bool layout_phases(DevSchedule& d, int n_phases, int stage_cap, int node_cap) {
+    int so = 0, no = 0;
+    for (int p = 0; p < n_phases; ++p) {
+        const int h = d.horizon[p];
+        if (h < 1 || so + h > stage_cap || no + h + 1 > node_cap) return false;
+        d.node_off[p] = no; d.stage_off[p] = so;
+        for (int k = 0; k < h; ++k) d.ph_of_stage[so + k] = (unsigned char)p;
+        for (int k = 0; k <= h; ++k) d.ph_of_node[no + k] = (unsigned char)p;
+        no += h + 1; so += h;
+    }
+    d.n_phases = n_phases; d.n_stages = so; d.n_nodes = no;
+    return true;
+}
+
+// legs that go from swing (not in the phase's contact mask) to stance (in the contact after it): one touchdown-constraint object
+__host__ __device__ inline unsigned touchdown_legs(unsigned cmask, unsigned nmask) { return ~cmask & nmask & 15u; }
 
 // solver scalars of one problem (MultiPhaseDDP.h:92-104) + bookkeeping
 struct SolverState {

@@ -735,7 +735,12 @@ struct GaitLib {
     const int* row_off;                          // first row of gait g
     const int* n_rows;                           // rows of gait g
     const float* dt;                             // sample period of gait g
+    float plan;                                  // plan duration of every schedule of the batch
+    int node_stride;                             // reference rows per schedule slot
 };
+
+// dt_sim (one MPC tick) and dt_mpc (the stage length) of the reference's MPC loop: both 0.01 s
+constexpr float kTickDt = 0.01f;
 
 // Per-schedule state of the receding-horizon update (HKDProblemData of HKDProblem.h:28-66 + QuadReference::k_cur / t_cur):
 // everything HKDProblem::update needs beyond the phase table itself.
@@ -766,16 +771,24 @@ __device__ __forceinline__ int ref_index_at(float t, float dt, int sz) {
     return k;
 }
 
-// pass 1: phase tables, one thread per schedule.  status[i] != 0 marks an unusable window.  Schedule i goes to slot
-// slot[i] (nullptr: slot i) and may have at most stage_cap stages.
-__global__ void k_build_phase_tables(GaitLib lib, int n_sched, const int* sched_gait, const int* sched_window, float plan, int node_stride,
-                                     DevSchedule* out, int* status, MpcSched* mpc, const int* slot, int stage_cap) {
+// samples in the reference window of a schedule: plan duration over the gait's sample period, plus one
+__device__ __forceinline__ int ref_window_size(const GaitLib& lib, float dtg) { return (int)roundf(__fdiv_rn(lib.plan, dtg)) + 1; }
+
+__device__ __forceinline__ unsigned contact_mask_at(const GaitLib& lib, size_t row) {
+    const int* c = lib.contact + 4 * row;
+    return (c[0] ? 1u : 0u) | (c[1] ? 2u : 0u) | (c[2] ? 4u : 0u) | (c[3] ? 8u : 0u);
+}
+
+// pass 1: phase tables and update state, one thread per schedule.  status[i] != 0 marks an unusable window.  Schedule i
+// goes to slot slot[i] (nullptr: slot i) and may have at most stage_cap stages.
+__global__ void k_build_phase_tables(GaitLib lib, int n_sched, const int* sched_gait, const int* sched_window, const int* slot, int stage_cap,
+                                     DevSchedule* out, MpcSched* mpc, int* status) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n_sched) return;
     const int si = slot ? slot[i] : i;
     const int gi = sched_gait[i], k0 = sched_window[i];
     const float dtg = lib.dt[gi];
-    const int sz = (int)roundf(__fdiv_rn(plan, dtg)) + 1;
+    const int sz = ref_window_size(lib, dtg);
     DevSchedule d;
     memset(&d, 0, sizeof d);
     MpcSched m;
@@ -783,102 +796,80 @@ __global__ void k_build_phase_tables(GaitLib lib, int n_sched, const int* sched_
     m.new_td_phase = -1; m.new_td_object = -1;
     int st = 0;
     if (k0 < 0 || k0 + sz >= lib.n_rows[gi]) st = 1;
-    const int* contact = lib.contact + 4 * (size_t)(lib.row_off[gi] + k0);
-    const float dt_sim = 0.01f, dt_mpc = 0.01f;
-    int n_phases = 0, so = 0, no = 0;
+    const size_t row0 = (size_t)(lib.row_off[gi] + k0);
     if (!st) {
-        int cprev[4], ccur[4];
+        int n_phases = 0;
         float phase_start = 0.f, t = 0.f;
-        { const int* c = contact + 4 * ref_index_at(t, dtg, sz); for (int l = 0; l < 4; ++l) cprev[l] = c[l]; }
-        while (approx_leq_f(t, plan)) {
-            { const int* c = contact + 4 * ref_index_at(t, dtg, sz); for (int l = 0; l < 4; ++l) ccur[l] = c[l]; }
+        size_t rprev = row0 + ref_index_at(t, dtg, sz);  // sample whose contact flags the current phase has
+        while (approx_leq_f(t, lib.plan)) {
+            const size_t r = row0 + ref_index_at(t, dtg, sz);
             bool change = false;
-            for (int l = 0; l < 4; ++l) change = change || (ccur[l] != cprev[l]);
-            if (change || approx_geq_f(t, plan)) {
+            for (int l = 0; l < 4; ++l) change = change || (lib.contact[4 * r + l] != lib.contact[4 * rprev + l]);
+            if (change || approx_geq_f(t, lib.plan)) {
                 if (n_phases >= MAXPH) { st = 2; break; }
-                const int hz = (int)roundf(__fdiv_rn(__fsub_rn(t, phase_start), dt_sim));
-                if (hz < 1 || so + hz > stage_cap) { st = 2; break; }
-                d.horizon[n_phases] = hz; d.node_off[n_phases] = no; d.stage_off[n_phases] = so;
-                unsigned cm = 0;
-                for (int l = 0; l < 4; ++l) cm |= (cprev[l] ? 1u : 0u) << l;
-                d.cmask[n_phases] = cm;
-                // phase start time, kept as float bits in nmask until the table is complete
-                d.nmask[n_phases] = __float_as_uint(phase_start);
+                const int hz = (int)roundf(__fdiv_rn(__fsub_rn(t, phase_start), kTickDt));
+                d.horizon[n_phases] = hz;
+                d.cmask[n_phases] = contact_mask_at(lib, rprev);
                 d.ss_size[n_phases] = (unsigned char)(hz + 1);  // update_SS_config(horizon + 1), HKDProblem.cpp:104
                 m.start[n_phases] = phase_start; m.end[n_phases] = t; m.reach_end[n_phases] = 0; m.has_tconstr[n_phases] = 1;
-                for (int k = 0; k < hz; ++k) d.ph_of_stage[so + k] = (unsigned char)n_phases;
-                for (int k = 0; k <= hz; ++k) d.ph_of_node[no + k] = (unsigned char)n_phases;
-                no += hz + 1; so += hz;
                 ++n_phases;
-                for (int l = 0; l < 4; ++l) cprev[l] = ccur[l];
+                rprev = r;
                 phase_start = t;
             }
-            t = __fadd_rn(t, dt_sim);
+            t = __fadd_rn(t, kTickDt);
         }
+        if (!st && (n_phases < 1 || !layout_phases(d, n_phases, stage_cap, lib.node_stride))) st = 2;
     }
-    if (!st && (n_phases < 1 || no > node_stride)) st = 2;
-    d.n_phases = n_phases; d.n_stages = so; d.n_nodes = no; d.dt = (double)dt_sim;
-    d.ref_off = (long long)si * node_stride;
+    d.dt = (double)kTickDt;
+    d.ref_off = (long long)si * lib.node_stride;
     out[si] = d;
     status[i] = st;
     m.status = st;
-    if (mpc) mpc[si] = m;
-    (void)dt_mpc;
+    mpc[si] = m;
 }
 
-// pass 2: reference rows, one thread per (schedule, node); also turns the start times parked in nmask into the
-// contact-after-phase masks (thread of node 0 of each schedule, after every node of that schedule has read them —
-// so the start times are first copied to shared memory by the whole block).
-__global__ void k_build_reference_rows(GaitLib lib, int n_sched, const int* sched_gait, const int* sched_window, float plan, int node_stride,
-                                       DevSchedule* scheds, const int* status, double* xr, double* ur, double* prel, double* xinit, const int* slot) {
+// pass 2: reference rows, one block per entry i: schedule slot slot[i] (nullptr: slot i) of gait gait[i] and initial window
+// window[i], whose phase table and update state are in place.  Entries of a free slot (gait -1) or of a failed build or
+// update are skipped.  xinit != nullptr: the call completes a build (pass 1): it also writes the initial-guess rows and the
+// contact after each phase with its touchdown legs.
+__global__ void k_reference_rows(GaitLib lib, int n, const int* gait, const int* window, const int* slot,
+                                 DevSchedule* scheds, const MpcSched* mpc, double* xr, double* ur, double* prel, double* xinit) {
     const int i = blockIdx.x;
-    if (i >= n_sched || status[i]) return;
-    __shared__ float start_time[MAXPH];
-    DevSchedule& d = scheds[slot ? slot[i] : i];
-    const int n_phases = d.n_phases;
-    if (threadIdx.x < n_phases) start_time[threadIdx.x] = __uint_as_float(d.nmask[threadIdx.x]);
-    __syncthreads();
-    const int gi = sched_gait[i], k0 = sched_window[i];
+    if (i >= n) return;
+    const int si = slot ? slot[i] : i, gi = gait[i];
+    if (gi < 0 || mpc[si].status) return;
+    DevSchedule& d = scheds[si];
+    const MpcSched& m = mpc[si];
     const float dtg = lib.dt[gi];
-    const int sz = (int)roundf(__fdiv_rn(plan, dtg)) + 1;
-    const size_t row0 = (size_t)(lib.row_off[gi] + k0);
-    const float dt_sim = 0.01f, dt_mpc = 0.01f;
-    for (int n = threadIdx.x; n < d.n_nodes; n += blockDim.x) {
-        const int ph = d.ph_of_node[n], k = n - d.node_off[ph];
-        const size_t node = (size_t)d.ref_off + n;
-        // time seen by the cost callbacks: float(t_offset + k*dt), dt widened to double (SinglePhase.cpp:243,254)
-        const float t_offset = __fsub_rn(start_time[ph], start_time[0]);
+    const int sz = ref_window_size(lib, dtg);
+    const size_t row0 = (size_t)(lib.row_off[gi] + window[i] + m.k_cur);
+    // HKDReference.cpp:33-56 (Q12): foot placement if the SAMPLE's contact flag is set, else joint angle
+    auto state_row = [&](size_t r, double* x) {
+        for (int j = 0; j < 12; ++j) x[j] = lib.body_state[12 * r + j];
+        for (int l = 0; l < 4; ++l)
+            for (int j = 0; j < 3; ++j)
+                x[12 + 3 * l + j] = (lib.contact[4 * r + l] > 0) ? lib.foot[12 * r + 3 * l + j] : lib.qJ[12 * r + 3 * l + j];
+    };
+    for (int nd = threadIdx.x; nd < d.n_nodes; nd += blockDim.x) {
+        const int ph = d.ph_of_node[nd], k = nd - d.node_off[ph];
+        const size_t node = (size_t)d.ref_off + nd;
+        // time seen by the cost callbacks: float(t_offset + k*dt), t_offset = start - start[0] in float (set_time_offset),
+        // dt widened to double (SinglePhase.cpp:243,254)
+        const float t_offset = __fsub_rn(m.start[ph], m.start[0]);
         const float tc = (float)__dadd_rn((double)t_offset, __dmul_rn((double)k, d.dt));
-        const int kc = ref_index_at(tc, dtg, sz);
-        // time used for the initial guess: float(phase_start + k*dt_sim), all float (HKDProblem.cpp:86-90)
-        const float ti = __fadd_rn(start_time[ph], __fmul_rn((float)k, dt_sim));
-        const int ki = ref_index_at(ti, dtg, sz);
-#pragma unroll 1
-        for (int pass = 0; pass < 2; ++pass) {  // HKDReference.cpp:33-56 (Q12): foot placement if the SAMPLE's contact flag is set, else joint angle
-            const size_t r = row0 + (pass ? ki : kc);
-            double* x = (pass ? xinit : xr) + 24 * node;
-            for (int j = 0; j < 12; ++j) x[j] = lib.body_state[12 * r + j];
-            for (int l = 0; l < 4; ++l)
-                for (int j = 0; j < 3; ++j)
-                    x[12 + 3 * l + j] = (lib.contact[4 * r + l] > 0) ? lib.foot[12 * r + 3 * l + j] : lib.qJ[12 * r + 3 * l + j];
-        }
-        const size_t r = row0 + kc;
+        const size_t r = row0 + ref_index_at(tc, dtg, sz);
+        state_row(r, xr + 24 * node);
         for (int j = 0; j < 12; ++j) { ur[24 * node + j] = lib.grf[12 * r + j]; ur[24 * node + 12 + j] = 0.0; }  // qJd is never loaded: zeros
         for (int l = 0; l < 4; ++l)
             for (int j = 0; j < 3; ++j) prel[12 * node + 3 * l + j] = lib.foot[12 * r + 3 * l + j] - lib.body_state[12 * r + 3 + j];
+        // time used for the initial guess: float(phase_start + k*dt_sim), all float (HKDProblem.cpp:86-90)
+        if (xinit) state_row(row0 + ref_index_at(__fadd_rn(m.start[ph], __fmul_rn((float)k, kTickDt)), dtg, sz), xinit + 24 * node);
     }
-    __syncthreads();
-    if (threadIdx.x < n_phases) {  // contact after each phase (reset map / touchdown wiring), HKDProblem.cpp:268-299, Q17
+    if (xinit && threadIdx.x < d.n_phases) {  // contact after each phase (reset map / touchdown wiring), HKDProblem.cpp:268-299, Q17
         const int p = threadIdx.x;
-        unsigned nm;
-        if (p < n_phases - 1) nm = d.cmask[p + 1];
-        else {
-            const int* c = lib.contact + 4 * (row0 + ref_index_at(__fadd_rn(plan, dt_mpc), dtg, sz));
-            nm = 0;
-            for (int l = 0; l < 4; ++l) nm |= (c[l] ? 1u : 0u) << l;
-        }
+        const unsigned nm = p < d.n_phases - 1 ? d.cmask[p + 1] : contact_mask_at(lib, row0 + ref_index_at(__fadd_rn(lib.plan, kTickDt), dtg, sz));
         d.nmask[p] = nm;
-        d.tdmask[0][p] = (unsigned char)(~d.cmask[p] & nm & 15u);  // legs going swing -> stance: one touchdown-constraint object
+        d.tdmask[0][p] = (unsigned char)touchdown_legs(d.cmask[p], nm);
         d.tdmask[1][p] = 0;
     }
 }
@@ -890,16 +881,11 @@ __global__ void k_build_reference_rows(GaitLib lib, int n_sched, const int* sche
 //   k_mpc_update_schedules  one thread per schedule: QuadReference::step (QuadReference.cpp:33-47), front end (drop the first
 //                           node or the whole first phase), back end (grow the last phase or open a new one; add_tconstr_one_phase
 //                           when the last phase has reached its end), shooting sets -- with the reference's float time arithmetic
-//   k_mpc_reference_rows    the per-node reference rows of the shifted window (HKDReference.cpp:8-57)
+//   k_reference_rows        the per-node reference rows of the shifted window (HKDReference.cpp:8-57)
 //   k_mpc_shift             one block per problem: Trajectory::pop_front / push_back_state (TrajectoryManagement.cpp:118-207),
 //                           PathConstraintBase::pop_front / push_back (ConstraintsBase.h:271-280) on the problem-major arrays
 // ---------------------------------------------------------------------------
-__device__ __forceinline__ unsigned contact_mask_at(const GaitLib& lib, size_t row) {
-    const int* c = lib.contact + 4 * row;
-    return (c[0] ? 1u : 0u) | (c[1] ? 2u : 0u) | (c[2] ? 4u : 0u) | (c[3] ? 8u : 0u);
-}
-
-__global__ void k_mpc_update_schedules(GaitLib lib, int n_sched, const int* sched_gait, const int* sched_window, float plan, int node_stride,
+__global__ void k_mpc_update_schedules(GaitLib lib, int n_sched, const int* sched_gait, const int* sched_window,
                                        DevSchedule* scheds, MpcSched* mpc, int* err) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n_sched) return;
@@ -908,18 +894,17 @@ __global__ void k_mpc_update_schedules(GaitLib lib, int n_sched, const int* sche
     DevSchedule d = scheds[i];
     MpcSched m = mpc[i];
     const float dtg = lib.dt[gi];
-    const float dt_sim = 0.01f, dt_mpc = 0.01f;
-    const int sz = (int)roundf(__fdiv_rn(plan, dtg)) + 1;
+    const int sz = ref_window_size(lib, dtg);
     m.old_n_nodes = d.n_nodes;
     m.new_td_phase = -1; m.new_td_object = -1;
     // QuadReference::step(dt_sim)
-    for (int q = 1; approx_leq_f(__fmul_rn((float)q, dtg), dt_sim); ++q) { m.k_cur++; m.t_cur = __fadd_rn(m.t_cur, dtg); }
-    const float new_start = m.t_cur, new_end = __fadd_rn(m.t_cur, plan);
+    for (int q = 1; approx_leq_f(__fmul_rn((float)q, dtg), kTickDt); ++q) { m.k_cur++; m.t_cur = __fadd_rn(m.t_cur, dtg); }
+    const float new_start = m.t_cur, new_end = __fadd_rn(m.t_cur, lib.plan);
     const size_t row0 = (size_t)(lib.row_off[gi] + sched_window[i] + m.k_cur);
     if (sched_window[i] + m.k_cur + sz >= lib.n_rows[gi]) { m.status = 1; mpc[i] = m; atomicMax(err, 1); return; }
     int n = d.n_phases;
     // ---- front end ----
-    m.start[0] = __fadd_rn(m.start[0], dt_sim);
+    m.start[0] = __fadd_rn(m.start[0], kTickDt);
     if (approx_leq_f(m.end[0], new_start)) {  // the first phase has shrunk to a point: pop_front_phase
         m.front_nodes = d.horizon[0] + 1; m.front_phase_popped = 1;
         for (int p = 0; p + 1 < n; ++p) {
@@ -939,7 +924,7 @@ __global__ void k_mpc_update_schedules(GaitLib lib, int n_sched, const int* sche
     if (change && m.reach_end[n - 1]) {
         if (n >= MAXPH) { m.status = 2; mpc[i] = m; atomicMax(err, 2); return; }
         m.start[n] = m.end[n - 1]; m.end[n] = new_end; m.reach_end[n] = 0; m.has_tconstr[n] = 0;
-        d.horizon[n] = (int)roundf(__fdiv_rn(__fsub_rn(m.end[n], m.start[n]), dt_sim));
+        d.horizon[n] = (int)roundf(__fdiv_rn(__fsub_rn(m.end[n], m.start[n]), kTickDt));
         d.cmask[n] = newc; d.nmask[n] = 0; d.tdmask[0][n] = 0; d.tdmask[1][n] = 0; d.ss_size[n] = 0;  // (SinglePhase::initialization clears SS_set)
         m.back_new_phase = 1;
         ++n;
@@ -950,9 +935,9 @@ __global__ void k_mpc_update_schedules(GaitLib lib, int n_sched, const int* sche
         m.back_new_phase = 0;
     }
     if (m.reach_end[n - 1]) {  // add_tconstr_one_phase(last phase): the contact after it is the reference's at plan_duration + dt_mpc
-        const unsigned nm = contact_mask_at(lib, row0 + ref_index_at(__fadd_rn(plan, dt_mpc), dtg, sz));
+        const unsigned nm = contact_mask_at(lib, row0 + ref_index_at(__fadd_rn(lib.plan, kTickDt), dtg, sz));
         d.nmask[n - 1] = nm; m.has_tconstr[n - 1] = 1;
-        const unsigned td = ~d.cmask[n - 1] & nm & 15u;
+        const unsigned td = touchdown_legs(d.cmask[n - 1], nm);
         if (td) {
             const int ob = d.tdmask[0][n - 1] ? (d.tdmask[1][n - 1] ? 2 : 1) : 0;
             if (ob >= 2) { m.status = 2; mpc[i] = m; atomicMax(err, 2); return; }  // (needs a one-sample contact blip in the reference)
@@ -961,46 +946,11 @@ __global__ void k_mpc_update_schedules(GaitLib lib, int n_sched, const int* sche
         }
     }
     // ---- shooting configuration (HKDProblem.cpp:205-221) and the derived tables ----
-    int so = 0, no = 0;
-    for (int p = 0; p < n; ++p) {
+    for (int p = 0; p < n; ++p)
         if ((p == n - 1 && d.horizon[p] > 2) || p < n - 1) d.ss_size[p] = (unsigned char)(d.horizon[p] + 1);
-        d.node_off[p] = no; d.stage_off[p] = so;
-        if (d.horizon[p] < 1 || so + d.horizon[p] > HSDDP_MAX_STAGES || no + d.horizon[p] + 1 > node_stride) { m.status = 2; mpc[i] = m; atomicMax(err, 2); return; }
-        for (int k = 0; k < d.horizon[p]; ++k) d.ph_of_stage[so + k] = (unsigned char)p;
-        for (int k = 0; k <= d.horizon[p]; ++k) d.ph_of_node[no + k] = (unsigned char)p;
-        no += d.horizon[p] + 1; so += d.horizon[p];
-    }
-    d.n_phases = n; d.n_stages = so; d.n_nodes = no;
+    if (!layout_phases(d, n, HSDDP_MAX_STAGES, lib.node_stride)) { m.status = 2; mpc[i] = m; atomicMax(err, 2); return; }
     scheds[i] = d;
     mpc[i] = m;
-}
-
-__global__ void k_mpc_reference_rows(GaitLib lib, int n_sched, const int* sched_gait, const int* sched_window, float plan,
-                                     const DevSchedule* scheds, const MpcSched* mpc, double* xr, double* ur, double* prel) {
-    const int i = blockIdx.x;
-    if (i >= n_sched || mpc[i].status || sched_gait[i] < 0) return;  // (gait -1: a free slot)
-    const DevSchedule& d = scheds[i];
-    const MpcSched& m = mpc[i];
-    const int gi = sched_gait[i];
-    const float dtg = lib.dt[gi];
-    const int sz = (int)roundf(__fdiv_rn(plan, dtg)) + 1;
-    const size_t row0 = (size_t)(lib.row_off[gi] + sched_window[i] + m.k_cur);
-    for (int n = threadIdx.x; n < d.n_nodes; n += blockDim.x) {
-        const int ph = d.ph_of_node[n], k = n - d.node_off[ph];
-        const size_t node = (size_t)d.ref_off + n;
-        // time seen by the cost callbacks: float(t_offset + k*dt), t_offset = start - start[0] in float (set_time_offset)
-        const float t_offset = __fsub_rn(m.start[ph], m.start[0]);
-        const float tc = (float)__dadd_rn((double)t_offset, __dmul_rn((double)k, d.dt));
-        const size_t r = row0 + ref_index_at(tc, dtg, sz);
-        double* x = xr + 24 * node;
-        for (int j = 0; j < 12; ++j) x[j] = lib.body_state[12 * r + j];
-        for (int l = 0; l < 4; ++l)
-            for (int j = 0; j < 3; ++j)
-                x[12 + 3 * l + j] = (lib.contact[4 * r + l] > 0) ? lib.foot[12 * r + 3 * l + j] : lib.qJ[12 * r + 3 * l + j];
-        for (int j = 0; j < 12; ++j) { ur[24 * node + j] = lib.grf[12 * r + j]; ur[24 * node + 12 + j] = 0.0; }
-        for (int l = 0; l < 4; ++l)
-            for (int j = 0; j < 3; ++j) prel[12 * node + 3 * l + j] = lib.foot[12 * r + 3 * l + j] - lib.body_state[12 * r + 3 + j];
-    }
 }
 
 // rows [shift, total) of a row-major array move down to [0, total - shift); the last `shift` rows are then filled by the caller.
@@ -1215,8 +1165,7 @@ struct hsddp_batch {
     GaitLib lib{};
     int *d_sched_gait = nullptr, *d_sched_window = nullptr, *d_mpc_err = nullptr;
     MpcSched* d_mpc = nullptr;
-    float plan = 0.f;
-    int node_stride = 0, n_sched = 0;
+    int n_sched = 0;
     bool h_sched_stale = false;
     cudaEvent_t ev_u0 = nullptr, ev_u1 = nullptr;
     int n_gaits = 0;
@@ -1261,6 +1210,14 @@ int dalloc_bytes(hsddp_batch* b, void** p, size_t bytes) {
 
 template <class T>
 int dalloc(hsddp_batch* b, T** p, size_t n) { return dalloc_bytes(b, (void**)p, n * sizeof(T)); }
+
+// *d := a new device copy of the n elements at h, kept in `allocs`
+template <class T>
+int upload(hsddp_batch* b, const T** d, const T* h, size_t n) {
+    if (int rc = dalloc(b, d, n)) return rc;
+    CK(cudaMemcpy((void*)*d, h, n * sizeof(T), cudaMemcpyHostToDevice));
+    return HSDDP_OK;
+}
 
 // *p := q in `allocs`; the old allocation (if any) is freed, so nothing may still use it on the device
 void replace_alloc(hsddp_batch* b, void** p, void* q) {
@@ -1366,7 +1323,7 @@ struct SlotArray { void** field; size_t bytes; };
 
 std::vector<SlotArray> slot_arrays(hsddp_batch* b) {
     BatchPtrs& bp = b->bp;
-    const size_t rows = (size_t)b->node_stride, D = sizeof(double);
+    const size_t rows = (size_t)b->lib.node_stride, D = sizeof(double);
     return {
         {(void**)&bp.sched, sizeof(DevSchedule)}, {(void**)&b->d_mpc, sizeof(MpcSched)},
         {(void**)&b->d_sched_gait, sizeof(int)}, {(void**)&b->d_sched_window, sizeof(int)},
@@ -1395,6 +1352,13 @@ hsddp_options default_options() {
     o.max_DDP_iter = 10; o.max_AL_iter = 5; o.cost_thresh = 1e-3; o.tconstr_thresh = 1e-3; o.pconstr_thresh = 1e-3;
     o.dynamics_feas_thresh = 1e-3; o.merit_scale = 0.2; o.merit_offset = 1e2; o.AL_active = 1; o.ReB_active = 1; o.MS = 1;
     return o;
+}
+
+hsddp_constraint_params default_constraint_params() {
+    hsddp_constraint_params cp;
+    std::memset(&cp, 0, sizeof cp);
+    cp.grf_delta = 0.1; cp.grf_delta_min = 0.1; cp.grf_eps = 0.1; cp.td_sigma = 50; cp.td_sigma_max = 1e4; cp.td_lambda = 0; cp.mu = 0.7;
+    return cp;
 }
 
 // the iteration budget rules of check_opt
@@ -1508,6 +1472,27 @@ static int alloc_workspace(hsddp_batch* b) {
     return HSDDP_OK;
 }
 
+// first step of both ways to set the problems: schedule_id checked and kept (host and device), bp cleared and given the
+// constraint parameters
+static int begin_problem_set(hsddp_batch* b, int n_schedules, int n_problems, const int32_t* schedule_id, const hsddp_constraint_params* cparams) {
+    for (int i = 0; i < n_problems; ++i)
+        if (schedule_id[i] < 0 || schedule_id[i] >= n_schedules) { g_last_error = "schedule_id out of range"; return HSDDP_ERR_ARG; }
+    b->h_sched_id.assign(schedule_id, schedule_id + n_problems);
+    BatchPtrs& bp = b->bp;
+    std::memset(&bp, 0, sizeof bp);
+    bp.n_problems = n_problems;
+    bp.cp = cparams ? *cparams : default_constraint_params();
+    return upload(b, &bp.sched_id, schedule_id, (size_t)n_problems);
+}
+
+// last step of both: the workspace for these row counts, then the batch reset
+static int finish_problem_set(hsddp_batch* b, int max_stages, int max_nodes) {
+    b->bp.max_stages = max_stages; b->bp.max_nodes = max_nodes;
+    if (int rc = alloc_workspace(b)) return rc;
+    b->has_problems = true;
+    return hsddp_batch_reset(b);
+}
+
 int hsddp_batch_set_problems(hsddp_batch* b, int n_schedules, const hsddp_schedule* schedules, int n_problems,
                              const int32_t* schedule_id, const hsddp_constraint_params* cparams) {
     return guarded([&]() -> int {
@@ -1525,34 +1510,26 @@ int hsddp_batch_set_problems(hsddp_batch* b, int n_schedules, const hsddp_schedu
             return HSDDP_ERR_ARG;
         }
         DevSchedule& d = b->h_sched[i];
-        d.n_phases = s.n_phases; d.n_stages = s.n_stages; d.n_nodes = s.n_nodes; d.dt = s.dt; d.ref_off = (long long)total_nodes;
-        int no = 0, so = 0;
+        d.dt = s.dt; d.ref_off = (long long)total_nodes;
         for (int p = 0; p < s.n_phases; ++p) {
             if (s.horizon[p] < 1) { g_last_error = "phase with empty horizon"; return HSDDP_ERR_ARG; }
-            d.horizon[p] = s.horizon[p]; d.node_off[p] = no; d.stage_off[p] = so;
+            d.horizon[p] = s.horizon[p];
             unsigned cm = 0, nm = 0;
             for (int l = 0; l < 4; ++l) { cm |= (s.contact[p][l] ? 1u : 0u) << l; nm |= (s.next_contact[p][l] ? 1u : 0u) << l; }
             d.cmask[p] = cm; d.nmask[p] = nm;
             d.ss_size[p] = (unsigned char)(s.horizon[p] + 1);
-            d.tdmask[0][p] = (unsigned char)(~cm & nm & 15u); d.tdmask[1][p] = 0;
-            for (int k = 0; k < s.horizon[p] && so + k < HSDDP_MAX_STAGES; ++k) d.ph_of_stage[so + k] = (unsigned char)p;
-            for (int k = 0; k <= s.horizon[p] && no + k < HSDDP_MAX_STAGES + MAXPH; ++k) d.ph_of_node[no + k] = (unsigned char)p;
-            no += s.horizon[p] + 1; so += s.horizon[p];
+            d.tdmask[0][p] = (unsigned char)touchdown_legs(cm, nm); d.tdmask[1][p] = 0;
         }
-        if (no != s.n_nodes || so != s.n_stages) { g_last_error = "schedule node/stage counts inconsistent"; return HSDDP_ERR_ARG; }
+        if (!layout_phases(d, s.n_phases, HSDDP_MAX_STAGES, HSDDP_MAX_STAGES + MAXPH) || d.n_nodes != s.n_nodes || d.n_stages != s.n_stages) {
+            g_last_error = "schedule node/stage counts inconsistent";
+            return HSDDP_ERR_ARG;
+        }
         total_nodes += (size_t)s.n_nodes;
         max_stages = std::max(max_stages, s.n_stages);
         max_nodes = std::max(max_nodes, s.n_nodes);
     }
-    for (int i = 0; i < n_problems; ++i)
-        if (schedule_id[i] < 0 || schedule_id[i] >= n_schedules) { g_last_error = "schedule_id out of range"; return HSDDP_ERR_ARG; }
-    b->h_sched_id.assign(schedule_id, schedule_id + n_problems);
-
-    BatchPtrs& bp = b->bp;
-    std::memset(&bp, 0, sizeof bp);
-    bp.n_problems = n_problems; bp.max_stages = max_stages; bp.max_nodes = max_nodes;
-    if (cparams) bp.cp = *cparams;
-    else { bp.cp.grf_delta = 0.1; bp.cp.grf_delta_min = 0.1; bp.cp.grf_eps = 0.1; bp.cp.td_sigma = 50; bp.cp.td_sigma_max = 1e4; bp.cp.td_lambda = 0; bp.cp.mu = 0.7; }
+    int rc;
+    if ((rc = begin_problem_set(b, n_schedules, n_problems, schedule_id, cparams))) return rc;
 
     std::vector<double> xr(total_nodes * 24), ur(total_nodes * 24), prel(total_nodes * 12), xinit(total_nodes * 24);
     for (int i = 0; i < n_schedules; ++i) {
@@ -1563,28 +1540,24 @@ int hsddp_batch_set_problems(hsddp_batch* b, int n_schedules, const hsddp_schedu
         std::memcpy(&prel[o * 12], s.prel_r, nn * 12 * sizeof(double));
         std::memcpy(&xinit[o * 24], s.xinit, nn * 24 * sizeof(double));
     }
-    DevSchedule* d_sched; int* d_sid; double *d_xr, *d_ur, *d_prel, *d_xinit;
-    int rc;
-    if ((rc = dalloc(b, &d_sched, (size_t)n_schedules))) return rc;
-    if ((rc = dalloc(b, &d_sid, (size_t)n_problems))) return rc;
-    if ((rc = dalloc(b, &d_xr, xr.size()))) return rc;
-    if ((rc = dalloc(b, &d_ur, ur.size()))) return rc;
-    if ((rc = dalloc(b, &d_prel, prel.size()))) return rc;
-    if ((rc = dalloc(b, &d_xinit, xinit.size()))) return rc;
-    CK(cudaMemcpy(d_sched, b->h_sched.data(), sizeof(DevSchedule) * n_schedules, cudaMemcpyHostToDevice));
-    CK(cudaMemcpy(d_sid, schedule_id, sizeof(int) * n_problems, cudaMemcpyHostToDevice));
-    CK(cudaMemcpy(d_xr, xr.data(), xr.size() * sizeof(double), cudaMemcpyHostToDevice));
-    CK(cudaMemcpy(d_ur, ur.data(), ur.size() * sizeof(double), cudaMemcpyHostToDevice));
-    CK(cudaMemcpy(d_prel, prel.data(), prel.size() * sizeof(double), cudaMemcpyHostToDevice));
-    CK(cudaMemcpy(d_xinit, xinit.data(), xinit.size() * sizeof(double), cudaMemcpyHostToDevice));
-    bp.sched = d_sched; bp.sched_id = d_sid; bp.xr = d_xr; bp.ur = d_ur; bp.prel = d_prel; bp.xinit = d_xinit;
-
-    if ((rc = alloc_workspace(b))) return rc;
-    b->has_problems = true;
-    return hsddp_batch_reset(b);
+    BatchPtrs& bp = b->bp;
+    if ((rc = upload(b, &bp.sched, (const DevSchedule*)b->h_sched.data(), (size_t)n_schedules)) || (rc = upload(b, &bp.xr, xr.data(), xr.size())) ||
+        (rc = upload(b, &bp.ur, ur.data(), ur.size())) || (rc = upload(b, &bp.prel, prel.data(), prel.size())) ||
+        (rc = upload(b, &bp.xinit, xinit.data(), xinit.size())))
+        return rc;
+    return finish_problem_set(b, max_stages, max_nodes);
     });
 }
 
+// builds schedule slot slot[i] (nullptr: slot i) from gait[i] and window[i] for i < n: phase table, update state, reference
+// rows.  status[i] != 0: the window does not fit the gait table (1) or the schedule exceeds the table limits (2).
+static void launch_schedule_build(hsddp_batch* b, int n, const int* gait, const int* window, const int* slot, int stage_cap, int* status) {
+    DevSchedule* sched = const_cast<DevSchedule*>(b->bp.sched);
+    k_build_phase_tables<<<(n + 127) / 128, 128, 0, b->stream>>>(b->lib, n, gait, window, slot, stage_cap, sched, b->d_mpc, status);
+    k_reference_rows<<<n, 128, 0, b->stream>>>(b->lib, n, gait, window, slot, sched, b->d_mpc, const_cast<double*>(b->bp.xr),
+                                               const_cast<double*>(b->bp.ur), const_cast<double*>(b->bp.prel), const_cast<double*>(b->bp.xinit));
+    b->n_step_launches += 2;
+}
 
 int hsddp_batch_set_problems_from_gaits(hsddp_batch* b, int n_gaits, const int32_t* gait_rows, const float* gait_dt,
                                         const double* body_state, const double* qJ, const double* foot_placements, const double* grf,
@@ -1596,74 +1569,45 @@ int hsddp_batch_set_problems_from_gaits(hsddp_batch* b, int n_gaits, const int32
         return HSDDP_ERR_ARG;
     CK(cudaSetDevice(b->device));
     free_problem_allocs(b);
+    for (int i = 0; i < n_schedules; ++i)
+        if (sched_gait[i] < 0 || sched_gait[i] >= n_gaits) { g_last_error = "sched_gait out of range"; return HSDDP_ERR_ARG; }
+    int rc;
+    if ((rc = begin_problem_set(b, n_schedules, n_problems, schedule_id, cparams))) return rc;
+    // gait library -> HBM
     std::vector<int> row_off(n_gaits);
     size_t rows = 0;
     for (int g = 0; g < n_gaits; ++g) { row_off[g] = (int)rows; rows += (size_t)gait_rows[g]; }
-    for (int i = 0; i < n_schedules; ++i)
-        if (sched_gait[i] < 0 || sched_gait[i] >= n_gaits) { g_last_error = "sched_gait out of range"; return HSDDP_ERR_ARG; }
-    for (int i = 0; i < n_problems; ++i)
-        if (schedule_id[i] < 0 || schedule_id[i] >= n_schedules) { g_last_error = "schedule_id out of range"; return HSDDP_ERR_ARG; }
-    // gait library -> HBM
-    double *d_bs, *d_qj, *d_ft, *d_grf; int *d_ct, *d_ro, *d_nr, *d_status; float* d_dt;
-    int rc;
-    if ((rc = dalloc(b, &d_bs, rows * 12)) || (rc = dalloc(b, &d_qj, rows * 12)) || (rc = dalloc(b, &d_ft, rows * 12)) || (rc = dalloc(b, &d_grf, rows * 12)) ||
-        (rc = dalloc(b, &d_ct, rows * 4)) || (rc = dalloc(b, &d_ro, (size_t)n_gaits)) || (rc = dalloc(b, &d_nr, (size_t)n_gaits)) || (rc = dalloc(b, &d_dt, (size_t)n_gaits)) ||
-        (rc = dalloc(b, &d_status, (size_t)n_schedules)))
+    GaitLib& lib = b->lib;
+    if ((rc = upload(b, &lib.body_state, body_state, rows * 12)) || (rc = upload(b, &lib.qJ, qJ, rows * 12)) ||
+        (rc = upload(b, &lib.foot, foot_placements, rows * 12)) || (rc = upload(b, &lib.grf, grf, rows * 12)) ||
+        (rc = upload(b, &lib.contact, contact, rows * 4)) || (rc = upload(b, &lib.row_off, row_off.data(), (size_t)n_gaits)) ||
+        (rc = upload(b, &lib.n_rows, gait_rows, (size_t)n_gaits)) || (rc = upload(b, &lib.dt, gait_dt, (size_t)n_gaits)))
         return rc;
-    CK(cudaMemcpy(d_bs, body_state, rows * 12 * sizeof(double), cudaMemcpyHostToDevice));
-    CK(cudaMemcpy(d_qj, qJ, rows * 12 * sizeof(double), cudaMemcpyHostToDevice));
-    CK(cudaMemcpy(d_ft, foot_placements, rows * 12 * sizeof(double), cudaMemcpyHostToDevice));
-    CK(cudaMemcpy(d_grf, grf, rows * 12 * sizeof(double), cudaMemcpyHostToDevice));
-    CK(cudaMemcpy(d_ct, contact, rows * 4 * sizeof(int), cudaMemcpyHostToDevice));
-    CK(cudaMemcpy(d_ro, row_off.data(), n_gaits * sizeof(int), cudaMemcpyHostToDevice));
-    CK(cudaMemcpy(d_nr, gait_rows, n_gaits * sizeof(int), cudaMemcpyHostToDevice));
-    CK(cudaMemcpy(d_dt, gait_dt, n_gaits * sizeof(float), cudaMemcpyHostToDevice));
-    GaitLib lib{d_bs, d_qj, d_ft, d_grf, d_ct, d_ro, d_nr, d_dt};
-
-    BatchPtrs& bp = b->bp;
-    std::memset(&bp, 0, sizeof bp);
-    if (cparams) bp.cp = *cparams;
-    else { bp.cp.grf_delta = 0.1; bp.cp.grf_delta_min = 0.1; bp.cp.grf_eps = 0.1; bp.cp.td_sigma = 50; bp.cp.td_sigma_max = 1e4; bp.cp.td_lambda = 0; bp.cp.mu = 0.7; }
-    const int node_stride = std::min(HSDDP_MAX_STAGES, (int)std::lround(plan_duration / 0.01f) + 1) + MAXPH;
-    b->node_stride = node_stride;
+    lib.plan = plan_duration;
+    lib.node_stride = std::min(HSDDP_MAX_STAGES, (int)std::lround(plan_duration / kTickDt) + 1) + MAXPH;
     for (const SlotArray& a : slot_arrays(b))  // one schedule slot per schedule
         if ((rc = dalloc_bytes(b, a.field, (size_t)n_schedules * a.bytes))) return rc;
-    int *d_sid, *d_err;
-    if ((rc = dalloc(b, &d_sid, (size_t)n_problems)) || (rc = dalloc(b, &d_err, (size_t)4))) return rc;
+    int *d_status, *d_err;
+    if ((rc = dalloc(b, &d_status, (size_t)n_schedules)) || (rc = dalloc(b, &d_err, (size_t)4))) return rc;
     CK(cudaMemcpy(b->d_sched_gait, sched_gait, n_schedules * sizeof(int), cudaMemcpyHostToDevice));
     CK(cudaMemcpy(b->d_sched_window, sched_window, n_schedules * sizeof(int), cudaMemcpyHostToDevice));
-    CK(cudaMemcpy(d_sid, schedule_id, sizeof(int) * n_problems, cudaMemcpyHostToDevice));
     CK(cudaMemsetAsync(d_err, 0, 4 * sizeof(int), b->stream));
-    DevSchedule* d_sched = const_cast<DevSchedule*>(bp.sched);
-    k_build_phase_tables<<<(n_schedules + 127) / 128, 128, 0, b->stream>>>(lib, n_schedules, b->d_sched_gait, b->d_sched_window, plan_duration, node_stride, d_sched,
-                                                                           d_status, b->d_mpc, nullptr, HSDDP_MAX_STAGES);
-    k_build_reference_rows<<<n_schedules, 128, 0, b->stream>>>(lib, n_schedules, b->d_sched_gait, b->d_sched_window, plan_duration, node_stride, d_sched, d_status,
-                                                               const_cast<double*>(bp.xr), const_cast<double*>(bp.ur), const_cast<double*>(bp.prel),
-                                                               const_cast<double*>(bp.xinit), nullptr);
+    launch_schedule_build(b, n_schedules, b->d_sched_gait, b->d_sched_window, nullptr, HSDDP_MAX_STAGES, d_status);
     CK(cudaGetLastError());
-    b->n_step_launches += 2;
     // the host keeps the phase tables too (dense gain / Jacobian getters, workspace sizing)
     b->h_sched.assign(n_schedules, DevSchedule{});
     std::vector<int> status(n_schedules);
-    CK(cudaMemcpyAsync(b->h_sched.data(), d_sched, sizeof(DevSchedule) * n_schedules, cudaMemcpyDeviceToHost, b->stream));
+    CK(cudaMemcpyAsync(b->h_sched.data(), b->bp.sched, sizeof(DevSchedule) * n_schedules, cudaMemcpyDeviceToHost, b->stream));
     CK(cudaMemcpyAsync(status.data(), d_status, sizeof(int) * n_schedules, cudaMemcpyDeviceToHost, b->stream));
     CK(cudaStreamSynchronize(b->stream));
-    int max_stages = 0, max_nodes = 0;
+    int max_stages = 0;
     for (int i = 0; i < n_schedules; ++i) {
         if (status[i]) { g_last_error = status[i] == 1 ? "window does not fit the gait table" : "schedule exceeds HSDDP_MAX_PHASES / HSDDP_MAX_STAGES"; free_problem_allocs(b); return status[i] == 1 ? HSDDP_ERR_ARG : HSDDP_ERR_UNSUPPORTED; }
         max_stages = std::max(max_stages, b->h_sched[i].n_stages);
-        max_nodes = std::max(max_nodes, b->h_sched[i].n_nodes);
     }
-    b->h_sched_id.assign(schedule_id, schedule_id + n_problems);
+    b->d_mpc_err = d_err; b->n_sched = n_schedules; b->n_gaits = n_gaits; b->mpc_ready = true;
     // (node rows with headroom: a receding-horizon update can add phases, i.e. nodes, while the stage count stays the same)
-    max_nodes = std::min(node_stride, max_stages + MAXPH);
-    bp.n_problems = n_problems; bp.max_stages = max_stages; bp.max_nodes = max_nodes;
-    bp.sched_id = d_sid;
-    if ((rc = alloc_workspace(b))) return rc;
-    b->has_problems = true;
-    b->lib = lib; b->d_mpc_err = d_err;
-    b->plan = plan_duration; b->n_sched = n_schedules; b->n_gaits = n_gaits; b->mpc_ready = true;
-    return hsddp_batch_reset(b);
+    return finish_problem_set(b, max_stages, std::min(lib.node_stride, max_stages + MAXPH));
     });
 }
 
@@ -1675,10 +1619,10 @@ int hsddp_batch_mpc_update(hsddp_batch* b) {
     CK(cudaSetDevice(b->device));
     CK(cudaEventRecord(b->ev_u0, b->stream));
     DevSchedule* d_sched = const_cast<DevSchedule*>(b->bp.sched);
-    k_mpc_update_schedules<<<(b->n_sched + 127) / 128, 128, 0, b->stream>>>(b->lib, b->n_sched, b->d_sched_gait, b->d_sched_window, b->plan, b->node_stride,
-                                                                              d_sched, b->d_mpc, b->d_mpc_err);
-    k_mpc_reference_rows<<<b->n_sched, 128, 0, b->stream>>>(b->lib, b->n_sched, b->d_sched_gait, b->d_sched_window, b->plan, d_sched, b->d_mpc,
-                                                            const_cast<double*>(b->bp.xr), const_cast<double*>(b->bp.ur), const_cast<double*>(b->bp.prel));
+    k_mpc_update_schedules<<<(b->n_sched + 127) / 128, 128, 0, b->stream>>>(b->lib, b->n_sched, b->d_sched_gait, b->d_sched_window, d_sched, b->d_mpc,
+                                                                              b->d_mpc_err);
+    k_reference_rows<<<b->n_sched, 128, 0, b->stream>>>(b->lib, b->n_sched, b->d_sched_gait, b->d_sched_window, nullptr, d_sched, b->d_mpc,
+                                                        const_cast<double*>(b->bp.xr), const_cast<double*>(b->bp.ur), const_cast<double*>(b->bp.prel), nullptr);
     k_mpc_shift<<<b->bp.n_problems, kThreads, 0, b->stream>>>(b->bp, b->d_mpc);
     CK(cudaGetLastError());
     b->n_step_launches += 3;
@@ -1837,13 +1781,8 @@ int hsddp_batch_restart_problems(hsddp_batch* b, int n, const int32_t* problem, 
     // build into the free slots, then one host synchronise for the build status
     const int *d_bg = d + 2 * n, *d_bw = d_bg + m, *d_bs = d_bw + m;
     int* d_st = const_cast<int*>(d_bs + m);
-    DevSchedule* d_sched = const_cast<DevSchedule*>(b->bp.sched);
-    k_build_phase_tables<<<(m + 127) / 128, 128, 0, b->stream>>>(b->lib, m, d_bg, d_bw, b->plan, b->node_stride, d_sched, d_st, b->d_mpc, d_bs,
-                                                                 b->bp.max_stages);
-    k_build_reference_rows<<<m, 128, 0, b->stream>>>(b->lib, m, d_bg, d_bw, b->plan, b->node_stride, d_sched, d_st, const_cast<double*>(b->bp.xr),
-                                                     const_cast<double*>(b->bp.ur), const_cast<double*>(b->bp.prel), const_cast<double*>(b->bp.xinit), d_bs);
+    launch_schedule_build(b, m, d_bg, d_bw, d_bs, b->bp.max_stages, d_st);
     CK(cudaGetLastError());
-    b->n_step_launches += 2;
     CK(cudaMemcpyAsync(a_st, d_st, sizeof(int) * m, cudaMemcpyDeviceToHost, b->stream));
     CK(cudaStreamSynchronize(b->stream));
     for (int j = 0; j < m; ++j) {
