@@ -145,6 +145,11 @@ def lib():
         L.hsddp_batch_last_update_ms.argtypes = [vp, C.POINTER(C.c_float)]
         L.hsddp_batch_restart_problems.argtypes = [vp, C.c_int, ip, ip, ip, dp, C.POINTER(Options)]
         L.hsddp_batch_get_schedule_ids.argtypes = [vp, ip]
+        L.hsddp_batch_mpc_update_problems.argtypes = [vp, C.c_int, ip]
+        L.hsddp_batch_set_initial_condition_problems.argtypes = [vp, C.c_int, ip, dp]
+        L.hsddp_batch_solve_problems.argtypes = [vp, C.c_int, ip, C.POINTER(Options)]
+        L.hsddp_batch_solve_problems_async.argtypes = [vp, C.c_int, ip, C.POINTER(Options)]
+        L.hsddp_batch_get_mpc_command_problems.argtypes = [vp, C.c_int, C.c_int, ip, vp]
         for f in ("hsddp_batch_solve", "hsddp_batch_solve_async", "hsddp_batch_compute_cost", "hsddp_batch_lq_approximation",
                   "hsddp_batch_prepare_merit", "hsddp_batch_update_al_params", "hsddp_batch_update_reb_params"):
             getattr(L, f).argtypes = [vp, C.POINTER(Options)]
@@ -198,6 +203,11 @@ def _ip(a):
 
 def _fp(a):
     return a.ctypes.data_as(C.POINTER(C.c_float))
+
+
+def _plist(problems):
+    """A problem-index list as the C ABI takes it (int32, contiguous)."""
+    return np.ascontiguousarray(np.asarray(problems, np.int32).ravel())
 
 
 def _check(rc, what):
@@ -358,15 +368,26 @@ class MultiPhaseDDPBatch:
         nn = int(hz[:P].sum()) + P
         return dict(n_phases=P, horizon=hz[:P].tolist(), contact=c[:P].tolist(), next_contact=cn[:P].tolist(), xr=xr[:nn], ur=ur[:nn], prel_r=pr[:nn], xinit=xi[:nn])
 
-    def set_initial_condition(self, x0):
+    def set_initial_condition(self, x0, problems=None):
+        """x0: [n_problems][24], or with `problems` (indices) one row per listed problem, which alone get a new state."""
+        if problems is not None:
+            p = _plist(problems)
+            x0 = np.ascontiguousarray(x0, np.float64).reshape(len(p), 24)
+            _check(lib().hsddp_batch_set_initial_condition_problems(self.h, len(p), _ip(p), _dp(x0)), "hsddp_batch_set_initial_condition_problems")
+            return
         x0 = np.ascontiguousarray(x0, np.float64).reshape(self.n, 24)
         _check(lib().hsddp_batch_set_initial_condition(self.h, _dp(x0)), "hsddp_batch_set_initial_condition")
 
     def reset(self):
         _check(lib().hsddp_batch_reset(self.h), "hsddp_batch_reset")
 
-    def mpc_update(self):
-        """HKDProblem::update for every problem (receding-horizon shift by one MPC step, on the device)."""
+    def mpc_update(self, problems=None):
+        """HKDProblem::update for every problem (receding-horizon shift by one MPC step, on the device), or only for the listed
+        `problems` (indices): the others keep everything, bit for bit."""
+        if problems is not None:
+            p = _plist(problems)
+            _check(lib().hsddp_batch_mpc_update_problems(self.h, len(p), _ip(p)), "hsddp_batch_mpc_update_problems")
+            return
         _check(lib().hsddp_batch_mpc_update(self.h), "hsddp_batch_mpc_update")
 
     def restart(self, problems, gait, window, x0, first_solve=None):
@@ -393,12 +414,21 @@ class MultiPhaseDDPBatch:
         _check(lib().hsddp_batch_last_update_ms(self.h, C.byref(ms)), "hsddp_batch_last_update_ms")
         return ms.value
 
-    def solve(self, opt=None):
+    def solve(self, opt=None, problems=None):
+        """Solve every problem, or only the listed `problems` (indices), in the kernel a batch of that many would run."""
         opt = opt or Options()
+        if problems is not None:
+            p = _plist(problems)
+            _check(lib().hsddp_batch_solve_problems(self.h, len(p), _ip(p), C.byref(opt)), "hsddp_batch_solve_problems")
+            return
         _check(lib().hsddp_batch_solve(self.h, C.byref(opt)), "hsddp_batch_solve")
 
-    def solve_async(self, opt=None):
+    def solve_async(self, opt=None, problems=None):
         opt = opt or Options()
+        if problems is not None:
+            p = _plist(problems)
+            _check(lib().hsddp_batch_solve_problems_async(self.h, len(p), _ip(p), C.byref(opt)), "hsddp_batch_solve_problems_async")
+            return
         _check(lib().hsddp_batch_solve_async(self.h, C.byref(opt)), "hsddp_batch_solve_async")
 
     def set_solve_mode(self, mode):
@@ -497,8 +527,16 @@ class MultiPhaseDDPBatch:
         _check(lib().hsddp_batch_get_gains_compact(self.h, int(row0), int(nrows), _dp(out)), "get_gains_compact")
         return out
 
-    def mpc_command(self, n_steps=8, out=None):
-        """hkd_command_lcmt payload of every problem (HKDMPC.cpp:207-298), packed on the device."""
+    def mpc_command(self, n_steps=8, out=None, problems=None):
+        """hkd_command_lcmt payload of every problem (HKDMPC.cpp:207-298), packed on the device; with `problems` (indices) one
+        record per listed problem, in list order."""
+        if problems is not None:
+            p = _plist(problems)
+            if out is None:
+                out = np.zeros(len(p), dtype=CMD_DTYPE)
+            _check(lib().hsddp_batch_get_mpc_command_problems(self.h, int(n_steps), len(p), _ip(p), out.ctypes.data_as(C.c_void_p)),
+                   "get_mpc_command_problems")
+            return out
         if out is None:
             out = np.zeros(self.n, dtype=CMD_DTYPE)
         _check(lib().hsddp_batch_get_mpc_command(self.h, int(n_steps), out.ctypes.data_as(C.c_void_p)), "get_mpc_command")

@@ -80,6 +80,10 @@ __device__ inline bool line_search_block(Smem& sm, double& eps_out, int& n_trial
 // ---------------------------------------------------------------------------
 struct TrialPtrs { double *X, *U, *U_t, *Xsim_t, *Defect, *gcon, *hcon; };
 
+// The trial arrays, results and mailbox of a cluster belong to its position in the launch, not to its problem: a solve of listed
+// problems (hsddp_batch_solve_problems) in a batch of more than kClusterLsMax problems has them for kClusterLsMax positions only.
+__device__ __forceinline__ int ls_pos() { return (int)blockIdx.x >> 2; }
+
 __device__ inline TrialPtrs swap_trial_arrays(Smem& sm, const TrialPtrs& t) {
     TrialPtrs old = {sm.X, sm.U, sm.U_t, sm.Xsim_t, sm.Defect, sm.gcon, sm.hcon};
     __syncthreads();
@@ -87,14 +91,14 @@ __device__ inline TrialPtrs swap_trial_arrays(Smem& sm, const TrialPtrs& t) {
     __syncthreads();
     return old;
 }
-__device__ inline TrialPtrs trial_arrays(const BatchPtrs& bp, int pid, int r) {
-    const size_t q = (size_t)pid * 4 + r, sn = (size_t)bp.max_nodes * 24, ss = (size_t)bp.max_stages * 24;
+__device__ inline TrialPtrs trial_arrays(const BatchPtrs& bp, int pos, int r) {
+    const size_t q = (size_t)pos * 4 + r, sn = (size_t)bp.max_nodes * 24, ss = (size_t)bp.max_stages * 24;
     return TrialPtrs{bp.ls_X + q * sn, bp.ls_U + q * ss, bp.ls_Ut + q * ss, bp.ls_Xsim + q * sn, bp.ls_Defect + q * sn,
                      bp.ls_gcon + q * bp.max_stages * 20, bp.ls_hcon + q * MAXPH * 4};
 }
 // one trial into the trial arrays of step r; the block's own arrays are untouched
 __device__ inline void run_trial(Smem& sm, const BatchPtrs& bp, int r, double eps) {
-    const TrialPtrs keep = swap_trial_arrays(sm, trial_arrays(bp, sm.pid, r));
+    const TrialPtrs keep = swap_trial_arrays(sm, trial_arrays(bp, ls_pos(), r));
     // (touchdown values of legs without a constraint are never written by a rollout: start from the current ones)
     for (int e = threadIdx.x; e < MAXPH * 4; e += kThreads) sm.hcon[e] = keep.hcon[e];
     for (int e = threadIdx.x; e < sm.sc.n_stages * 20; e += kThreads) sm.gcon[e] = keep.gcon[e];  // (likewise the rows of swing legs)
@@ -102,20 +106,20 @@ __device__ inline void run_trial(Smem& sm, const BatchPtrs& bp, int r, double ep
     const bool ok = hybrid_rollout_block<true>(sm, eps);
     compute_cost_block(sm);
     if (threadIdx.x == 0) {
-        double* res = bp.ls_res + ((size_t)sm.pid * 4 + r) * 8;
+        double* res = bp.ls_res + ((size_t)ls_pos() * 4 + r) * 8;
         res[0] = sm.st.actual_cost; res[1] = sm.st.feas; res[2] = sm.st.max_pconstr; res[3] = sm.st.max_tconstr; res[4] = ok ? 1.0 : 0.0;
     }
     swap_trial_arrays(sm, keep);
 }
 __device__ inline void commit_trial(Smem& sm, const BatchPtrs& bp, int r) {
-    const TrialPtrs t = trial_arrays(bp, sm.pid, r);
+    const TrialPtrs t = trial_arrays(bp, ls_pos(), r);
     const DevSchedule& sc = sm.sc;
     for (int e = threadIdx.x; e < sc.n_nodes * 24; e += kThreads) { sm.X[e] = t.X[e]; sm.Defect[e] = t.Defect[e]; }
     for (int e = threadIdx.x; e < sc.n_stages * 24; e += kThreads) sm.U[e] = t.U[e];
     for (int e = threadIdx.x; e < sc.n_stages * 20; e += kThreads) sm.gcon[e] = t.gcon[e];
     for (int e = threadIdx.x; e < MAXPH * 4; e += kThreads) sm.hcon[e] = t.hcon[e];
     if (threadIdx.x == 0) {
-        const double* res = bp.ls_res + ((size_t)sm.pid * 4 + r) * 8;
+        const double* res = bp.ls_res + ((size_t)ls_pos() * 4 + r) * 8;
         sm.st.actual_cost = res[0]; sm.st.feas = res[1]; sm.st.max_pconstr = res[2]; sm.st.max_tconstr = res[3]; sm.st.rollout_ok = 1;
         sm.ctl.trial_cost = res[0]; sm.ctl.trial_feas = res[1]; sm.ctl.have_trial = 1;
     }
@@ -131,7 +135,7 @@ __device__ inline bool line_search_cluster(Smem& sm, const BatchPtrs& bp, double
     int nv = 0;
     for (double e = 1; e > 1e-3 && nv < 4; e *= sm.opt.alpha) epsv[nv++] = e;  // 1, .1, .010000000000000002, .0010000000000000002 (Q6)
     __syncthreads();
-    if (threadIdx.x == 0) { bp.ls_mail[sm.pid] = 1; __threadfence(); }
+    if (threadIdx.x == 0) { bp.ls_mail[ls_pos()] = 1; __threadfence(); }
     cg::this_cluster().sync();  // [A] the helpers start their trials
     if (nv > 0) run_trial(sm, bp, 0, epsv[0]);
     __threadfence();
@@ -139,7 +143,7 @@ __device__ inline bool line_search_cluster(Smem& sm, const BatchPtrs& bp, double
     bool diverged = false;
     int accepted = -1;
     for (int r = 0; r < nv; ++r) {
-        const double* res = bp.ls_res + ((size_t)sm.pid * 4 + r) * 8;
+        const double* res = bp.ls_res + ((size_t)ls_pos() * 4 + r) * 8;
         const double cost = __ldcg(res), feas = __ldcg(res + 1);
         const bool ok = __ldcg(res + 4) != 0.0;
         if (!ok) { diverged = true; break; }
@@ -181,7 +185,7 @@ __device__ inline void line_search_helper_loop(Smem& sm, const BatchPtrs& bp, in
     namespace cg = cooperative_groups;
     for (;;) {
         cg::this_cluster().sync();  // [A]
-        const int op = *((volatile int*)(bp.ls_mail + sm.pid));
+        const int op = *((volatile int*)(bp.ls_mail + ls_pos()));
         if (op != 1) break;
         double eps = 1;
         for (int q = 0; q < r; ++q) eps *= sm.opt.alpha;
@@ -514,18 +518,18 @@ __global__ void __launch_bounds__(kThreads, 2) k_solve_lat(BatchPtrs bp, hsddp_o
 }
 
 // latency build with the concurrent line search: one cluster of four blocks per problem (block rank 0 solves, ranks 1..3 evaluate
-// the other step sizes of every line search)
+// the other step sizes of every line search).  Cluster q solves problem bp.order[q] (nullptr: problem q).
 __global__ void __cluster_dims__(4, 1, 1) __launch_bounds__(kThreads, 2) k_solve_lat4(BatchPtrs bp, hsddp_options opt) {
     namespace cg = cooperative_groups;
     __shared__ Smem sm;
-    const int pid = blockIdx.x >> 2, r = (int)cg::this_cluster().block_rank();
+    const int pid = bp.order ? bp.order[ls_pos()] : ls_pos(), r = (int)cg::this_cluster().block_rank();
     if (threadIdx.x == 0) assign_rotation(bp.sm_slots, sm.rot);
     bind_problem(sm, bp, pid);
     if (threadIdx.x == 0) sm.opt = opt;
     __syncthreads();
     if (r == 0) {
         solve_block<true>(sm, bp);
-        if (threadIdx.x == 0) { bp.state[pid] = sm.st; bp.ctl[pid] = sm.ctl; bp.ls_mail[pid] = 2; __threadfence(); }
+        if (threadIdx.x == 0) { bp.state[pid] = sm.st; bp.ctl[pid] = sm.ctl; bp.ls_mail[ls_pos()] = 2; __threadfence(); }
         cg::this_cluster().sync();  // [A] of the helpers' last round: exit
     } else {
         line_search_helper_loop(sm, bp, r);
@@ -668,11 +672,12 @@ __global__ void __launch_bounds__(kThreads, HSDDP_MIN_BLOCKS) k_step(BatchPtrs b
 }
 
 // HKDMPCSolver::publish_mpc_cmd + update_foot_placement (HKDMPC/HKDMPC.cpp:207-298): one block per problem packs the
-// command record.  Stage k of the command = stage s of phase i, walked with the reference's (k, s, i) loop.
-__global__ void k_command(BatchPtrs bp, int n_steps, hsddp_mpc_command* out) {
-    const int pid = blockIdx.x;
+// command record.  Stage k of the command = stage s of phase i, walked with the reference's (k, s, i) loop.  Block j packs
+// problem list[j] (nullptr: problem j) into out[j].
+__global__ void k_command(BatchPtrs bp, int n_steps, hsddp_mpc_command* out, const int* list) {
+    const int pid = list ? list[blockIdx.x] : (int)blockIdx.x;
     const DevSchedule& sc = bp.sched[bp.sched_id[pid]];
-    hsddp_mpc_command& cmd = out[pid];
+    hsddp_mpc_command& cmd = out[blockIdx.x];
     __shared__ int s_stage[HSDDP_CMD_MAX_STEPS], s_node[HSDDP_CMD_MAX_STEPS], s_phase[HSDDP_CMD_MAX_STEPS];
     if (threadIdx.x == 0) {
         int s = 0, i = 0;
@@ -878,21 +883,21 @@ __global__ void k_reference_rows(GaitLib lib, int n, const int* gait, const int*
 // N1: receding-horizon update on the device (HKDProblem::update, HKDMPC/HKD-TrajOpt/HKDProblem.cpp:117-222, as
 // HKDMPCSolver::update drives it every MPC step, HKDMPC.cpp:97-166).  All problems of a batch tick together, so a
 // schedule (gait, initial window) stays shared by the problems that use it:
-//   k_mpc_update_schedules  one thread per schedule: QuadReference::step (QuadReference.cpp:33-47), front end (drop the first
+//   k_mpc_update_schedules  one thread per schedule (entry i: slot slot[i], nullptr: slot i): QuadReference::step (QuadReference.cpp:33-47), front end (drop the first
 //                           node or the whole first phase), back end (grow the last phase or open a new one; add_tconstr_one_phase
 //                           when the last phase has reached its end), shooting sets -- with the reference's float time arithmetic
 //   k_reference_rows        the per-node reference rows of the shifted window (HKDReference.cpp:8-57)
 //   k_mpc_shift             one block per problem: Trajectory::pop_front / push_back_state (TrajectoryManagement.cpp:118-207),
 //                           PathConstraintBase::pop_front / push_back (ConstraintsBase.h:271-280) on the problem-major arrays
 // ---------------------------------------------------------------------------
-__global__ void k_mpc_update_schedules(GaitLib lib, int n_sched, const int* sched_gait, const int* sched_window,
+__global__ void k_mpc_update_schedules(GaitLib lib, int n_sched, const int* sched_gait, const int* sched_window, const int* slot,
                                        DevSchedule* scheds, MpcSched* mpc, int* err) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n_sched) return;
-    const int gi = sched_gait[i];
+    const int gi = sched_gait[i], si = slot ? slot[i] : i;
     if (gi < 0) return;  // a free slot (hsddp_batch_restart_problems)
-    DevSchedule d = scheds[i];
-    MpcSched m = mpc[i];
+    DevSchedule d = scheds[si];
+    MpcSched m = mpc[si];
     const float dtg = lib.dt[gi];
     const int sz = ref_window_size(lib, dtg);
     m.old_n_nodes = d.n_nodes;
@@ -901,7 +906,7 @@ __global__ void k_mpc_update_schedules(GaitLib lib, int n_sched, const int* sche
     for (int q = 1; approx_leq_f(__fmul_rn((float)q, dtg), kTickDt); ++q) { m.k_cur++; m.t_cur = __fadd_rn(m.t_cur, dtg); }
     const float new_start = m.t_cur, new_end = __fadd_rn(m.t_cur, lib.plan);
     const size_t row0 = (size_t)(lib.row_off[gi] + sched_window[i] + m.k_cur);
-    if (sched_window[i] + m.k_cur + sz >= lib.n_rows[gi]) { m.status = 1; mpc[i] = m; atomicMax(err, 1); return; }
+    if (sched_window[i] + m.k_cur + sz >= lib.n_rows[gi]) { m.status = 1; mpc[si] = m; atomicMax(err, 1); return; }
     int n = d.n_phases;
     // ---- front end ----
     m.start[0] = __fadd_rn(m.start[0], kTickDt);
@@ -922,7 +927,7 @@ __global__ void k_mpc_update_schedules(GaitLib lib, int n_sched, const int* sche
     const unsigned newc = contact_mask_at(lib, row0 + ref_index_at(__fsub_rn(new_end, new_start), dtg, sz));
     const bool change = newc != d.cmask[n - 1];
     if (change && m.reach_end[n - 1]) {
-        if (n >= MAXPH) { m.status = 2; mpc[i] = m; atomicMax(err, 2); return; }
+        if (n >= MAXPH) { m.status = 2; mpc[si] = m; atomicMax(err, 2); return; }
         m.start[n] = m.end[n - 1]; m.end[n] = new_end; m.reach_end[n] = 0; m.has_tconstr[n] = 0;
         d.horizon[n] = (int)roundf(__fdiv_rn(__fsub_rn(m.end[n], m.start[n]), kTickDt));
         d.cmask[n] = newc; d.nmask[n] = 0; d.tdmask[0][n] = 0; d.tdmask[1][n] = 0; d.ss_size[n] = 0;  // (SinglePhase::initialization clears SS_set)
@@ -940,7 +945,7 @@ __global__ void k_mpc_update_schedules(GaitLib lib, int n_sched, const int* sche
         const unsigned td = touchdown_legs(d.cmask[n - 1], nm);
         if (td) {
             const int ob = d.tdmask[0][n - 1] ? (d.tdmask[1][n - 1] ? 2 : 1) : 0;
-            if (ob >= 2) { m.status = 2; mpc[i] = m; atomicMax(err, 2); return; }  // (needs a one-sample contact blip in the reference)
+            if (ob >= 2) { m.status = 2; mpc[si] = m; atomicMax(err, 2); return; }  // (needs a one-sample contact blip in the reference)
             d.tdmask[ob][n - 1] = (unsigned char)td;
             m.new_td_phase = n - 1; m.new_td_object = ob;
         }
@@ -948,9 +953,9 @@ __global__ void k_mpc_update_schedules(GaitLib lib, int n_sched, const int* sche
     // ---- shooting configuration (HKDProblem.cpp:205-221) and the derived tables ----
     for (int p = 0; p < n; ++p)
         if ((p == n - 1 && d.horizon[p] > 2) || p < n - 1) d.ss_size[p] = (unsigned char)(d.horizon[p] + 1);
-    if (!layout_phases(d, n, HSDDP_MAX_STAGES, lib.node_stride)) { m.status = 2; mpc[i] = m; atomicMax(err, 2); return; }
-    scheds[i] = d;
-    mpc[i] = m;
+    if (!layout_phases(d, n, HSDDP_MAX_STAGES, lib.node_stride)) { m.status = 2; mpc[si] = m; atomicMax(err, 2); return; }
+    scheds[si] = d;
+    mpc[si] = m;
 }
 
 // rows [shift, total) of a row-major array move down to [0, total - shift); the last `shift` rows are then filled by the caller.
@@ -969,8 +974,9 @@ __device__ inline void shift_rows_down(double* a, int total_rows, int row_len, i
     }
 }
 
-__global__ void __launch_bounds__(kThreads) k_mpc_shift(BatchPtrs bp, const MpcSched* mpc) {
-    const int pid = blockIdx.x, tid = threadIdx.x;
+// block j shifts problem list[j] (nullptr: problem j)
+__global__ void __launch_bounds__(kThreads) k_mpc_shift(BatchPtrs bp, const MpcSched* mpc, const int* list) {
+    const int pid = list ? list[blockIdx.x] : (int)blockIdx.x, tid = threadIdx.x;
     const int sid = bp.sched_id[pid];
     const MpcSched& m = mpc[sid];
     if (m.status) return;
@@ -1075,6 +1081,43 @@ __global__ void __launch_bounds__(kThreads) k_restart(BatchPtrs bp, RestartArgs 
     if (threadIdx.x == 0) bp.state[pid] = sm.st;
 }
 
+// ---------------------------------------------------------------------------
+// Receding-horizon update of listed problems (hsddp_batch_mpc_update_problems).  Problems share a schedule slot, so a slot that
+// listed problems use is first copied, one block per slot: slot src[j] goes to the free slot dst[j] in every slot array, the copy
+// gets its own reference rows (ref_off = dst[j] x node_stride), and gait / window of entry j are listed for the update kernels,
+// which then step the copies only.
+// ---------------------------------------------------------------------------
+constexpr int kSlotArraysMax = 8;
+struct SlotCopyArgs {
+    const int *src, *dst;                    // [n]
+    const int *sched_gait, *sched_window;    // per slot
+    int *gait, *window;                      // [n] out
+    DevSchedule* sched;
+    int node_stride, n_arrays;
+    struct { unsigned* base; size_t words; } arr[kSlotArraysMax];  // slot arrays: base, 4-byte words per slot
+};
+
+__global__ void k_copy_slots(SlotCopyArgs a) {
+    const int j = blockIdx.x;
+    const size_t s = (size_t)a.src[j], t = (size_t)a.dst[j];
+    for (int k = 0; k < a.n_arrays; ++k)
+        for (size_t e = threadIdx.x; e < a.arr[k].words; e += blockDim.x) a.arr[k].base[t * a.arr[k].words + e] = a.arr[k].base[s * a.arr[k].words + e];
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        a.sched[t].ref_off = (long long)t * a.node_stride;
+        a.gait[j] = a.sched_gait[s]; a.window[j] = a.sched_window[s];
+    }
+}
+
+// row idx[j] of dst := row j of src (src_stride 0: the same row for every j), rows of `words` 4-byte words.  Writes the per-problem
+// rows of the list-driven entry points: initial states, schedule slots, cleared budgets, free-slot marks.
+__global__ void k_scatter_rows(unsigned* dst, int words, const int* idx, const unsigned* src, int src_stride, int n) {
+    const long long e = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (e >= (long long)n * words) return;
+    const int j = (int)(e / words), w = (int)(e % words);
+    dst[(size_t)idx[j] * words + w] = src[(size_t)j * src_stride + w];
+}
+
 // FP64 throughput probes (roofline denominators measured on the box)
 __global__ void k_dfma_probe(double* out, int iters) {
     double a0 = threadIdx.x * 1e-3, a1 = a0 + 1, a2 = a0 + 2, a3 = a0 + 3, a4 = a0 + 4, a5 = a0 + 5, a6 = a0 + 6, a7 = a0 + 7;
@@ -1173,11 +1216,13 @@ struct hsddp_batch {
     // the schedule SLOTS; a slot is free when no problem uses it (gait -1 on the device, listed in slot_free).
     std::vector<int> slot_refs;    // problems per slot (empty until the first restart)
     std::vector<int> slot_free;    // free slots, marked on the device
-    int* d_restart = nullptr;      // per-call argument lists (ints), d_restart_cap of them
-    double* d_restart_x0 = nullptr;
-    size_t d_restart_cap = 0, d_restart_x0_cap = 0;
+    int* d_args = nullptr;         // per-call argument lists of the calls that take problem lists (ints), d_args_cap of them
+    double* d_args_x0 = nullptr;
+    size_t d_args_cap = 0, d_args_x0_cap = 0;
     int* d_budget = nullptr;       // BatchPtrs::budget
     long long budget_rounds = -1;  // largest max_AL_iter x max_DDP_iter among the pending overrides (-1: none pending)
+    std::vector<char> budget_pending;  // [P] the problem's override is still pending (allocated with d_budget)
+    int n_budget_pending = 0;
     bool slots_marked = false;     // the slots no problem used are on the free list (done by the first restart)
 };
 
@@ -1339,8 +1384,8 @@ void free_problem_allocs(hsddp_batch* b) {
     b->mpc_ready = false;
     b->h_sched_stale = false;
     b->slot_refs.clear(); b->slot_free.clear();
-    b->d_restart = nullptr; b->d_restart_x0 = nullptr; b->d_restart_cap = b->d_restart_x0_cap = 0;
-    b->d_budget = nullptr; b->budget_rounds = -1;
+    b->d_args = nullptr; b->d_args_x0 = nullptr; b->d_args_cap = b->d_args_x0_cap = 0;
+    b->d_budget = nullptr; b->budget_rounds = -1; b->budget_pending.clear(); b->n_budget_pending = 0;
     b->d_spec_int = nullptr; b->d_spec_rec = nullptr; b->d_spec_out = nullptr; b->d_spec_int_cap = b->d_spec_rec_cap = b->d_spec_out_cap = 0;
     b->slots_marked = false;
 }
@@ -1619,11 +1664,11 @@ int hsddp_batch_mpc_update(hsddp_batch* b) {
     CK(cudaSetDevice(b->device));
     CK(cudaEventRecord(b->ev_u0, b->stream));
     DevSchedule* d_sched = const_cast<DevSchedule*>(b->bp.sched);
-    k_mpc_update_schedules<<<(b->n_sched + 127) / 128, 128, 0, b->stream>>>(b->lib, b->n_sched, b->d_sched_gait, b->d_sched_window, d_sched, b->d_mpc,
-                                                                              b->d_mpc_err);
+    k_mpc_update_schedules<<<(b->n_sched + 127) / 128, 128, 0, b->stream>>>(b->lib, b->n_sched, b->d_sched_gait, b->d_sched_window, nullptr, d_sched,
+                                                                              b->d_mpc, b->d_mpc_err);
     k_reference_rows<<<b->n_sched, 128, 0, b->stream>>>(b->lib, b->n_sched, b->d_sched_gait, b->d_sched_window, nullptr, d_sched, b->d_mpc,
                                                         const_cast<double*>(b->bp.xr), const_cast<double*>(b->bp.ur), const_cast<double*>(b->bp.prel), nullptr);
-    k_mpc_shift<<<b->bp.n_problems, kThreads, 0, b->stream>>>(b->bp, b->d_mpc);
+    k_mpc_shift<<<b->bp.n_problems, kThreads, 0, b->stream>>>(b->bp, b->d_mpc, nullptr);
     CK(cudaGetLastError());
     b->n_step_launches += 3;
     CK(cudaEventRecord(b->ev_u1, b->stream));
@@ -1710,6 +1755,65 @@ static int grow_slots(hsddp_batch* b, int add) {
     return HSDDP_OK;
 }
 
+// problems per slot, counted by the first call that moves problems between slots (restart, per-problem update)
+static void init_slot_refs(hsddp_batch* b) {
+    if (!b->slot_refs.empty()) return;
+    b->slot_refs.assign(b->n_sched, 0);
+    for (int s : b->h_sched_id) b->slot_refs[s]++;
+}
+
+// at least m free slots for a call on n problems
+static int ensure_free_slots(hsddp_batch* b, int m, int n) {
+    if ((int)b->slot_free.size() >= m) return HSDDP_OK;
+    // grow by half the capacity at least (a growth copies every slot), but never beyond the n_problems + n slots a call can
+    // need: at most n_problems are referenced, plus the m <= n being built
+    const int need = m - (int)b->slot_free.size();
+    return grow_slots(b, std::max(need, std::min(b->n_sched / 2, b->bp.n_problems + n - b->n_sched)));
+}
+
+// the slots that reference counts `refs` leave without a problem and that are not free yet: the old slots of the listed problems
+// (and, before the first such call, every slot no problem used from the start)
+static std::vector<int> released_slots(hsddp_batch* b, const std::vector<int>& refs, const std::vector<int>& free_after, int n, const int32_t* problem) {
+    std::vector<char> on_free(b->n_sched, 0);
+    for (int s : free_after) on_free[s] = 1;
+    std::vector<int> freed;
+    auto release = [&](int s) { if (refs[s] == 0 && !on_free[s]) { on_free[s] = 1; freed.push_back(s); } };
+    if (!b->slots_marked) for (int s = 0; s < b->n_sched; ++s) release(s);
+    else for (int k = 0; k < n; ++k) release(b->h_sched_id[problem[k]]);
+    return freed;
+}
+
+// a host list of n distinct problem indices, 1 <= n <= n_problems
+static int check_problem_list(hsddp_batch* b, int n, const int32_t* problem, const char* what) {
+    const int P = b->bp.n_problems;
+    if (n <= 0 || n > P || !problem) { g_last_error = std::string(what) + ": n must be in [1, n_problems] and the list given"; return HSDDP_ERR_ARG; }
+    std::vector<char> seen(P, 0);
+    for (int k = 0; k < n; ++k) {
+        if (problem[k] < 0 || problem[k] >= P) { g_last_error = std::string(what) + ": problem index out of range"; return HSDDP_ERR_ARG; }
+        if (seen[problem[k]]) { g_last_error = std::string(what) + ": repeated problem index"; return HSDDP_ERR_ARG; }
+        seen[problem[k]] = 1;
+    }
+    return HSDDP_OK;
+}
+
+// *d := the host ints h in the call's device argument list (queued on the handle's stream)
+static int stage_ints(hsddp_batch* b, const std::vector<int>& h, int** d) {
+    if (int rc = scratch(b, &b->d_args, &b->d_args_cap, h.size())) return rc;
+    CK(cudaMemcpyAsync(b->d_args, h.data(), h.size() * sizeof(int), cudaMemcpyHostToDevice, b->stream));
+    *d = b->d_args;
+    return HSDDP_OK;
+}
+
+// k_scatter_rows on the handle's stream: row idx[j] of dst := row j of src (src_stride 0: one row for all), for j < n
+static int scatter_rows(hsddp_batch* b, void* dst, int words, const int* idx, const void* src, int src_stride, int n) {
+    if (n <= 0) return HSDDP_OK;
+    const long long total = (long long)n * words;
+    k_scatter_rows<<<(unsigned)((total + 255) / 256), 256, 0, b->stream>>>((unsigned*)dst, words, idx, (const unsigned*)src, src_stride, n);
+    CK(cudaGetLastError());
+    b->n_step_launches++;
+    return HSDDP_OK;
+}
+
 int hsddp_batch_restart_problems(hsddp_batch* b, int n, const int32_t* problem, const int32_t* gait, const int32_t* window,
                                  const double* x0, const hsddp_options* first_solve) {
     return guarded([&]() -> int {
@@ -1729,15 +1833,13 @@ int hsddp_batch_restart_problems(hsddp_batch* b, int n, const int32_t* problem, 
         if (window[k] < 0) { g_last_error = "restart: window does not fit the gait table"; return HSDDP_ERR_ARG; }
     }
     CK(cudaSetDevice(b->device));
-    if (b->slot_refs.empty()) {
-        b->slot_refs.assign(b->n_sched, 0);
-        for (int s : b->h_sched_id) b->slot_refs[s]++;
-    }
+    init_slot_refs(b);
     int rc;
     if (first_solve && !b->d_budget) {
         if ((rc = dalloc(b, &b->d_budget, (size_t)2 * P))) return rc;
         CK(cudaMemsetAsync(b->d_budget, 0xff, sizeof(int) * 2 * P, b->stream));
         b->bp.budget = b->d_budget;
+        b->budget_pending.assign(P, 0);
     }
     // the call's distinct (gait, window) pairs, one new slot each
     std::map<std::pair<int, int>, int> pair_index;
@@ -1748,23 +1850,12 @@ int hsddp_batch_restart_problems(hsddp_batch* b, int n, const int32_t* problem, 
         pair_of[k] = it.first->second;
     }
     const int m = (int)bgait.size();
-    if ((int)b->slot_free.size() < m) {
-        // grow by half the capacity at least (a growth copies every slot), but never beyond the n_problems + n slots a call can
-        // need: at most n_problems are referenced, plus the m <= n being built
-        const int need = m - (int)b->slot_free.size();
-        const int add = std::max(need, std::min(b->n_sched / 2, P + n - b->n_sched));
-        if ((rc = grow_slots(b, add))) return rc;
-    }
+    if ((rc = ensure_free_slots(b, m, n))) return rc;
     // slot bookkeeping after the call (applied only once the build has succeeded)
     std::vector<int> free_after = b->slot_free, bslot(m), refs = b->slot_refs;
     for (int j = 0; j < m; ++j) { bslot[j] = free_after.back(); free_after.pop_back(); }
     for (int k = 0; k < n; ++k) { refs[b->h_sched_id[problem[k]]]--; refs[bslot[pair_of[k]]]++; }
-    std::vector<char> on_free(b->n_sched, 0);
-    for (int s : free_after) on_free[s] = 1;
-    std::vector<int> freed;
-    auto release = [&](int s) { if (refs[s] == 0 && !on_free[s]) { on_free[s] = 1; freed.push_back(s); } };
-    if (!b->slots_marked) for (int s = 0; s < b->n_sched; ++s) release(s);  // (also the slots no problem used from the start)
-    else for (int k = 0; k < n; ++k) release(b->h_sched_id[problem[k]]);
+    const std::vector<int> freed = released_slots(b, refs, free_after, n, problem);
     const int c = m + (int)freed.size();
     // argument lists: problem[n] slot[n] | gait[m] window[m] slot[m] status[m] | commit slot[c] gait[c] window[c]
     std::vector<int> h(2 * (size_t)n + 4 * (size_t)m + 3 * (size_t)c);
@@ -1774,10 +1865,9 @@ int hsddp_batch_restart_problems(hsddp_batch* b, int n, const int32_t* problem, 
     for (int k = 0; k < n; ++k) { a_prob[k] = problem[k]; a_slot[k] = bslot[pair_of[k]]; }
     for (int j = 0; j < m; ++j) { a_bg[j] = bgait[j]; a_bw[j] = bwin[j]; a_bs[j] = bslot[j]; a_st[j] = 0; a_cs[j] = bslot[j]; a_cg[j] = bgait[j]; a_cw[j] = bwin[j]; }
     for (int j = m; j < c; ++j) { a_cs[j] = freed[j - m]; a_cg[j] = -1; a_cw[j] = 0; }
-    if ((rc = scratch(b, &b->d_restart, &b->d_restart_cap, h.size())) || (rc = scratch(b, &b->d_restart_x0, &b->d_restart_x0_cap, (size_t)n * 24))) return rc;
-    int* d = b->d_restart;
-    CK(cudaMemcpyAsync(d, h.data(), h.size() * sizeof(int), cudaMemcpyHostToDevice, b->stream));
-    CK(cudaMemcpyAsync(b->d_restart_x0, x0, (size_t)n * 24 * sizeof(double), cudaMemcpyHostToDevice, b->stream));
+    int* d;
+    if ((rc = stage_ints(b, h, &d)) || (rc = scratch(b, &b->d_args_x0, &b->d_args_x0_cap, (size_t)n * 24))) return rc;
+    CK(cudaMemcpyAsync(b->d_args_x0, x0, (size_t)n * 24 * sizeof(double), cudaMemcpyHostToDevice, b->stream));
     // build into the free slots, then one host synchronise for the build status
     const int *d_bg = d + 2 * n, *d_bw = d_bg + m, *d_bs = d_bw + m;
     int* d_st = const_cast<int*>(d_bs + m);
@@ -1789,10 +1879,11 @@ int hsddp_batch_restart_problems(hsddp_batch* b, int n, const int32_t* problem, 
         if (a_st[j] == 1) { g_last_error = "restart: window does not fit the gait table"; return HSDDP_ERR_ARG; }
         if (a_st[j]) { g_last_error = "restart: schedule exceeds HSDDP_MAX_PHASES / the batch's node capacity"; return HSDDP_ERR_UNSUPPORTED; }
     }
-    RestartArgs ra{d, d + n, d_st + m, d_st + m + c, d_st + m + 2 * c, b->d_restart_x0, c,
+    RestartArgs ra{d, d + n, d_st + m, d_st + m + c, d_st + m + 2 * c, b->d_args_x0, c,
                    first_solve ? first_solve->max_AL_iter : -1, first_solve ? first_solve->max_DDP_iter : -1, b->d_sched_gait, b->d_sched_window, 0, {}};
+    // (the trial arrays of a batch larger than kClusterLsMax belong to launch positions, not to problems: hsddp_batch_solve_problems)
     for (const WsArray& a : workspace_arrays(b))
-        if ((a.flags & WS_RESTART) && *a.field) {
+        if ((a.flags & WS_RESTART) && *a.field && !((a.flags & WS_SMALL) && P > hsddp_batch::kClusterLsMax)) {
             if (ra.n_clear == kRestartClearMax) { g_last_error = "restart: more workspace arrays than kRestartClearMax"; return HSDDP_ERR_STATE; }
             ra.clear[ra.n_clear++] = {(unsigned*)*a.field, a.bytes() / sizeof(unsigned)};
         }
@@ -1807,6 +1898,88 @@ int hsddp_batch_restart_problems(hsddp_batch* b, int n, const int32_t* problem, 
     CK(cudaGetLastError());
     b->n_step_launches++;
     if (first_solve) b->budget_rounds = std::max(b->budget_rounds, (long long)first_solve->max_AL_iter * first_solve->max_DDP_iter);
+    if (b->d_budget)
+        for (int k = 0; k < n; ++k) {
+            char& q = b->budget_pending[problem[k]];
+            b->n_budget_pending += (first_solve ? 1 : 0) - q;
+            q = first_solve ? 1 : 0;
+        }
+    if (b->d_budget && b->n_budget_pending == 0) b->budget_rounds = -1;
+    return HSDDP_OK;
+    });
+}
+
+/* HKDProblem::update of the listed problems (see hsddp_batch_mpc_update and k_copy_slots).  Built before it is committed: the
+ * slots of the listed problems are copied to free slots and the copies stepped; only when every copy has succeeded do the listed
+ * problems move to them and get shifted, so a refusal leaves the batch as it was. */
+int hsddp_batch_mpc_update_problems(hsddp_batch* b, int n, const int32_t* problem) {
+    return guarded([&]() -> int {
+    if (!b || !b->has_problems) { g_last_error = "no problems set"; return HSDDP_ERR_STATE; }
+    if (!b->mpc_ready) { g_last_error = "hsddp_batch_mpc_update_problems needs the gait library on the device: set the problems with hsddp_batch_set_problems_from_gaits"; return HSDDP_ERR_STATE; }
+    int rc;
+    if ((rc = check_problem_list(b, n, problem, "mpc_update_problems"))) return rc;
+    CK(cudaSetDevice(b->device));
+    init_slot_refs(b);
+    // the distinct slots of the listed problems, one copy each (problems that share a slot share its copy)
+    std::map<int, int> copy_of;
+    std::vector<int> src, entry(n);
+    for (int k = 0; k < n; ++k) {
+        auto it = copy_of.emplace(b->h_sched_id[problem[k]], (int)src.size());
+        if (it.second) src.push_back(b->h_sched_id[problem[k]]);
+        entry[k] = it.first->second;
+    }
+    const int m = (int)src.size();
+    if ((rc = ensure_free_slots(b, m, n))) return rc;
+    // slot bookkeeping after the call (applied only once every copy has been stepped)
+    std::vector<int> free_after = b->slot_free, dst(m), refs = b->slot_refs;
+    for (int j = 0; j < m; ++j) { dst[j] = free_after.back(); free_after.pop_back(); }
+    for (int k = 0; k < n; ++k) { refs[src[entry[k]]]--; refs[dst[entry[k]]]++; }
+    const std::vector<int> freed = released_slots(b, refs, free_after, n, problem);
+    const int f = (int)freed.size();
+    // argument list: problem[n] slot[n] | src[m] dst[m] gait[m] window[m] | freed[f] | -1 | error flag
+    std::vector<int> h(2 * (size_t)n + 4 * (size_t)m + f + 2, 0);
+    for (int k = 0; k < n; ++k) { h[k] = problem[k]; h[n + k] = dst[entry[k]]; }
+    for (int j = 0; j < m; ++j) { h[2 * n + j] = src[j]; h[2 * n + m + j] = dst[j]; }
+    for (int j = 0; j < f; ++j) h[2 * n + 4 * m + j] = freed[j];
+    h[2 * n + 4 * m + f] = -1;
+    int* d;
+    if ((rc = stage_ints(b, h, &d))) return rc;
+    int *d_slot = d + n, *d_src = d + 2 * n, *d_dst = d_src + m, *d_gait = d_dst + m, *d_win = d_gait + m, *d_freed = d_win + m;
+    int *d_m1 = d_freed + f, *d_err = d_m1 + 1;
+    DevSchedule* sched = const_cast<DevSchedule*>(b->bp.sched);
+    SlotCopyArgs ca{d_src, d_dst, b->d_sched_gait, b->d_sched_window, d_gait, d_win, sched, b->lib.node_stride, 0, {}};
+    for (const SlotArray& a : slot_arrays(b)) {
+        if (ca.n_arrays == kSlotArraysMax) { g_last_error = "mpc_update_problems: more slot arrays than kSlotArraysMax"; return HSDDP_ERR_STATE; }
+        ca.arr[ca.n_arrays++] = {(unsigned*)*a.field, a.bytes / sizeof(unsigned)};
+    }
+    CK(cudaEventRecord(b->ev_u0, b->stream));
+    k_copy_slots<<<m, 128, 0, b->stream>>>(ca);
+    k_mpc_update_schedules<<<(m + 127) / 128, 128, 0, b->stream>>>(b->lib, m, d_gait, d_win, d_dst, sched, b->d_mpc, d_err);
+    k_reference_rows<<<m, 128, 0, b->stream>>>(b->lib, m, d_gait, d_win, d_dst, sched, b->d_mpc, const_cast<double*>(b->bp.xr),
+                                              const_cast<double*>(b->bp.ur), const_cast<double*>(b->bp.prel), nullptr);
+    CK(cudaGetLastError());
+    b->n_step_launches += 3;
+    int err = 0;
+    CK(cudaMemcpyAsync(&err, d_err, sizeof(int), cudaMemcpyDeviceToHost, b->stream));
+    CK(cudaStreamSynchronize(b->stream));
+    if (err) {  // the copies are dropped: their slots stay on the free list, marked free again on the device
+        if ((rc = scatter_rows(b, b->d_sched_gait, 1, d_dst, d_m1, 0, m))) return rc;
+        CK(cudaEventRecord(b->ev_u1, b->stream));
+        g_last_error = err == 1 ? "receding-horizon update: the reference table is exhausted" : "receding-horizon update: schedule exceeds HSDDP_MAX_PHASES / node capacity";
+        return err == 1 ? HSDDP_ERR_ARG : HSDDP_ERR_UNSUPPORTED;
+    }
+    // commit: the listed problems move to the stepped copies, slots nobody uses any more are freed, then the shift
+    if ((rc = scatter_rows(b, const_cast<int*>(b->bp.sched_id), 1, d, d_slot, 1, n)) || (rc = scatter_rows(b, b->d_sched_gait, 1, d_freed, d_m1, 0, f))) return rc;
+    k_mpc_shift<<<n, kThreads, 0, b->stream>>>(b->bp, b->d_mpc, d);
+    CK(cudaGetLastError());
+    b->n_step_launches++;
+    CK(cudaEventRecord(b->ev_u1, b->stream));
+    b->slot_refs.swap(refs);
+    for (int s : freed) free_after.push_back(s);
+    b->slot_free.swap(free_after);
+    for (int k = 0; k < n; ++k) b->h_sched_id[problem[k]] = dst[entry[k]];
+    b->h_sched_stale = true;
+    b->slots_marked = true;
     return HSDDP_OK;
     });
 }
@@ -1824,6 +1997,18 @@ int hsddp_batch_set_initial_condition(hsddp_batch* b, const double* x0) {
     CK(cudaMemcpyAsync(b->bp.x0, x0, sizeof(double) * 24 * b->bp.n_problems, cudaMemcpyHostToDevice, b->stream));
     CK(cudaStreamSynchronize(b->stream));
     return HSDDP_OK;
+}
+
+int hsddp_batch_set_initial_condition_problems(hsddp_batch* b, int n, const int32_t* problem, const double* x0) {
+    return guarded([&]() -> int {
+    if (!b || !b->has_problems || !x0) return HSDDP_ERR_ARG;
+    int rc, *d;
+    if ((rc = check_problem_list(b, n, problem, "set_initial_condition_problems"))) return rc;
+    CK(cudaSetDevice(b->device));
+    if ((rc = stage_ints(b, std::vector<int>(problem, problem + n), &d)) || (rc = scratch(b, &b->d_args_x0, &b->d_args_x0_cap, (size_t)n * 24))) return rc;
+    CK(cudaMemcpyAsync(b->d_args_x0, x0, (size_t)n * 24 * sizeof(double), cudaMemcpyHostToDevice, b->stream));
+    return scatter_rows(b, b->bp.x0, 48, d, b->d_args_x0, 48, n);
+    });
 }
 
 int hsddp_batch_reset(hsddp_batch* b) {
@@ -1878,8 +2063,8 @@ __global__ void k_order_by_iterations(const hsddp_info* info, int n, int* order)
     }
 }
 
-static int solve_phased(hsddp_batch* b, const hsddp_options& o) {
-    const int P = b->bp.n_problems;
+// problem[0 .. P) run (nullptr: every problem of the batch, P = n_problems)
+static int solve_phased(hsddp_batch* b, const hsddp_options& o, int P, const int32_t* problem) {
     const int G = std::min(hsddp_batch::kMaxGroups, std::max(1, P / hsddp_batch::kPhasedMinGroup));  // problems per group at least kPhasedMinGroup
     for (int g = 0; g < G; ++g) {
         if (!b->gstream[g]) {
@@ -1888,7 +2073,7 @@ static int solve_phased(hsddp_batch* b, const hsddp_options& o) {
         }
     }
     const int S = b->sweep_spec, cap = hsddp_batch::kSpecCap;
-    const size_t slice = (size_t)b->bp.max_stages * 312 + 600, spec_ints = (size_t)G * (2 * cap + 2) + P;
+    const size_t slice = (size_t)b->bp.max_stages * 312 + 600, spec_ints = (size_t)G * (2 * cap + 2) + b->bp.n_problems;
     if (S) {
         int rs = scratch(b, &b->d_spec_int, &b->d_spec_int_cap, spec_ints);
         if (!rs) rs = scratch(b, &b->d_spec_rec, &b->d_spec_rec_cap, (size_t)G * cap * S);
@@ -1898,7 +2083,8 @@ static int solve_phased(hsddp_batch* b, const hsddp_options& o) {
     CK(cudaEventRecord(b->ev0, b->stream));
     CK(cudaMemsetAsync(b->d_count, 0, 2 * hsddp_batch::kMaxGroups * sizeof(int), b->stream));
     if (S) CK(cudaMemsetAsync(b->d_spec_int, 0, spec_ints * sizeof(int), b->stream));
-    k_iota<<<(P + 255) / 256, 256, 0, b->stream>>>(b->d_active[0], P);
+    if (problem) CK(cudaMemcpyAsync(b->d_active[0], problem, sizeof(int) * P, cudaMemcpyHostToDevice, b->stream));
+    else k_iota<<<(P + 255) / 256, 256, 0, b->stream>>>(b->d_active[0], P);
     CK(cudaEventRecord(b->ev_fork, b->stream));
     // (restarted problems may have a larger budget for this solve: BatchPtrs::budget)
     const int rounds = (int)std::min<long long>(std::max((long long)std::max(0, o.max_AL_iter) * (long long)std::max(0, o.max_DDP_iter), b->budget_rounds), 1000000LL);
@@ -1951,54 +2137,107 @@ int hsddp_batch_set_solve_mode(hsddp_batch* b, int mode) {
     return HSDDP_OK;
 }
 
-// the per-problem budgets of restarted problems apply to one solve: cleared on the stream once it is queued
-static int consume_budget(hsddp_batch* b) {
+// the per-problem budgets of restarted problems apply to one solve: those of the problems it ran (problem[0 .. n), nullptr:
+// every problem) are cleared on the stream once it is queued
+static int consume_budget(hsddp_batch* b, int n, const int32_t* problem) {
     if (b->budget_rounds < 0) return HSDDP_OK;
-    CK(cudaMemsetAsync(b->d_budget, 0xff, sizeof(int) * 2 * b->bp.n_problems, b->stream));
-    b->budget_rounds = -1;
+    if (!problem) {
+        CK(cudaMemsetAsync(b->d_budget, 0xff, sizeof(int) * 2 * b->bp.n_problems, b->stream));
+        std::fill(b->budget_pending.begin(), b->budget_pending.end(), 0);
+        b->n_budget_pending = 0;
+    } else {
+        std::vector<int> h;
+        for (int k = 0; k < n; ++k)
+            if (b->budget_pending[problem[k]]) { h.push_back(problem[k]); b->budget_pending[problem[k]] = 0; }
+        const int c = (int)h.size();
+        if (c) {
+            b->n_budget_pending -= c;
+            h.push_back(-1); h.push_back(-1);
+            int rc, *d;
+            if ((rc = stage_ints(b, h, &d)) || (rc = scatter_rows(b, b->d_budget, 2, d, d + c, 0, c))) return rc;
+        }
+    }
+    if (b->n_budget_pending == 0) b->budget_rounds = -1;
     return HSDDP_OK;
 }
 
-int hsddp_batch_solve_async(hsddp_batch* b, const hsddp_options* opt) {
-    if (!b || !b->has_problems) { g_last_error = "no problems set"; return HSDDP_ERR_STATE; }
+// trial arrays of k_solve_lat4 for kClusterLsMax launch positions, allocated by the first solve of at most kClusterLsMax listed
+// problems in a batch too large to have them per problem
+static int alloc_cluster_ls(hsddp_batch* b) {
+    for (const WsArray& a : workspace_arrays(b)) {
+        if (!(a.flags & WS_SMALL)) continue;
+        const size_t bytes = a.bytes() * hsddp_batch::kClusterLsMax;
+        if (int rc = dalloc_bytes(b, a.field, bytes)) return rc;
+        CK(cudaMemsetAsync(*a.field, 0, bytes, b->stream));
+    }
+    return HSDDP_OK;
+}
+
+// the solve of problem[0 .. n) (nullptr: every problem, n = n_problems), in the driver a batch of n problems takes
+static int solve_list(hsddp_batch* b, const hsddp_options* opt, int n, const int32_t* problem) {
     int rc = check_opt(opt);
     if (rc) return rc;
     CK(cudaSetDevice(b->device));
     const hsddp_options o = opt ? *opt : default_options();
+    const int P = b->bp.n_problems;
     // auto: the persistent kernel up to ~7 waves of blocks (its work queue visits the problems longest-first from the second
     // solve on, which keeps the tail short); beyond that the phased driver, whose phase-homogeneous kernels keep the
     // instruction cache hot and whose launch tails are hidden by driving four index ranges on their own streams
     // (measured on config 3, persistent vs phased, ms, final code of round 2: 2,048 problems 57 vs 69, 4,096: 98 vs 100,
     // 5,120: ~121 vs 117, 6,144: 145 vs 135, 8,192: 199 vs 163 -- profiles/r02an_*: the switch is at 5.5 waves of blocks, 4,884 problems)
-    const bool phased = b->solve_mode == 2 || (b->solve_mode == 0 && 2 * b->bp.n_problems >= 11 * b->n_sm * b->blocks_per_sm);
+    const bool phased = b->solve_mode == 2 || (b->solve_mode == 0 && 2 * n >= 11 * b->n_sm * b->blocks_per_sm);
     if (phased) {
-        rc = solve_phased(b, o);
-        if (rc == HSDDP_OK) rc = consume_budget(b);
+        rc = solve_phased(b, o, n, problem);
+        if (rc == HSDDP_OK) rc = consume_budget(b, n, problem);
         return rc;
+    }
+    const bool cluster = n <= hsddp_batch::kClusterLsMax && o.MS;
+    if (cluster && problem && !b->bp.ls_mail && (rc = alloc_cluster_ls(b))) return rc;
+    const int grid = (n <= 2 * b->n_sm) ? n : std::min(n, b->n_sm * b->blocks_per_sm);
+    BatchPtrs bp = b->bp;
+    if (problem) {
+        // the work queue (the cluster index of k_solve_lat4): the list, then n_problems, which ends a block, up to the last
+        // entry a block can draw.  It replaces the queue-order hint of the whole batch.
+        std::vector<int> q(std::min(P, n + grid), P);
+        std::copy(problem, problem + n, q.begin());
+        CK(cudaMemcpyAsync(b->d_order, q.data(), q.size() * sizeof(int), cudaMemcpyHostToDevice, b->stream));
+        bp.order = b->d_order;
+        b->have_order = false;
     }
     CK(cudaMemsetAsync(b->bp.work_counter, 0, sizeof(int), b->stream));
     CK(cudaEventRecord(b->ev0, b->stream));
-    if (b->bp.ls_mail && b->bp.n_problems <= hsddp_batch::kClusterLsMax && o.MS) {
-        k_solve_lat4<<<4 * b->bp.n_problems, kThreads, 0, b->stream>>>(b->bp, o);
-    } else if (b->bp.n_problems <= 2 * b->n_sm) {
-        k_solve_lat<<<b->bp.n_problems, kThreads, 0, b->stream>>>(b->bp, o);
+    if (b->bp.ls_mail && cluster) {
+        k_solve_lat4<<<4 * n, kThreads, 0, b->stream>>>(bp, o);
+    } else if (n <= 2 * b->n_sm) {
+        k_solve_lat<<<n, kThreads, 0, b->stream>>>(bp, o);
     } else {
-        const int grid = std::min(b->bp.n_problems, b->n_sm * b->blocks_per_sm);
-        BatchPtrs bp = b->bp;
-        bp.order = b->have_order ? b->d_order : nullptr;
+        if (!problem) bp.order = b->have_order ? b->d_order : nullptr;
         k_solve<<<grid, kThreads, 0, b->stream>>>(bp, o);
     }
     CK(cudaGetLastError());
     b->n_solve_launches++;
     CK(cudaEventRecord(b->ev1, b->stream));
-    if ((rc = consume_budget(b))) return rc;
-    if (b->bp.n_problems > 2 * b->n_sm) {  // (after the timed region of last_solve_ms: ~10 us, part of every bench step)
+    if ((rc = consume_budget(b, n, problem))) return rc;
+    if (!problem && P > 2 * b->n_sm) {  // (after the timed region of last_solve_ms: ~10 us, part of every bench step)
         k_order_by_iterations<<<1, 256, 0, b->stream>>>(b->bp.info, b->bp.n_problems, b->d_order);
         CK(cudaGetLastError());
         b->n_solve_launches++;
         b->have_order = true;
     }
     return HSDDP_OK;
+}
+
+int hsddp_batch_solve_async(hsddp_batch* b, const hsddp_options* opt) {
+    if (!b || !b->has_problems) { g_last_error = "no problems set"; return HSDDP_ERR_STATE; }
+    return solve_list(b, opt, b->bp.n_problems, nullptr);
+}
+
+int hsddp_batch_solve_problems_async(hsddp_batch* b, int n, const int32_t* problem, const hsddp_options* opt) {
+    return guarded([&]() -> int {
+    if (!b || !b->has_problems) { g_last_error = "no problems set"; return HSDDP_ERR_STATE; }
+    if (int rc = check_problem_list(b, n, problem, "solve_problems")) return rc;
+    return solve_list(b, opt, n, problem);
+    });
 }
 
 int hsddp_batch_sync(hsddp_batch* b) {
@@ -2010,6 +2249,12 @@ int hsddp_batch_sync(hsddp_batch* b) {
 
 int hsddp_batch_solve(hsddp_batch* b, const hsddp_options* opt) {
     int rc = hsddp_batch_solve_async(b, opt);
+    if (rc) return rc;
+    return hsddp_batch_sync(b);
+}
+
+int hsddp_batch_solve_problems(hsddp_batch* b, int n, const int32_t* problem, const hsddp_options* opt) {
+    int rc = hsddp_batch_solve_problems_async(b, n, problem, opt);
     if (rc) return rc;
     return hsddp_batch_sync(b);
 }
@@ -2219,22 +2464,37 @@ int hsddp_batch_get_gains_compact(hsddp_batch* b, int row0, int nrows, double* o
     return HSDDP_OK;
 }
 
-int hsddp_batch_get_mpc_command(hsddp_batch* b, int n_steps, hsddp_mpc_command* out) {
-    if (!b || !b->has_problems || !out || n_steps < 1 || n_steps > HSDDP_CMD_MAX_STEPS) return HSDDP_ERR_ARG;
+// the command records of problem[0 .. n) (nullptr: every problem, n = n_problems) into out[0 .. n), one transfer
+static int get_commands(hsddp_batch* b, int n_steps, int n, const int32_t* problem, hsddp_mpc_command* out) {
     CK(cudaSetDevice(b->device));
-    const size_t bytes = sizeof(hsddp_mpc_command) * (size_t)b->bp.n_problems;
     if (!b->d_cmd) {
         void* q = nullptr;
-        CK(cudaMalloc(&q, bytes));
+        CK(cudaMalloc(&q, sizeof(hsddp_mpc_command) * (size_t)b->bp.n_problems));
         b->allocs.push_back(q);
         b->d_cmd = (hsddp_mpc_command*)q;
     }
-    k_command<<<b->bp.n_problems, 128, 0, b->stream>>>(b->bp, n_steps, b->d_cmd);
+    int* d = nullptr;
+    if (problem)
+        if (int rc = stage_ints(b, std::vector<int>(problem, problem + n), &d)) return rc;
+    k_command<<<n, 128, 0, b->stream>>>(b->bp, n_steps, b->d_cmd, d);
     CK(cudaGetLastError());
     b->n_step_launches++;
-    CK(cudaMemcpyAsync(out, b->d_cmd, bytes, cudaMemcpyDeviceToHost, b->stream));
+    CK(cudaMemcpyAsync(out, b->d_cmd, sizeof(hsddp_mpc_command) * (size_t)n, cudaMemcpyDeviceToHost, b->stream));
     CK(cudaStreamSynchronize(b->stream));
     return HSDDP_OK;
+}
+
+int hsddp_batch_get_mpc_command(hsddp_batch* b, int n_steps, hsddp_mpc_command* out) {
+    if (!b || !b->has_problems || !out || n_steps < 1 || n_steps > HSDDP_CMD_MAX_STEPS) return HSDDP_ERR_ARG;
+    return get_commands(b, n_steps, b->bp.n_problems, nullptr, out);
+}
+
+int hsddp_batch_get_mpc_command_problems(hsddp_batch* b, int n_steps, int n, const int32_t* problem, hsddp_mpc_command* out) {
+    return guarded([&]() -> int {
+    if (!b || !b->has_problems || !out || n_steps < 1 || n_steps > HSDDP_CMD_MAX_STEPS) return HSDDP_ERR_ARG;
+    if (int rc = check_problem_list(b, n, problem, "get_mpc_command_problems")) return rc;
+    return get_commands(b, n_steps, n, problem, out);
+    });
 }
 
 int hsddp_batch_event_record(hsddp_batch* b, int slot) {

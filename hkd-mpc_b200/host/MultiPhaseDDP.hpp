@@ -140,6 +140,27 @@ public:
         check(hsddp_batch_get_schedule_ids(b_, v.data()), "hsddp_batch_get_schedule_ids");
         return v;
     }
+    // The MPC tick of the listed problems only (HKDMPCSolver::update of the robots whose mpc_data arrived, HKDMPC.cpp:169-200):
+    // update, initial states (24 doubles per listed problem), solve, commands (one per listed problem, in list order).  The other
+    // problems keep everything.
+    void update_problems(const std::vector<int32_t>& problem) {
+        check(hsddp_batch_mpc_update_problems(b_, (int)problem.size(), problem.data()), "hsddp_batch_mpc_update_problems");
+    }
+    void set_initial_condition_problems(const std::vector<int32_t>& problem, const std::vector<double>& x0) {
+        if (x0.size() != 24 * problem.size()) throw std::invalid_argument("x0 must hold 24 doubles per listed problem");
+        check(hsddp_batch_set_initial_condition_problems(b_, (int)problem.size(), problem.data(), x0.data()), "hsddp_batch_set_initial_condition_problems");
+    }
+    void solve_problems(const std::vector<int32_t>& problem, HSDDP_OPTION option) {
+        check(hsddp_batch_solve_problems(b_, (int)problem.size(), problem.data(), &option), "hsddp_batch_solve_problems");
+    }
+    void solve_problems_async(const std::vector<int32_t>& problem, HSDDP_OPTION option) {
+        check(hsddp_batch_solve_problems_async(b_, (int)problem.size(), problem.data(), &option), "hsddp_batch_solve_problems_async");
+    }
+    std::vector<hsddp_mpc_command> get_mpc_command_problems(const std::vector<int32_t>& problem, int n_steps = 8) {
+        std::vector<hsddp_mpc_command> v(problem.size());
+        check(hsddp_batch_get_mpc_command_problems(b_, n_steps, (int)problem.size(), problem.data(), v.data()), "hsddp_batch_get_mpc_command_problems");
+        return v;
+    }
     void set_initial_condition(const std::vector<double>& x0) {
         if ((int)x0.size() != 24 * n_) throw std::invalid_argument("x0 must hold 24 doubles per problem");
         check(hsddp_batch_set_initial_condition(b_, x0.data()), "hsddp_batch_set_initial_condition");
@@ -245,6 +266,25 @@ public:
             parts_[g]->set_multiPhaseProblem(used, sid, cparams);
         }
     }
+    // the same from the gait library (every device gets the whole library and the schedules its problems use): the form that
+    // supports update_problems and restart_problems
+    void set_multiPhaseProblem_from_gaits(const std::vector<int32_t>& gait_rows, const std::vector<float>& gait_dt, const std::vector<double>& body_state,
+                                          const std::vector<double>& qJ, const std::vector<double>& foot_placements, const std::vector<double>& grf,
+                                          const std::vector<int32_t>& contact, const std::vector<int32_t>& sched_gait, const std::vector<int32_t>& sched_window,
+                                          float plan_duration, const std::vector<int32_t>& schedule_id, const hsddp_constraint_params* cparams = nullptr) {
+        n_ = (int)schedule_id.size();
+        for (int g = 0; g < n_devices(); ++g) {
+            int lo, hi;
+            shard_range(n_, g, n_devices(), lo, hi);
+            std::vector<int32_t> remap(sched_gait.size(), -1), sid, sg, sw;
+            for (int i = lo; i < hi; ++i) {
+                int32_t& r = remap[schedule_id[i]];
+                if (r < 0) { r = (int32_t)sg.size(); sg.push_back(sched_gait[schedule_id[i]]); sw.push_back(sched_window[schedule_id[i]]); }
+                sid.push_back(r);
+            }
+            parts_[g]->set_multiPhaseProblem_from_gaits(gait_rows, gait_dt, body_state, qJ, foot_placements, grf, contact, sg, sw, plan_duration, sid, cparams);
+        }
+    }
     void set_initial_condition(const std::vector<double>& x0) {
         for (int g = 0; g < n_devices(); ++g) {
             int lo, hi;
@@ -259,27 +299,46 @@ public:
                           const std::vector<double>& x0, const HSDDP_OPTION* first_solve = nullptr) {
         if (gait.size() != problem.size() || window.size() != problem.size() || x0.size() != 24 * problem.size())
             throw std::invalid_argument("restart_problems: one gait, one window and 24 doubles of x0 per problem");
-        std::vector<char> seen(n_, 0);
-        for (int32_t p : problem) {
-            if (p < 0 || p >= n_ || seen[p]) throw std::invalid_argument("restart_problems: problem index out of range or repeated");
-            seen[p] = 1;
-        }
-        for (int g = 0; g < n_devices(); ++g) {
-            int lo, hi;
-            shard_range(n_, g, n_devices(), lo, hi);
-            std::vector<int32_t> lp, lg, lw;
+        split(problem, "restart_problems", [&](int g, const std::vector<int32_t>& lp, const std::vector<size_t>& at) {
+            std::vector<int32_t> lg, lw;
             std::vector<double> lx;
-            for (size_t k = 0; k < problem.size(); ++k) {
-                if (problem[k] < lo || problem[k] >= hi) continue;
-                lp.push_back(problem[k] - lo); lg.push_back(gait[k]); lw.push_back(window[k]);
+            for (size_t k : at) {
+                lg.push_back(gait[k]); lw.push_back(window[k]);
                 lx.insert(lx.end(), x0.begin() + 24 * k, x0.begin() + 24 * (k + 1));
             }
-            if (!lp.empty()) parts_[g]->restart_problems(lp, lg, lw, lx, first_solve);
-        }
+            parts_[g]->restart_problems(lp, lg, lw, lx, first_solve);
+        });
     }
     void solve(HSDDP_OPTION option) {
         for (auto& p : parts_) p->solve_async(option);
         for (auto& p : parts_) p->sync();
+    }
+    // The per-problem tick with GLOBAL problem indices, split per device as restart_problems does (a device with no listed
+    // problem is not called).  solve_problems queues every device's part before it waits for any; get_mpc_command_problems
+    // returns the records in the order of `problem`.
+    void update_problems(const std::vector<int32_t>& problem) {
+        split(problem, "update_problems", [&](int g, const std::vector<int32_t>& lp, const std::vector<size_t>&) { parts_[g]->update_problems(lp); });
+    }
+    void set_initial_condition_problems(const std::vector<int32_t>& problem, const std::vector<double>& x0) {
+        if (x0.size() != 24 * problem.size()) throw std::invalid_argument("x0 must hold 24 doubles per listed problem");
+        split(problem, "set_initial_condition_problems", [&](int g, const std::vector<int32_t>& lp, const std::vector<size_t>& at) {
+            std::vector<double> lx;
+            for (size_t k : at) lx.insert(lx.end(), x0.begin() + 24 * k, x0.begin() + 24 * (k + 1));
+            parts_[g]->set_initial_condition_problems(lp, lx);
+        });
+    }
+    void solve_problems(const std::vector<int32_t>& problem, HSDDP_OPTION option) {
+        std::vector<int> queued;
+        split(problem, "solve_problems", [&](int g, const std::vector<int32_t>& lp, const std::vector<size_t>&) { parts_[g]->solve_problems_async(lp, option); queued.push_back(g); });
+        for (int g : queued) parts_[g]->sync();
+    }
+    std::vector<hsddp_mpc_command> get_mpc_command_problems(const std::vector<int32_t>& problem, int n_steps = 8) {
+        std::vector<hsddp_mpc_command> all(problem.size());
+        split(problem, "get_mpc_command_problems", [&](int g, const std::vector<int32_t>& lp, const std::vector<size_t>& at) {
+            auto v = parts_[g]->get_mpc_command_problems(lp, n_steps);
+            for (size_t k = 0; k < at.size(); ++k) all[at[k]] = v[k];
+        });
+        return all;
     }
     std::vector<hsddp_info> get_info() {
         std::vector<hsddp_info> all;
@@ -293,6 +352,25 @@ public:
     }
     MultiPhaseDDP<double>& part(int g) { return *parts_[g]; }
 private:
+    // f(g, local indices, positions in `problem`) for every device g that holds a listed problem; the indices are checked for
+    // all devices first
+    template <class F>
+    void split(const std::vector<int32_t>& problem, const char* what, F&& f) {
+        std::vector<char> seen(n_, 0);
+        for (int32_t p : problem) {
+            if (p < 0 || p >= n_ || seen[p]) throw std::invalid_argument(std::string(what) + ": problem index out of range or repeated");
+            seen[p] = 1;
+        }
+        for (int g = 0; g < n_devices(); ++g) {
+            int lo, hi;
+            shard_range(n_, g, n_devices(), lo, hi);
+            std::vector<int32_t> lp;
+            std::vector<size_t> at;
+            for (size_t k = 0; k < problem.size(); ++k)
+                if (problem[k] >= lo && problem[k] < hi) { lp.push_back(problem[k] - lo); at.push_back(k); }
+            if (!lp.empty()) f(g, lp, at);
+        }
+    }
     std::vector<std::unique_ptr<MultiPhaseDDP<double>>> parts_;
     int n_ = 0;
 };

@@ -199,6 +199,30 @@ int hsddp_batch_restart_problems(hsddp_batch* b, int n, const int32_t* problem, 
 /* schedule index of every problem ([n_problems]); pass it to hsddp_batch_get_schedule */
 int hsddp_batch_get_schedule_ids(hsddp_batch* b, int32_t* out);
 
+/* Per-problem MPC ticks.  In the reference every robot runs HKDMPCSolver::update (HKDMPC/HKDMPC.cpp:169-200) when its own
+ * mpc_data LCM message arrives, so the robots of a fleet tick at their own times, not in lockstep.  These entry points tick
+ * the LISTED problems of a batch: `problem` is a host list of n distinct indices in [0, n_problems), 1 <= n <= n_problems
+ * (HSDDP_ERR_ARG otherwise, nothing changed).  Each listed problem gets exactly what the whole-batch call computes for it;
+ * every other problem keeps its trajectories, gains, ReB / AL parameters, info, trace, pending first_solve budget and schedule
+ * slot bit for bit.  A tick of some robots: update, initial states, solve, commands of the same list (restart a problem, if
+ * needed, after the update of its tick, as for the whole batch).
+ *
+ * HKDProblem::update (HKDProblem.cpp:117-222, as hsddp_batch_mpc_update) of the listed problems.  Schedules are shared by slot,
+ * so each slot a listed problem uses is copied to a free slot and the copy is stepped; once every copy has succeeded the listed
+ * problems move to their copies (problems of the call that shared a slot share its copy) and are shifted.  HSDDP_ERR_ARG (the
+ * reference table is exhausted) and HSDDP_ERR_UNSUPPORTED (table limits) leave the batch as it was.  A handle never holds more
+ * than n_problems + n slots (or the schedule count it was set with, if larger).  Needs the gait library on the device. */
+int hsddp_batch_mpc_update_problems(hsddp_batch* b, int n, const int32_t* problem);
+/* MultiPhaseDDP::set_initial_condition (MultiPhaseDDP.h:37) of the listed problems: x0 is [n][24] on the host, row k for
+ * problem[k] */
+int hsddp_batch_set_initial_condition_problems(hsddp_batch* b, int n, const int32_t* problem, const double* x0);
+/* MultiPhaseDDP::solve (MultiPhaseDDP.cpp:232-428) of the listed problems, in the kernel a batch of n problems would run
+ * (same thresholds and hsddp_batch_set_solve_mode rules).  Pending first_solve budgets of the listed problems are used and
+ * cleared; those of the other problems stay pending.  The _async form returns once the work is queued (pair with
+ * hsddp_batch_sync); one solve at a time per handle. */
+int hsddp_batch_solve_problems(hsddp_batch* b, int n, const int32_t* problem, const hsddp_options* opt);
+int hsddp_batch_solve_problems_async(hsddp_batch* b, int n, const int32_t* problem, const hsddp_options* opt);
+
 /* MultiPhaseDDP::solve(HSDDP_OPTION) (MultiPhaseDDP.cpp:232-428) for every problem:
  * one persistent kernel, one thread block per problem, iteration control on the device. */
 int hsddp_batch_solve(hsddp_batch* b, const hsddp_options* opt);
@@ -304,6 +328,9 @@ typedef struct hsddp_mpc_command {
 } hsddp_mpc_command;
 /* n_steps = nsteps_between_mpc + 7 (8 in the reference), at most HSDDP_CMD_MAX_STEPS; out: [n_problems] on the host */
 int hsddp_batch_get_mpc_command(hsddp_batch* b, int n_steps, hsddp_mpc_command* out);
+/* HKDMPCSolver::publish_mpc_cmd + update_foot_placement (HKDMPC.cpp:207-298) of the listed problems (see
+ * hsddp_batch_mpc_update_problems): out is [n] on the host, record k for problem[k] */
+int hsddp_batch_get_mpc_command_problems(hsddp_batch* b, int n_steps, int n, const int32_t* problem, hsddp_mpc_command* out);
 
 /* CUDA-event timing on the handle's stream (slots 0..7): record, then elapsed ms between two slots */
 int hsddp_batch_event_record(hsddp_batch* b, int slot);
