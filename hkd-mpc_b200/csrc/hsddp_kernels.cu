@@ -974,10 +974,30 @@ __device__ inline void shift_rows_down(double* a, int total_rows, int row_len, i
     }
 }
 
-// block j shifts problem list[j] (nullptr: problem j)
-__global__ void __launch_bounds__(kThreads) k_mpc_shift(BatchPtrs bp, const MpcSched* mpc, const int* list) {
-    const int pid = list ? list[blockIdx.x] : (int)blockIdx.x, tid = threadIdx.x;
-    const int sid = bp.sched_id[pid];
+// The device commit of a call that moves listed problems to new schedule slots (plan_slot_moves), once they have been built: block j
+// binds problem[j] to slot[j], block 0 writes gait / window of the m target slots and gait -1 of the f freed ones (a free slot
+// carries gait -1 on the device, which the receding-horizon update skips; the targets carry it until here).
+struct SlotMoves {
+    int *problem, *slot;          // [launch blocks] (problem nullptr: no move)
+    int *target, *gait, *window;  // [m]
+    int* freed;                   // [f]
+    int m, f;
+    int *sched_gait, *sched_window;  // per slot
+};
+
+__device__ inline void write_slot_moves(const SlotMoves& mv, const int* sched_id) {
+    if (threadIdx.x == 0) const_cast<int*>(sched_id)[mv.problem[blockIdx.x]] = mv.slot[blockIdx.x];
+    if (blockIdx.x != 0) return;
+    for (int e = threadIdx.x; e < mv.m; e += blockDim.x) { mv.sched_gait[mv.target[e]] = mv.gait[e]; mv.sched_window[mv.target[e]] = mv.window[e]; }
+    for (int e = threadIdx.x; e < mv.f; e += blockDim.x) mv.sched_gait[mv.freed[e]] = -1;
+}
+
+// block j shifts problem j, or with moves (hsddp_batch_mpc_update_problems) moves problem mv.problem[j] to its stepped copy
+// mv.slot[j] and shifts it there (a block reads its slot from the list, not the sched_id that another block writes)
+__global__ void __launch_bounds__(kThreads) k_mpc_shift(BatchPtrs bp, const MpcSched* mpc, SlotMoves mv) {
+    if (mv.problem) write_slot_moves(mv, bp.sched_id);
+    const int pid = mv.problem ? mv.problem[blockIdx.x] : (int)blockIdx.x, tid = threadIdx.x;
+    const int sid = mv.problem ? mv.slot[blockIdx.x] : bp.sched_id[pid];
     const MpcSched& m = mpc[sid];
     if (m.status) return;
     const DevSchedule& sc = bp.sched[sid];  // the schedule AFTER the update
@@ -1040,8 +1060,7 @@ __global__ void __launch_bounds__(kThreads) k_mpc_shift(BatchPtrs bp, const MpcS
 // ---------------------------------------------------------------------------
 // HKDMPCSolver::initialize (HKDMPC.cpp:44-69) for a subset of the batch (hsddp_batch_restart_problems).  Launched only after
 // the new schedules have been built and checked, so nothing here can fail.  One block per restarted problem j:
-//   - problem[j] is bound to schedule slot slot[j]; block 0 also writes the slot table of the call: gait / window of every new
-//     slot, gait -1 for every slot no problem uses any more (the receding-horizon update skips those);
+//   - the slot moves of the call (write_slot_moves: problem j is mv.problem[j]);
 //   - the workspace arrays marked WS_RESTART are zeroed over the batch's full row count (what a fresh batch starts from: rows
 //     the new schedule does not have stay zero, and no lq / tq record of the old schedule survives), info / ctl are reset,
 //     then the cold start of a new problem;
@@ -1049,21 +1068,16 @@ __global__ void __launch_bounds__(kThreads) k_mpc_shift(BatchPtrs bp, const MpcS
 // ---------------------------------------------------------------------------
 constexpr int kRestartClearMax = 32;
 struct RestartArgs {
-    const int *problem, *slot;           // [n]
-    const int *cslot, *cgait, *cwindow;  // [n_commit]
-    const double* x0;                    // [n][24]
-    int n_commit, max_al, max_ddp;
-    int *sched_gait, *sched_window;
+    const double* x0;  // [n][24]
+    int max_al, max_ddp;
     int n_clear;
     struct { unsigned* base; size_t words; } clear[kRestartClearMax];  // arrays to zero: base, 4-byte words per problem
 };
 
-__global__ void __launch_bounds__(kThreads) k_restart(BatchPtrs bp, RestartArgs ra) {
+__global__ void __launch_bounds__(kThreads) k_restart(BatchPtrs bp, SlotMoves mv, RestartArgs ra) {
     __shared__ Smem sm;
-    const int j = blockIdx.x, pid = ra.problem[j];
-    if (blockIdx.x == 0)
-        for (int e = threadIdx.x; e < ra.n_commit; e += kThreads) { ra.sched_gait[ra.cslot[e]] = ra.cgait[e]; ra.sched_window[ra.cslot[e]] = ra.cwindow[e]; }
-    if (threadIdx.x == 0) const_cast<int*>(bp.sched_id)[pid] = ra.slot[j];
+    const int j = blockIdx.x, pid = mv.problem[j];
+    write_slot_moves(mv, bp.sched_id);
     const size_t P = pid;
     for (int a = 0; a < ra.n_clear; ++a) {
         unsigned* p = ra.clear[a].base + P * ra.clear[a].words;
@@ -1083,9 +1097,9 @@ __global__ void __launch_bounds__(kThreads) k_restart(BatchPtrs bp, RestartArgs 
 
 // ---------------------------------------------------------------------------
 // Receding-horizon update of listed problems (hsddp_batch_mpc_update_problems).  Problems share a schedule slot, so a slot that
-// listed problems use is first copied, one block per slot: slot src[j] goes to the free slot dst[j] in every slot array, the copy
-// gets its own reference rows (ref_off = dst[j] x node_stride), and gait / window of entry j are listed for the update kernels,
-// which then step the copies only.
+// listed problems use is first copied, one block per slot: slot src[j] goes to the free slot dst[j] in every slot array but gait /
+// window (the copy stays free until the commit), the copy gets its own reference rows (ref_off = dst[j] x node_stride), and gait /
+// window of entry j are listed for the update kernels, which then step the copies only, and for the commit.
 // ---------------------------------------------------------------------------
 constexpr int kSlotArraysMax = 8;
 struct SlotCopyArgs {
@@ -1110,7 +1124,7 @@ __global__ void k_copy_slots(SlotCopyArgs a) {
 }
 
 // row idx[j] of dst := row j of src (src_stride 0: the same row for every j), rows of `words` 4-byte words.  Writes the per-problem
-// rows of the list-driven entry points: initial states, schedule slots, cleared budgets, free-slot marks.
+// rows of the list-driven entry points: initial states and cleared budgets.
 __global__ void k_scatter_rows(unsigned* dst, int words, const int* idx, const unsigned* src, int src_stride, int n) {
     const long long e = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (e >= (long long)n * words) return;
@@ -1668,7 +1682,7 @@ int hsddp_batch_mpc_update(hsddp_batch* b) {
                                                                               b->d_mpc, b->d_mpc_err);
     k_reference_rows<<<b->n_sched, 128, 0, b->stream>>>(b->lib, b->n_sched, b->d_sched_gait, b->d_sched_window, nullptr, d_sched, b->d_mpc,
                                                         const_cast<double*>(b->bp.xr), const_cast<double*>(b->bp.ur), const_cast<double*>(b->bp.prel), nullptr);
-    k_mpc_shift<<<b->bp.n_problems, kThreads, 0, b->stream>>>(b->bp, b->d_mpc, nullptr);
+    k_mpc_shift<<<b->bp.n_problems, kThreads, 0, b->stream>>>(b->bp, b->d_mpc, SlotMoves{});
     CK(cudaGetLastError());
     b->n_step_launches += 3;
     CK(cudaEventRecord(b->ev_u1, b->stream));
@@ -1755,34 +1769,6 @@ static int grow_slots(hsddp_batch* b, int add) {
     return HSDDP_OK;
 }
 
-// problems per slot, counted by the first call that moves problems between slots (restart, per-problem update)
-static void init_slot_refs(hsddp_batch* b) {
-    if (!b->slot_refs.empty()) return;
-    b->slot_refs.assign(b->n_sched, 0);
-    for (int s : b->h_sched_id) b->slot_refs[s]++;
-}
-
-// at least m free slots for a call on n problems
-static int ensure_free_slots(hsddp_batch* b, int m, int n) {
-    if ((int)b->slot_free.size() >= m) return HSDDP_OK;
-    // grow by half the capacity at least (a growth copies every slot), but never beyond the n_problems + n slots a call can
-    // need: at most n_problems are referenced, plus the m <= n being built
-    const int need = m - (int)b->slot_free.size();
-    return grow_slots(b, std::max(need, std::min(b->n_sched / 2, b->bp.n_problems + n - b->n_sched)));
-}
-
-// the slots that reference counts `refs` leave without a problem and that are not free yet: the old slots of the listed problems
-// (and, before the first such call, every slot no problem used from the start)
-static std::vector<int> released_slots(hsddp_batch* b, const std::vector<int>& refs, const std::vector<int>& free_after, int n, const int32_t* problem) {
-    std::vector<char> on_free(b->n_sched, 0);
-    for (int s : free_after) on_free[s] = 1;
-    std::vector<int> freed;
-    auto release = [&](int s) { if (refs[s] == 0 && !on_free[s]) { on_free[s] = 1; freed.push_back(s); } };
-    if (!b->slots_marked) for (int s = 0; s < b->n_sched; ++s) release(s);
-    else for (int k = 0; k < n; ++k) release(b->h_sched_id[problem[k]]);
-    return freed;
-}
-
 // a host list of n distinct problem indices, 1 <= n <= n_problems
 static int check_problem_list(hsddp_batch* b, int n, const int32_t* problem, const char* what) {
     const int P = b->bp.n_problems;
@@ -1804,9 +1790,63 @@ static int stage_ints(hsddp_batch* b, const std::vector<int>& h, int** d) {
     return HSDDP_OK;
 }
 
+// A call that moves the n listed problems to m new schedule slots (restart, per-problem update) plans the move before it builds
+// anything and commits it only once the build has succeeded (commit_slot_moves here, write_slot_moves on the device), so a
+// refused call leaves the slots as they were.  Listed problem k goes to the call's new slot entry[k] < m.
+struct SlotPlan {
+    std::vector<int> slot;              // [n] new slot of listed problem k
+    std::vector<int> target;            // [m] the new slots, taken from the free list
+    std::vector<int> freed;             // slots the call leaves without a problem
+    std::vector<int> refs, free_after;  // slot_refs and slot_free (without the freed slots) after the call
+};
+
+static int plan_slot_moves(hsddp_batch* b, int n, const int32_t* problem, const std::vector<int>& entry, int m, SlotPlan* p) {
+    if (b->slot_refs.empty()) {  // problems per slot, counted by the first such call
+        b->slot_refs.assign(b->n_sched, 0);
+        for (int s : b->h_sched_id) b->slot_refs[s]++;
+    }
+    // at least m free slots: grow by half the capacity at least (a growth copies every slot), but never beyond the n_problems + n
+    // slots a call can need (at most n_problems are referenced, plus the m <= n being built)
+    const int need = m - (int)b->slot_free.size();
+    if (need > 0)
+        if (int rc = grow_slots(b, std::max(need, std::min(b->n_sched / 2, b->bp.n_problems + n - b->n_sched)))) return rc;
+    p->refs = b->slot_refs; p->free_after = b->slot_free;
+    p->target.resize(m); p->slot.resize(n);
+    for (int j = 0; j < m; ++j) { p->target[j] = p->free_after.back(); p->free_after.pop_back(); }
+    for (int k = 0; k < n; ++k) { p->slot[k] = p->target[entry[k]]; p->refs[b->h_sched_id[problem[k]]]--; p->refs[p->slot[k]]++; }
+    // freed: old slots of the listed problems that no problem uses any more (at the first such call: every unused slot)
+    std::vector<char> on_free(b->n_sched, 0);
+    for (int s : p->free_after) on_free[s] = 1;
+    auto release = [&](int s) { if (p->refs[s] == 0 && !on_free[s]) { on_free[s] = 1; p->freed.push_back(s); } };
+    if (!b->slots_marked) for (int s = 0; s < b->n_sched; ++s) release(s);
+    else for (int k = 0; k < n; ++k) release(b->h_sched_id[problem[k]]);
+    return HSDDP_OK;
+}
+
+static void commit_slot_moves(hsddp_batch* b, SlotPlan& p, int n, const int32_t* problem) {
+    b->slot_refs.swap(p.refs);
+    for (int s : p.freed) p.free_after.push_back(s);
+    b->slot_free.swap(p.free_after);
+    for (int k = 0; k < n; ++k) b->h_sched_id[problem[k]] = p.slot[k];
+    b->h_sched_stale = true;
+    b->slots_marked = true;
+}
+
+// the device list of a slot move, problem[n] slot[n] | target[m] gait[m] window[m] | freed[f], then the caller's `tail` (*d_tail)
+static int stage_slot_moves(hsddp_batch* b, const SlotPlan& p, int n, const int32_t* problem, const std::vector<int>& gait,
+                            const std::vector<int>& window, const std::vector<int>& tail, SlotMoves* mv, int** d_tail) {
+    std::vector<int> h(problem, problem + n);
+    for (const std::vector<int>* v : {&p.slot, &p.target, &gait, &window, &p.freed, &tail}) h.insert(h.end(), v->begin(), v->end());
+    int* d;
+    if (int rc = stage_ints(b, h, &d)) return rc;
+    const int m = (int)p.target.size(), f = (int)p.freed.size();
+    *mv = SlotMoves{d, d + n, d + 2 * n, d + 2 * n + m, d + 2 * n + 2 * m, d + 2 * n + 3 * m, m, f, b->d_sched_gait, b->d_sched_window};
+    *d_tail = d + 2 * n + 3 * m + f;
+    return HSDDP_OK;
+}
+
 // k_scatter_rows on the handle's stream: row idx[j] of dst := row j of src (src_stride 0: one row for all), for j < n
 static int scatter_rows(hsddp_batch* b, void* dst, int words, const int* idx, const void* src, int src_stride, int n) {
-    if (n <= 0) return HSDDP_OK;
     const long long total = (long long)n * words;
     k_scatter_rows<<<(unsigned)((total + 255) / 256), 256, 0, b->stream>>>((unsigned*)dst, words, idx, (const unsigned*)src, src_stride, n);
     CK(cudaGetLastError());
@@ -1821,20 +1861,16 @@ int hsddp_batch_restart_problems(hsddp_batch* b, int n, const int32_t* problem, 
     if (!b->has_problems) { g_last_error = "no problems set"; return HSDDP_ERR_STATE; }
     if (!b->mpc_ready) { g_last_error = "hsddp_batch_restart_problems needs the gait library on the device: set the problems with hsddp_batch_set_problems_from_gaits"; return HSDDP_ERR_STATE; }
     const int P = b->bp.n_problems;
-    if (n <= 0 || n > P || !problem || !gait || !window || !x0) { g_last_error = "restart: n must be in [1, n_problems] and every list given"; return HSDDP_ERR_ARG; }
+    int rc;
+    if ((rc = check_problem_list(b, n, problem, "restart"))) return rc;
+    if (!gait || !window || !x0) { g_last_error = "restart: gait, window and x0 must be given"; return HSDDP_ERR_ARG; }
     if (first_solve)
         if (const char* bad = check_budget(first_solve->max_AL_iter, first_solve->max_DDP_iter)) { g_last_error = std::string("invalid first_solve: ") + bad; return HSDDP_ERR_ARG; }
-    std::vector<char> seen(P, 0);
     for (int k = 0; k < n; ++k) {
-        if (problem[k] < 0 || problem[k] >= P) { g_last_error = "restart: problem index out of range"; return HSDDP_ERR_ARG; }
-        if (seen[problem[k]]) { g_last_error = "restart: repeated problem index"; return HSDDP_ERR_ARG; }
-        seen[problem[k]] = 1;
         if (gait[k] < 0 || gait[k] >= b->n_gaits) { g_last_error = "restart: unknown gait"; return HSDDP_ERR_ARG; }
         if (window[k] < 0) { g_last_error = "restart: window does not fit the gait table"; return HSDDP_ERR_ARG; }
     }
     CK(cudaSetDevice(b->device));
-    init_slot_refs(b);
-    int rc;
     if (first_solve && !b->d_budget) {
         if ((rc = dalloc(b, &b->d_budget, (size_t)2 * P))) return rc;
         CK(cudaMemsetAsync(b->d_budget, 0xff, sizeof(int) * 2 * P, b->stream));
@@ -1850,51 +1886,31 @@ int hsddp_batch_restart_problems(hsddp_batch* b, int n, const int32_t* problem, 
         pair_of[k] = it.first->second;
     }
     const int m = (int)bgait.size();
-    if ((rc = ensure_free_slots(b, m, n))) return rc;
-    // slot bookkeeping after the call (applied only once the build has succeeded)
-    std::vector<int> free_after = b->slot_free, bslot(m), refs = b->slot_refs;
-    for (int j = 0; j < m; ++j) { bslot[j] = free_after.back(); free_after.pop_back(); }
-    for (int k = 0; k < n; ++k) { refs[b->h_sched_id[problem[k]]]--; refs[bslot[pair_of[k]]]++; }
-    const std::vector<int> freed = released_slots(b, refs, free_after, n, problem);
-    const int c = m + (int)freed.size();
-    // argument lists: problem[n] slot[n] | gait[m] window[m] slot[m] status[m] | commit slot[c] gait[c] window[c]
-    std::vector<int> h(2 * (size_t)n + 4 * (size_t)m + 3 * (size_t)c);
-    int* hp = h.data();
-    int *a_prob = hp, *a_slot = hp + n, *a_bg = hp + 2 * n, *a_bw = a_bg + m, *a_bs = a_bw + m, *a_st = a_bs + m;
-    int *a_cs = a_st + m, *a_cg = a_cs + c, *a_cw = a_cg + c;
-    for (int k = 0; k < n; ++k) { a_prob[k] = problem[k]; a_slot[k] = bslot[pair_of[k]]; }
-    for (int j = 0; j < m; ++j) { a_bg[j] = bgait[j]; a_bw[j] = bwin[j]; a_bs[j] = bslot[j]; a_st[j] = 0; a_cs[j] = bslot[j]; a_cg[j] = bgait[j]; a_cw[j] = bwin[j]; }
-    for (int j = m; j < c; ++j) { a_cs[j] = freed[j - m]; a_cg[j] = -1; a_cw[j] = 0; }
-    int* d;
-    if ((rc = stage_ints(b, h, &d)) || (rc = scratch(b, &b->d_args_x0, &b->d_args_x0_cap, (size_t)n * 24))) return rc;
+    SlotPlan plan;
+    SlotMoves mv;
+    std::vector<int> status(m, 0);
+    int* d_st;
+    if ((rc = plan_slot_moves(b, n, problem, pair_of, m, &plan)) || (rc = stage_slot_moves(b, plan, n, problem, bgait, bwin, status, &mv, &d_st)) ||
+        (rc = scratch(b, &b->d_args_x0, &b->d_args_x0_cap, (size_t)n * 24))) return rc;
     CK(cudaMemcpyAsync(b->d_args_x0, x0, (size_t)n * 24 * sizeof(double), cudaMemcpyHostToDevice, b->stream));
     // build into the free slots, then one host synchronise for the build status
-    const int *d_bg = d + 2 * n, *d_bw = d_bg + m, *d_bs = d_bw + m;
-    int* d_st = const_cast<int*>(d_bs + m);
-    launch_schedule_build(b, m, d_bg, d_bw, d_bs, b->bp.max_stages, d_st);
+    launch_schedule_build(b, m, mv.gait, mv.window, mv.target, b->bp.max_stages, d_st);
     CK(cudaGetLastError());
-    CK(cudaMemcpyAsync(a_st, d_st, sizeof(int) * m, cudaMemcpyDeviceToHost, b->stream));
+    CK(cudaMemcpyAsync(status.data(), d_st, sizeof(int) * m, cudaMemcpyDeviceToHost, b->stream));
     CK(cudaStreamSynchronize(b->stream));
     for (int j = 0; j < m; ++j) {
-        if (a_st[j] == 1) { g_last_error = "restart: window does not fit the gait table"; return HSDDP_ERR_ARG; }
-        if (a_st[j]) { g_last_error = "restart: schedule exceeds HSDDP_MAX_PHASES / the batch's node capacity"; return HSDDP_ERR_UNSUPPORTED; }
+        if (status[j] == 1) { g_last_error = "restart: window does not fit the gait table"; return HSDDP_ERR_ARG; }
+        if (status[j]) { g_last_error = "restart: schedule exceeds HSDDP_MAX_PHASES / the batch's node capacity"; return HSDDP_ERR_UNSUPPORTED; }
     }
-    RestartArgs ra{d, d + n, d_st + m, d_st + m + c, d_st + m + 2 * c, b->d_args_x0, c,
-                   first_solve ? first_solve->max_AL_iter : -1, first_solve ? first_solve->max_DDP_iter : -1, b->d_sched_gait, b->d_sched_window, 0, {}};
+    RestartArgs ra{b->d_args_x0, first_solve ? first_solve->max_AL_iter : -1, first_solve ? first_solve->max_DDP_iter : -1, 0, {}};
     // (the trial arrays of a batch larger than kClusterLsMax belong to launch positions, not to problems: hsddp_batch_solve_problems)
     for (const WsArray& a : workspace_arrays(b))
         if ((a.flags & WS_RESTART) && *a.field && !((a.flags & WS_SMALL) && P > hsddp_batch::kClusterLsMax)) {
             if (ra.n_clear == kRestartClearMax) { g_last_error = "restart: more workspace arrays than kRestartClearMax"; return HSDDP_ERR_STATE; }
             ra.clear[ra.n_clear++] = {(unsigned*)*a.field, a.bytes() / sizeof(unsigned)};
         }
-    // commit
-    b->slot_refs.swap(refs);
-    for (int s : freed) free_after.push_back(s);
-    b->slot_free.swap(free_after);
-    for (int k = 0; k < n; ++k) b->h_sched_id[problem[k]] = bslot[pair_of[k]];
-    b->h_sched_stale = true;
-    b->slots_marked = true;
-    k_restart<<<n, kThreads, 0, b->stream>>>(b->bp, ra);
+    commit_slot_moves(b, plan, n, problem);
+    k_restart<<<n, kThreads, 0, b->stream>>>(b->bp, mv, ra);
     CK(cudaGetLastError());
     b->n_step_launches++;
     if (first_solve) b->budget_rounds = std::max(b->budget_rounds, (long long)first_solve->max_AL_iter * first_solve->max_DDP_iter);
@@ -1919,7 +1935,6 @@ int hsddp_batch_mpc_update_problems(hsddp_batch* b, int n, const int32_t* proble
     int rc;
     if ((rc = check_problem_list(b, n, problem, "mpc_update_problems"))) return rc;
     CK(cudaSetDevice(b->device));
-    init_slot_refs(b);
     // the distinct slots of the listed problems, one copy each (problems that share a slot share its copy)
     std::map<int, int> copy_of;
     std::vector<int> src, entry(n);
@@ -1929,57 +1944,41 @@ int hsddp_batch_mpc_update_problems(hsddp_batch* b, int n, const int32_t* proble
         entry[k] = it.first->second;
     }
     const int m = (int)src.size();
-    if ((rc = ensure_free_slots(b, m, n))) return rc;
-    // slot bookkeeping after the call (applied only once every copy has been stepped)
-    std::vector<int> free_after = b->slot_free, dst(m), refs = b->slot_refs;
-    for (int j = 0; j < m; ++j) { dst[j] = free_after.back(); free_after.pop_back(); }
-    for (int k = 0; k < n; ++k) { refs[src[entry[k]]]--; refs[dst[entry[k]]]++; }
-    const std::vector<int> freed = released_slots(b, refs, free_after, n, problem);
-    const int f = (int)freed.size();
-    // argument list: problem[n] slot[n] | src[m] dst[m] gait[m] window[m] | freed[f] | -1 | error flag
-    std::vector<int> h(2 * (size_t)n + 4 * (size_t)m + f + 2, 0);
-    for (int k = 0; k < n; ++k) { h[k] = problem[k]; h[n + k] = dst[entry[k]]; }
-    for (int j = 0; j < m; ++j) { h[2 * n + j] = src[j]; h[2 * n + m + j] = dst[j]; }
-    for (int j = 0; j < f; ++j) h[2 * n + 4 * m + j] = freed[j];
-    h[2 * n + 4 * m + f] = -1;
-    int* d;
-    if ((rc = stage_ints(b, h, &d))) return rc;
-    int *d_slot = d + n, *d_src = d + 2 * n, *d_dst = d_src + m, *d_gait = d_dst + m, *d_win = d_gait + m, *d_freed = d_win + m;
-    int *d_m1 = d_freed + f, *d_err = d_m1 + 1;
+    SlotPlan plan;
+    SlotMoves mv;
+    int* d_src;  // src[m] | error flag
+    std::vector<int> tail = src, gw(m, 0);  // (gait / window of the copies: written by k_copy_slots)
+    tail.push_back(0);
+    if ((rc = plan_slot_moves(b, n, problem, entry, m, &plan)) || (rc = stage_slot_moves(b, plan, n, problem, gw, gw, tail, &mv, &d_src))) return rc;
+    int* d_err = d_src + m;
     DevSchedule* sched = const_cast<DevSchedule*>(b->bp.sched);
-    SlotCopyArgs ca{d_src, d_dst, b->d_sched_gait, b->d_sched_window, d_gait, d_win, sched, b->lib.node_stride, 0, {}};
+    SlotCopyArgs ca{d_src, mv.target, b->d_sched_gait, b->d_sched_window, mv.gait, mv.window, sched, b->lib.node_stride, 0, {}};
     for (const SlotArray& a : slot_arrays(b)) {
+        if (a.field == (void**)&b->d_sched_gait || a.field == (void**)&b->d_sched_window) continue;  // (written by the commit)
         if (ca.n_arrays == kSlotArraysMax) { g_last_error = "mpc_update_problems: more slot arrays than kSlotArraysMax"; return HSDDP_ERR_STATE; }
         ca.arr[ca.n_arrays++] = {(unsigned*)*a.field, a.bytes / sizeof(unsigned)};
     }
     CK(cudaEventRecord(b->ev_u0, b->stream));
     k_copy_slots<<<m, 128, 0, b->stream>>>(ca);
-    k_mpc_update_schedules<<<(m + 127) / 128, 128, 0, b->stream>>>(b->lib, m, d_gait, d_win, d_dst, sched, b->d_mpc, d_err);
-    k_reference_rows<<<m, 128, 0, b->stream>>>(b->lib, m, d_gait, d_win, d_dst, sched, b->d_mpc, const_cast<double*>(b->bp.xr),
+    k_mpc_update_schedules<<<(m + 127) / 128, 128, 0, b->stream>>>(b->lib, m, mv.gait, mv.window, mv.target, sched, b->d_mpc, d_err);
+    k_reference_rows<<<m, 128, 0, b->stream>>>(b->lib, m, mv.gait, mv.window, mv.target, sched, b->d_mpc, const_cast<double*>(b->bp.xr),
                                               const_cast<double*>(b->bp.ur), const_cast<double*>(b->bp.prel), nullptr);
     CK(cudaGetLastError());
     b->n_step_launches += 3;
     int err = 0;
     CK(cudaMemcpyAsync(&err, d_err, sizeof(int), cudaMemcpyDeviceToHost, b->stream));
     CK(cudaStreamSynchronize(b->stream));
-    if (err) {  // the copies are dropped: their slots stay on the free list, marked free again on the device
-        if ((rc = scatter_rows(b, b->d_sched_gait, 1, d_dst, d_m1, 0, m))) return rc;
+    if (err) {  // the copies are dropped: their slots stay on the free list and were never marked in use on the device
         CK(cudaEventRecord(b->ev_u1, b->stream));
         g_last_error = err == 1 ? "receding-horizon update: the reference table is exhausted" : "receding-horizon update: schedule exceeds HSDDP_MAX_PHASES / node capacity";
         return err == 1 ? HSDDP_ERR_ARG : HSDDP_ERR_UNSUPPORTED;
     }
-    // commit: the listed problems move to the stepped copies, slots nobody uses any more are freed, then the shift
-    if ((rc = scatter_rows(b, const_cast<int*>(b->bp.sched_id), 1, d, d_slot, 1, n)) || (rc = scatter_rows(b, b->d_sched_gait, 1, d_freed, d_m1, 0, f))) return rc;
-    k_mpc_shift<<<n, kThreads, 0, b->stream>>>(b->bp, b->d_mpc, d);
+    // commit: the listed problems move to the stepped copies and slots nobody uses any more are freed, in the shift's launch
+    k_mpc_shift<<<n, kThreads, 0, b->stream>>>(b->bp, b->d_mpc, mv);
     CK(cudaGetLastError());
     b->n_step_launches++;
     CK(cudaEventRecord(b->ev_u1, b->stream));
-    b->slot_refs.swap(refs);
-    for (int s : freed) free_after.push_back(s);
-    b->slot_free.swap(free_after);
-    for (int k = 0; k < n; ++k) b->h_sched_id[problem[k]] = dst[entry[k]];
-    b->h_sched_stale = true;
-    b->slots_marked = true;
+    commit_slot_moves(b, plan, n, problem);
     return HSDDP_OK;
     });
 }
