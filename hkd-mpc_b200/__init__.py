@@ -16,6 +16,7 @@ hyphen (the repository's contract), so import it with
 import ctypes as C
 import os
 import subprocess
+import sys
 import numpy as np
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
@@ -150,6 +151,9 @@ def lib():
         L.hsddp_batch_solve_problems.argtypes = [vp, C.c_int, ip, C.POINTER(Options)]
         L.hsddp_batch_solve_problems_async.argtypes = [vp, C.c_int, ip, C.POINTER(Options)]
         L.hsddp_batch_get_mpc_command_problems.argtypes = [vp, C.c_int, C.c_int, ip, vp]
+        L.hsddp_batch_set_initial_condition_dev.argtypes = [vp, C.c_int, ip, vp, vp]
+        L.hsddp_batch_set_measured_state_dev.argtypes = [vp, C.c_int, ip, vp, vp, vp]
+        L.hsddp_batch_get_mpc_command_dev.argtypes = [vp, C.c_int, C.c_int, ip, vp, vp]
         for f in ("hsddp_batch_solve", "hsddp_batch_solve_async", "hsddp_batch_compute_cost", "hsddp_batch_lq_approximation",
                   "hsddp_batch_prepare_merit", "hsddp_batch_update_al_params", "hsddp_batch_update_reb_params"):
             getattr(L, f).argtypes = [vp, C.POINTER(Options)]
@@ -213,6 +217,12 @@ def _plist(problems):
 def _check(rc, what):
     if rc != 0:
         raise HsddpError(f"{what} failed with code {rc}: {lib().hsddp_last_error().decode()}", rc)
+
+
+def _torch_tensor(a):
+    """torch if `a` is a torch tensor, else None.  torch is never imported here: a tensor implies it is loaded already."""
+    torch = sys.modules.get("torch")
+    return torch if torch is not None and isinstance(a, torch.Tensor) else None
 
 
 # --------------------------------------------------------------------------
@@ -319,6 +329,7 @@ class MultiPhaseDDPBatch:
         h = C.c_void_p()
         _check(lib().hsddp_batch_create(int(device), C.byref(h)), "hsddp_batch_create")
         self.h = h
+        self.device = int(device)
         self.n = 0
 
     def __del__(self):
@@ -368,8 +379,32 @@ class MultiPhaseDDPBatch:
         nn = int(hz[:P].sum()) + P
         return dict(n_phases=P, horizon=hz[:P].tolist(), contact=c[:P].tolist(), next_contact=cn[:P].tolist(), xr=xr[:nn], ur=ur[:nn], prel_r=pr[:nn], xinit=xi[:nn])
 
+    def _device_io(self, t, dtype, cols, problems, what):
+        """(n, problem list or None, CUDA stream) of a _dev call on tensor t: contiguous, `dtype`, shape (n, cols), on the
+        handle's GPU; HsddpError(ERR_ARG) otherwise, before the library is called."""
+        torch = _torch_tensor(t)
+        if torch is None or not t.is_cuda:
+            raise HsddpError(f"{what}: a torch CUDA tensor is required", ERR_ARG)
+        p = None if problems is None else _plist(problems)
+        n = self.n if p is None else len(p)
+        if t.device.index != self.device:
+            raise HsddpError(f"{what}: tensor on {t.device}, the batch is on cuda:{self.device}", ERR_ARG)
+        if t.dtype != getattr(torch, dtype):
+            raise HsddpError(f"{what}: dtype {t.dtype}, expected torch.{dtype}", ERR_ARG)
+        if tuple(t.shape) != (n, cols):
+            raise HsddpError(f"{what}: shape {tuple(t.shape)}, expected {(n, cols)}", ERR_ARG)
+        if not t.is_contiguous():
+            raise HsddpError(f"{what}: the tensor must be contiguous", ERR_ARG)
+        return n, p, C.c_void_p(torch.cuda.current_stream(t.device).cuda_stream or None)
+
     def set_initial_condition(self, x0, problems=None):
-        """x0: [n_problems][24], or with `problems` (indices) one row per listed problem, which alone get a new state."""
+        """x0: [n_problems][24], or with `problems` (indices) one row per listed problem, which alone get a new state.  A torch
+        CUDA tensor (float64, contiguous, on the batch's GPU) is read on the device, ordered on the current stream."""
+        if _torch_tensor(x0) is not None and x0.is_cuda:
+            n, p, s = self._device_io(x0, "float64", 24, problems, "set_initial_condition")
+            _check(lib().hsddp_batch_set_initial_condition_dev(self.h, n, None if p is None else _ip(p), x0.data_ptr(), s),
+                   "hsddp_batch_set_initial_condition_dev")
+            return
         if problems is not None:
             p = _plist(problems)
             x0 = np.ascontiguousarray(x0, np.float64).reshape(len(p), 24)
@@ -377,6 +412,18 @@ class MultiPhaseDDPBatch:
             return
         x0 = np.ascontiguousarray(x0, np.float64).reshape(self.n, 24)
         _check(lib().hsddp_batch_set_initial_condition(self.h, _dp(x0)), "hsddp_batch_set_initial_condition")
+
+    def set_measured_state(self, meas, problems=None, contact=None):
+        """Initial states from the robots' measurements, on the device, ordered on the current stream (torch CUDA tensors only).
+        meas: float64 [n][24] = eul pos omega_body v_world qJ[12], one row per problem (or per listed problem); x0 = [meas[:12],
+        compute_hkd_state(eul, pos, qJ, contact)] with contact = int32 [n][4] (nonzero = stance) if given, else the contact
+        flags of the problem's first phase as the device holds it (after this tick's mpc_update)."""
+        n, p, s = self._device_io(meas, "float64", 24, problems, "set_measured_state")
+        if contact is not None:
+            self._device_io(contact, "int32", 4, problems, "set_measured_state (contact)")
+        _check(lib().hsddp_batch_set_measured_state_dev(self.h, n, None if p is None else _ip(p), meas.data_ptr(),
+                                                        None if contact is None else contact.data_ptr(), s),
+               "hsddp_batch_set_measured_state_dev")
 
     def reset(self):
         _check(lib().hsddp_batch_reset(self.h), "hsddp_batch_reset")
@@ -529,7 +576,13 @@ class MultiPhaseDDPBatch:
 
     def mpc_command(self, n_steps=8, out=None, problems=None):
         """hkd_command_lcmt payload of every problem (HKDMPC.cpp:207-298), packed on the device; with `problems` (indices) one
-        record per listed problem, in list order."""
+        record per listed problem, in list order.  `out` a torch CUDA tensor (uint8, contiguous, [n][CMD_DTYPE.itemsize], on the
+        batch's GPU): the records are packed straight into it, ordered on the current stream, and `out` is returned."""
+        if _torch_tensor(out) is not None and out.is_cuda:
+            n, p, s = self._device_io(out, "uint8", CMD_DTYPE.itemsize, problems, "mpc_command")
+            _check(lib().hsddp_batch_get_mpc_command_dev(self.h, int(n_steps), n, None if p is None else _ip(p), out.data_ptr(), s),
+                   "hsddp_batch_get_mpc_command_dev")
+            return out
         if problems is not None:
             p = _plist(problems)
             if out is None:

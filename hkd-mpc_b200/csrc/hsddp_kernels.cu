@@ -1132,6 +1132,25 @@ __global__ void k_scatter_rows(unsigned* dst, int words, const int* idx, const u
     dst[(size_t)idx[j] * words + w] = src[(size_t)j * src_stride + w];
 }
 
+// HKDMPCSolver::update's initial condition from the robot's measurement (hsddp_batch_set_measured_state_dev), one thread per
+// listed problem: x0 row list[j] (nullptr: row j) := [meas[0:12], compute_hkd_state(eul, pos, qJ, contact)] (HKDModel.h:65-96)
+// with meas row j = eul pos omega_body v_world qJ[12].  contact: the caller's flags row j (nonzero = stance) or, without them,
+// the first phase of the problem's schedule as it stands when the kernel runs.
+__global__ void k_measured_state(BatchPtrs bp, const double* meas, const int* contact, const int* list, int n) {
+    const int j = blockIdx.x * blockDim.x + threadIdx.x;
+    if (j >= n) return;
+    const int p = list ? list[j] : j;
+    const double* m = meas + (size_t)j * 24;
+    unsigned cm = 0;
+    if (contact) for (int l = 0; l < 4; ++l) cm |= contact[4 * j + l] ? 1u << l : 0u;
+    else cm = bp.sched[bp.sched_id[p]].cmask[0];
+    double x[24];
+    for (int i = 0; i < 12; ++i) x[i] = m[i];
+    hkd::hkd_state(m, m + 3, m + 12, cm, x + 12);
+    double* x0 = bp.x0 + (size_t)p * 24;
+    for (int i = 0; i < 24; ++i) x0[i] = x[i];
+}
+
 // FP64 throughput probes (roofline denominators measured on the box)
 __global__ void k_dfma_probe(double* out, int iters) {
     double a0 = threadIdx.x * 1e-3, a1 = a0 + 1, a2 = a0 + 2, a3 = a0 + 3, a4 = a0 + 4, a5 = a0 + 5, a6 = a0 + 6, a7 = a0 + 7;
@@ -1238,6 +1257,13 @@ struct hsddp_batch {
     std::vector<char> budget_pending;  // [P] the problem's override is still pending (allocated with d_budget)
     int n_budget_pending = 0;
     bool slots_marked = false;     // the slots no problem used are on the free list (done by the first restart)
+    // the _dev entry points (buffers in device memory, ordered on the caller's stream): ev_in joins the caller's stream into the
+    // handle's at the start of a call, ev_out the handle's stream into the caller's after its last launch
+    cudaEvent_t ev_in = nullptr, ev_out = nullptr;
+    // their problem lists go up from pinned host buffers: a pageable source lets cudaMemcpyAsync wait for the handle's stream,
+    // which waits for the caller's work.  A buffer is reused once the copy that read it has run (`read`).
+    struct PinnedList { int* h = nullptr; size_t cap = 0; cudaEvent_t read = nullptr; };
+    std::vector<PinnedList> pinned_lists;
 };
 
 namespace {
@@ -1477,6 +1503,8 @@ static int batch_init(hsddp_batch* b, int device) {
     CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&b->blocks_per_sm, k_solve, kThreads, 0));
     if (b->blocks_per_sm < 1) b->blocks_per_sm = 1;
     CK(cudaEventCreateWithFlags(&b->ev_fork, cudaEventDisableTiming));
+    CK(cudaEventCreateWithFlags(&b->ev_in, cudaEventDisableTiming));
+    CK(cudaEventCreateWithFlags(&b->ev_out, cudaEventDisableTiming));
     CK(cudaFuncSetAttribute(k_sweep_w1, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
     CK(cudaFuncSetAttribute(k_lr_w1, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
     if (const char* e = getenv("HSDDP_SWEEP_SPEC")) { const int v = atoi(e); b->sweep_spec = (v >= 2 && v <= 32) ? v : 0; }
@@ -1510,6 +1538,12 @@ int hsddp_batch_destroy(hsddp_batch* b) {
     for (int i = 0; i < 8; ++i) if (b->slots[i]) cudaEventDestroy(b->slots[i]);
     if (b->stream) cudaStreamDestroy(b->stream);
     if (b->ev_fork) cudaEventDestroy(b->ev_fork);
+    if (b->ev_in) cudaEventDestroy(b->ev_in);
+    if (b->ev_out) cudaEventDestroy(b->ev_out);
+    for (auto& s : b->pinned_lists) {
+        if (s.read) cudaEventDestroy(s.read);
+        if (s.h) cudaFreeHost(s.h);
+    }
     for (int g = 0; g < hsddp_batch::kMaxGroups; ++g) {
         if (b->gevent[g]) cudaEventDestroy(b->gevent[g]);
         if (b->gstream[g]) cudaStreamDestroy(b->gstream[g]);
@@ -1644,8 +1678,13 @@ int hsddp_batch_set_problems_from_gaits(hsddp_batch* b, int n_gaits, const int32
         return rc;
     lib.plan = plan_duration;
     lib.node_stride = std::min(HSDDP_MAX_STAGES, (int)std::lround(plan_duration / kTickDt) + 1) + MAXPH;
-    for (const SlotArray& a : slot_arrays(b))  // one schedule slot per schedule
+    for (const SlotArray& a : slot_arrays(b)) {  // one schedule slot per schedule
         if ((rc = dalloc_bytes(b, a.field, (size_t)n_schedules * a.bytes))) return rc;
+        // zero-filled as grow_slots fills new slots: an update adds node rows it does not write (xinit), and those must read
+        // back the same in every handle whatever the allocation held before (gait and window are copied in below)
+        if (a.field != (void**)&b->d_sched_gait && a.field != (void**)&b->d_sched_window)
+            CK(cudaMemsetAsync(*a.field, 0, (size_t)n_schedules * a.bytes, b->stream));
+    }
     int *d_status, *d_err;
     if ((rc = dalloc(b, &d_status, (size_t)n_schedules)) || (rc = dalloc(b, &d_err, (size_t)4))) return rc;
     CK(cudaMemcpy(b->d_sched_gait, sched_gait, n_schedules * sizeof(int), cudaMemcpyHostToDevice));
@@ -2493,6 +2532,129 @@ int hsddp_batch_get_mpc_command_problems(hsddp_batch* b, int n_steps, int n, con
     if (!b || !b->has_problems || !out || n_steps < 1 || n_steps > HSDDP_CMD_MAX_STEPS) return HSDDP_ERR_ARG;
     if (int rc = check_problem_list(b, n, problem, "get_mpc_command_problems")) return rc;
     return get_commands(b, n_steps, n, problem, out);
+    });
+}
+
+// --- the _dev entry points: buffers in device memory of the handle's GPU, ordered on the caller's stream ---
+
+// a list the _dev calls take: n distinct indices, or nullptr for every problem in index order (then n == n_problems)
+static int check_dev_list(hsddp_batch* b, int n, const int32_t* problem, const char* what) {
+    if (problem) return check_problem_list(b, n, problem, what);
+    if (n != b->bp.n_problems) { g_last_error = std::string(what) + ": without a list n must be n_problems"; return HSDDP_ERR_ARG; }
+    return HSDDP_OK;
+}
+
+// p must be device or managed memory of the handle's GPU, aligned to `align` bytes
+static int check_dev_buffer(hsddp_batch* b, const void* p, size_t align, const char* what) {
+    if (!p) { g_last_error = std::string(what) + ": NULL buffer"; return HSDDP_ERR_ARG; }
+    cudaPointerAttributes a{};
+    if (cudaPointerGetAttributes(&a, p) != cudaSuccess) {
+        cudaGetLastError();  // (not a sticky error: clear it so that it is not reported by a later call)
+        g_last_error = std::string(what) + ": not a CUDA pointer";
+        return HSDDP_ERR_ARG;
+    }
+    if ((a.type != cudaMemoryTypeDevice && a.type != cudaMemoryTypeManaged) || a.device != b->device) {
+        g_last_error = std::string(what) + ": the buffer is not device memory of the handle's GPU";
+        return HSDDP_ERR_ARG;
+    }
+    if ((uintptr_t)p % align) { g_last_error = std::string(what) + ": misaligned buffer"; return HSDDP_ERR_ARG; }
+    return HSDDP_OK;
+}
+
+// *d := the listed indices in the call's device argument list, copied from a pinned host buffer on the handle's stream
+static int stage_list_pinned(hsddp_batch* b, int n, const int32_t* problem, int** d) {
+    hsddp_batch::PinnedList* s = nullptr;
+    for (auto& q : b->pinned_lists) {
+        if (q.cap < (size_t)n) continue;
+        const cudaError_t e = cudaEventQuery(q.read);
+        if (e == cudaSuccess) { s = &q; break; }
+        if (e != cudaErrorNotReady) CK(e);
+        cudaGetLastError();  // (clear the not-ready status)
+    }
+    if (!s) {
+        hsddp_batch::PinnedList q;
+        q.cap = std::max((size_t)n, (size_t)1024);
+        CK(cudaHostAlloc((void**)&q.h, q.cap * sizeof(int), cudaHostAllocDefault));
+        if (cudaEventCreateWithFlags(&q.read, cudaEventDisableTiming) != cudaSuccess) {
+            cudaFreeHost(q.h);
+            g_last_error = "cudaEventCreateWithFlags failed";
+            return HSDDP_ERR_CUDA;
+        }
+        b->pinned_lists.push_back(q);
+        s = &b->pinned_lists.back();
+    }
+    std::memcpy(s->h, problem, (size_t)n * sizeof(int));
+    if (int rc = scratch(b, &b->d_args, &b->d_args_cap, (size_t)n)) return rc;
+    CK(cudaMemcpyAsync(b->d_args, s->h, (size_t)n * sizeof(int), cudaMemcpyHostToDevice, b->stream));
+    CK(cudaEventRecord(s->read, b->stream));
+    *d = b->d_args;
+    return HSDDP_OK;
+}
+
+// The stream contract: the handle's stream waits for what the caller queued on `stream` before the call (join_caller), and
+// the caller's stream for the call's last launch (release_caller).  Neither synchronises the host.
+static int join_caller(hsddp_batch* b, void* stream) {
+    CK(cudaEventRecord(b->ev_in, (cudaStream_t)stream));
+    CK(cudaStreamWaitEvent(b->stream, b->ev_in, 0));
+    return HSDDP_OK;
+}
+
+static int release_caller(hsddp_batch* b, void* stream) {
+    CK(cudaEventRecord(b->ev_out, b->stream));
+    CK(cudaStreamWaitEvent((cudaStream_t)stream, b->ev_out, 0));
+    return HSDDP_OK;
+}
+
+int hsddp_batch_set_initial_condition_dev(hsddp_batch* b, int n, const int32_t* problem, const double* x0_dev, void* stream) {
+    return guarded([&]() -> int {
+    if (!b || !b->has_problems) { g_last_error = "no problems set"; return HSDDP_ERR_ARG; }
+    int rc, *d = nullptr;
+    if ((rc = check_dev_list(b, n, problem, "set_initial_condition_dev")) || (rc = check_dev_buffer(b, x0_dev, sizeof(double), "set_initial_condition_dev")))
+        return rc;
+    CK(cudaSetDevice(b->device));
+    if (problem && (rc = stage_list_pinned(b, n, problem, &d))) return rc;
+    if ((rc = join_caller(b, stream))) return rc;
+    if (problem) {
+        if ((rc = scatter_rows(b, b->bp.x0, 48, d, x0_dev, 48, n))) return rc;
+    } else {
+        CK(cudaMemcpyAsync(b->bp.x0, x0_dev, sizeof(double) * 24 * (size_t)n, cudaMemcpyDeviceToDevice, b->stream));
+    }
+    return release_caller(b, stream);
+    });
+}
+
+int hsddp_batch_set_measured_state_dev(hsddp_batch* b, int n, const int32_t* problem, const double* meas_dev,
+                                       const int32_t* contact_dev, void* stream) {
+    return guarded([&]() -> int {
+    if (!b || !b->has_problems) { g_last_error = "no problems set"; return HSDDP_ERR_ARG; }
+    int rc, *d = nullptr;
+    if ((rc = check_dev_list(b, n, problem, "set_measured_state_dev")) || (rc = check_dev_buffer(b, meas_dev, sizeof(double), "set_measured_state_dev")))
+        return rc;
+    if (contact_dev && (rc = check_dev_buffer(b, contact_dev, sizeof(int32_t), "set_measured_state_dev (contact)"))) return rc;
+    CK(cudaSetDevice(b->device));
+    if (problem && (rc = stage_list_pinned(b, n, problem, &d))) return rc;
+    if ((rc = join_caller(b, stream))) return rc;
+    k_measured_state<<<(n + 127) / 128, 128, 0, b->stream>>>(b->bp, meas_dev, contact_dev, d, n);
+    CK(cudaGetLastError());
+    b->n_step_launches++;
+    return release_caller(b, stream);
+    });
+}
+
+int hsddp_batch_get_mpc_command_dev(hsddp_batch* b, int n_steps, int n, const int32_t* problem, hsddp_mpc_command* out_dev, void* stream) {
+    return guarded([&]() -> int {
+    if (!b || !b->has_problems) { g_last_error = "no problems set"; return HSDDP_ERR_ARG; }
+    if (n_steps < 1 || n_steps > HSDDP_CMD_MAX_STEPS) { g_last_error = "get_mpc_command_dev: n_steps must be in [1, HSDDP_CMD_MAX_STEPS]"; return HSDDP_ERR_ARG; }
+    int rc, *d = nullptr;
+    if ((rc = check_dev_list(b, n, problem, "get_mpc_command_dev")) || (rc = check_dev_buffer(b, out_dev, alignof(hsddp_mpc_command), "get_mpc_command_dev")))
+        return rc;
+    CK(cudaSetDevice(b->device));
+    if (problem && (rc = stage_list_pinned(b, n, problem, &d))) return rc;
+    if ((rc = join_caller(b, stream))) return rc;
+    k_command<<<n, 128, 0, b->stream>>>(b->bp, n_steps, out_dev, d);
+    CK(cudaGetLastError());
+    b->n_step_launches++;
+    return release_caller(b, stream);
     });
 }
 

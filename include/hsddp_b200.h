@@ -332,6 +332,34 @@ int hsddp_batch_get_mpc_command(hsddp_batch* b, int n_steps, hsddp_mpc_command* 
  * hsddp_batch_mpc_update_problems): out is [n] on the host, record k for problem[k] */
 int hsddp_batch_get_mpc_command_problems(hsddp_batch* b, int n_steps, int n, const int32_t* problem, hsddp_mpc_command* out);
 
+/* Ticks from GPU memory: the robots' states come in and the command records go out through the CALLER's device buffers,
+ * ordered on the caller's CUDA stream, for fleets whose states are produced on the same GPU (e.g. a simulator's tensors).
+ *   - problem: a HOST list of n distinct indices (as the _problems entry points), or NULL for every problem in index order
+ *     (then n == n_problems); row / record k belongs to problem[k].
+ *   - stream: the caller's cudaStream_t passed as void* (NULL = the default stream, as in CUDA).
+ * Stream contract.  Each call records an event on `stream` and makes the handle's stream wait on it, so the inputs are read
+ * only after all work queued on `stream` before the call.  After its last launch it records an event on the handle's stream
+ * and makes `stream` wait on it, so work queued on `stream` afterwards sees the outputs and may reuse the input buffers.  None of
+ * the three synchronises the host: they return once the work is queued.  hsddp_batch_solve[_problems]_async queues on the
+ * handle's stream, so set_*_dev -> solve_async -> get_mpc_command_dev needs no further synchronisation.
+ * Refusals return before anything is queued and leave the batch unchanged: HSDDP_ERR_ARG for a handle without problems, a NULL
+ * buffer, a buffer that is not device or managed memory of the handle's GPU (pageable or pinned host memory, another GPU), a
+ * buffer not aligned to its element type (double, int32_t, hsddp_mpc_command), a bad problem list, or n_steps outside
+ * [1, HSDDP_CMD_MAX_STEPS]. */
+/* MultiPhaseDDP::set_initial_condition (MultiPhaseDDP.h:37): x0_dev is [n][24] doubles in device memory, row k for problem[k] */
+int hsddp_batch_set_initial_condition_dev(hsddp_batch* b, int n, const int32_t* problem, const double* x0_dev, void* stream);
+/* HKDMPCSolver::update's initial condition from the robot's measurement, on the device.
+ * meas_dev: [n][24] doubles = eul(yaw,pitch,roll) pos omega_body v_world (x0's first 12 entries) followed by qJ[12].
+ * x0 = [meas[0:12], compute_hkd_state(eul, pos, qJ, contact)] (hkd_compute_state) with contact = contact_dev[k][4] (nonzero =
+ * stance) if given, else the contact flags of the problem's FIRST PHASE as the device holds it when the kernel runs (after
+ * this tick's hsddp_batch_mpc_update).  That NULL rule is the one hkd_default_x0 and the workloads apply at the window start;
+ * the reference's own update-time source of the contact (HKDMPC.cpp:119-129) is not restated in this library, so a caller
+ * with contact sensing passes its own flags. */
+int hsddp_batch_set_measured_state_dev(hsddp_batch* b, int n, const int32_t* problem, const double* meas_dev,
+                                       const int32_t* contact_dev, void* stream);
+/* hsddp_batch_get_mpc_command[_problems] straight into out_dev ([n] records in device memory), record k for problem[k] */
+int hsddp_batch_get_mpc_command_dev(hsddp_batch* b, int n_steps, int n, const int32_t* problem, hsddp_mpc_command* out_dev, void* stream);
+
 /* CUDA-event timing on the handle's stream (slots 0..7): record, then elapsed ms between two slots */
 int hsddp_batch_event_record(hsddp_batch* b, int slot);
 int hsddp_batch_event_elapsed_ms(hsddp_batch* b, int slot0, int slot1, float* ms);
